@@ -24,6 +24,10 @@ halo-overlapped chunks) and 5 (WaveFlow) at the same GPU count, config 1's per-c
 the one model the reference itself records a speed for (its speed-test notebook's 48-flow ax WaveGlow, `--config 6`), and the
 per-call latency of WaveFlow in the layout of the author's trained checkpoints (h = 20, separable 7x7; fp32 CUDA-core mode);
 `--no-extra` skips them, `--config N` runs one alone.
+
+`--dump-outputs DIR` writes the waveform batch the timed path returned from its last timed step as DIR/audio.npy
+(float32; rank 0's batch), so that two builds run with the same arguments - hence the same seeded weights and inputs -
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -45,6 +49,21 @@ MODEL_KW = dict(n_mel_channels=80, n_flows=12, n_group=8, n_early_every=4, n_ear
                 WN_config=dict(n_layers=8, n_channels=256, kernel_size=3, speaker_embed_dim=0, rezero=False),
                 win_length=1024, hop_length=256)
 METRIC = "waveglow_infer_audio_samples_per_sec"
+
+
+DUMP_BUDGET = 64_000_000     # bytes of .npy data --dump-outputs may write
+
+
+def dump_outputs(out_dir, audio):
+    """--dump-outputs: `audio` (the last timed step's return value) as out_dir/audio.npy in float32.  A batch over the
+    budget is cut to a fixed seeded sample of its elements (sorted flat positions, the same for every run of the same
+    shape), stored 1-D."""
+    a = audio.detach().float().cpu().numpy()
+    keep = (DUMP_BUDGET - 4096) // a.itemsize          # room for the .npy header
+    if a.size > keep:
+        a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "audio.npy"), a)
 
 
 def algorithmic_macs(C=256, L=8, H=256, n_mel=80, G=8, J=4, flows=((8, 4),) * 4 + ((6, 3),) * 4 + ((4, 2),) * 4):
@@ -234,7 +253,7 @@ def run_reference(args):
         return
     kind, source, run = make_cpu_runner()
     allt = os.cpu_count() or 1
-    steps, warm = max(args.steps, 1), max(min(args.warmup, 1), 1)
+    steps, warm = args.steps, max(min(args.warmup, 1), 1)
     cal = timed_cpu(run, 1, 86, 1, 1, allt)
     b, tm = 1, 861
     for cand in (861, 430, 172, 86):
@@ -352,6 +371,8 @@ def run_waveflow(args):
     clocks = sampler.stop() if rank == 0 else None
     wf_layer_ms = np.array([[ev_b[i][j].elapsed_time(ev_e[i][j]) for j in range(n_ev)] for i in range(args.steps)]).mean(axis=0)
     finite_wf = bool(torch.isfinite(out).all())
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     launches_wf = int(model.launch_count() * args.steps)
     del model, out, mel, z
     torch.cuda.empty_cache()
@@ -417,6 +438,8 @@ def run_longform(args):
     if world > 1:
         t = torch.tensor([ms], device=dev, dtype=torch.float64); dist.all_reduce(t, op=dist.ReduceOp.MAX); ms = float(t.item())
     finite_lf = bool(torch.isfinite(out).all()) if out is not None else True
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     launches_lf = int(model.launch_count() * args.steps)
     plan = plan_chunks(Tm, world, model.pack_config)
     del model, out, mel, z
@@ -460,7 +483,14 @@ def main():
     ap.add_argument("--config", type=int, default=0, choices=[0, 1, 2, 3, 4, 5, 6],
                     help="BASELINE.json config preset (1-based); 0 = use the individual flags (default = config 2); "
                          "6 = the reference notebook's 48-flow ax WaveGlow, batch-1 latency (not a BASELINE.json config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the waveforms of the last timed step to DIR/audio.npy (float32, at most 64 MB: a larger "
+                         "batch is cut to a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs records the CUDA path's outputs; the reference arm times a CPU sample of other inputs")
     world_env = int(os.environ.get("WORLD_SIZE", "1"))
     if args.precision is None:
         args.precision = "f16f8" if (args.workload == "waveglow" and args.channels == 256 and args.config in (0, 1, 2)) else "bf16x3"
@@ -552,7 +582,7 @@ def run_notebook_latency(args):
     for _ in range(3):
         out = model.infer(mel, speaker_ids=ids, sigma=1.0, return_CPU=False, z=z)
     torch.cuda.synchronize()
-    n = 10
+    n = args.steps
     t0, t1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t0.record()
     for _ in range(n):
@@ -562,6 +592,8 @@ def run_notebook_latency(args):
     ms = t0.elapsed_time(t1) / n
     samples = int(out.shape[1])
     finite = bool(torch.isfinite(out).all())
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     del model
     torch.cuda.empty_cache()
     if rank != 0:
@@ -638,10 +670,10 @@ def with_extra_configs(args, line, rank):
                          ("config2_bf16x3", run_waveglow, dict(config=2, precision="bf16x3")),
                          ("config3", run_waveglow, dict(config=3)), ("config4", run_longform, dict(config=4)),
                          ("config5", run_waveflow, dict(config=5, workload="waveflow")),
-                         ("notebook_ax_latency", run_notebook_latency, dict(config=6)),
+                         ("notebook_ax_latency", run_notebook_latency, dict(config=6, steps=10)),
                          ("waveflow_trained_layout_latency", run_waveflow_trained_latency, dict(config=6))):
         a = copy.copy(args)
-        a.steps, a.warmup, a.no_cpu_baseline, a.precision = 3, 3, True, "bf16"
+        a.steps, a.warmup, a.no_cpu_baseline, a.precision, a.dump_outputs = 3, 3, True, "bf16", None
         for k, v in kw.items():
             setattr(a, k, v)
         if a.config == 3:
@@ -774,13 +806,16 @@ def run_waveglow(args):
     barrier()
     t0.record()
     for i in range(args.steps):
-        step_resident((ev_b[i], ev_e[i]))
+        last = step_resident((ev_b[i], ev_e[i]))
     drain()
     t1.record()
     barrier()
     ms_total = max_over_ranks(t0.elapsed_time(t1))
     clocks = sampler.stop() if rank == 0 else None
     layer_ms = np.array([[ev_b[i][j].elapsed_time(ev_e[i][j]) for j in range(n_layers_total)] for i in range(args.steps)])
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, last)
+    del last
 
     # ---- timed region 2: end to end through host buffers ----------------------------------
     for e in in_free:

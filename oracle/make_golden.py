@@ -137,10 +137,17 @@ CASES = {
 SPEAKERS = {"speaker": [5, 0, 77], "speaker256": [3, 200]}
 # Full-length cases (`python oracle/make_golden.py big`): one utterance of BASELINE.json configs[1] (T_mel = 861, 10 s).
 # mel and z are NOT stored (1.2 MB of noise): tests regenerate them from the seeds with `synthetic_inputs` and check the
-# stored CRC32s, so the file holds only the reference's fp32 and fp64 waveforms.
+# stored CRC32s, so the file holds only the reference's fp32 and fp64 waveforms.  To keep each file under 1 MB, the
+# waveforms are stored at a fixed seeded sample of positions (`sample_idx`, sorted; `n_samples` is the full length).
 BIG_CASES = {
     "config2_1x861": (dict(), 1, 861, 0.666, 1234, 0),
 }
+BIG_SAMPLES = 8192
+
+
+def sample_positions(n, k=BIG_SAMPLES, seed=0):
+    """Sorted seeded sample of k of n waveform positions (stored with the golden, so the draw need not be reproducible)."""
+    return np.sort(np.random.default_rng(seed).choice(n, k, replace=False)).astype(np.int32)
 
 
 def main_big():
@@ -155,10 +162,12 @@ def main_big():
         out64 = run_reference(ref_glow, cfg, sd, mel.astype(np.float64), z.astype(np.float64), sigma, torch.float64)
         print(f"{name}: out {out32.shape} rms {np.sqrt((out64 ** 2).mean()):.3f} max {np.abs(out64).max():.3f} "
               f"ref fp32-vs-fp64 max-abs {np.abs(out32 - out64).max():.2e}")
+        idx = sample_positions(out64.shape[1])
         np.savez_compressed(os.path.join(outdir, f"{name}.npz"),
                             config=json.dumps(kw), batch=batch, t_mel=t_mel, sigma=sigma, weight_seed=wseed, input_seed=iseed,
                             mel_crc32=zlib.crc32(np.ascontiguousarray(mel).tobytes()), z_crc32=zlib.crc32(np.ascontiguousarray(z).tobytes()),
-                            audio_ref_fp32=out32, audio_ref_fp64=out64.astype(np.float64))
+                            n_samples=out64.shape[1], sample_idx=idx,
+                            audio_ref_fp32=out32[:, idx], audio_ref_fp64=out64[:, idx].astype(np.float64))
 
 
 def main():

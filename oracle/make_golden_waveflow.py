@@ -27,7 +27,7 @@ ROOT = os.path.dirname(HERE)
 sys.path.insert(0, ROOT)
 
 from oracle.waveflow_oracle import WaveFlowConfig, synthetic_state_dict  # noqa: E402
-from oracle.make_golden import InjectedNormal  # noqa: E402
+from oracle.make_golden import InjectedNormal, sample_positions  # noqa: E402
 
 
 def load_reference_ax():
@@ -197,7 +197,8 @@ def main_ax(WaveGlowAx, outdir, only=()):
 
 BIG_CASES = {
     # BASELINE config 5 model on one full-length utterance (10 s, T_mel = 861): `python oracle/make_golden_waveflow.py big`.
-    # Only the reference's `inverse` outputs are stored; mel / z are regenerated from the seed and checked by CRC32.
+    # Only the reference's `inverse` outputs are stored, at the sampled positions of make_golden.sample_positions; mel / z
+    # are regenerated from the seed and checked by CRC32.
     "waveflow_config5_1x861": (dict(), 1, 861, 0.666, 1234, 0),
 }
 
@@ -225,10 +226,12 @@ def main_big():
             print(f"{name} {tag}: {time.time() - t:.1f} s", flush=True)
         print(f"{name}: out {outs['fp64'].shape} rms {np.sqrt((outs['fp64'] ** 2).mean()):.3f} "
               f"fp32-vs-fp64 {np.abs(outs['fp32'] - outs['fp64']).max():.2e}")
+        idx = sample_positions(outs["fp64"].shape[1])
         np.savez_compressed(os.path.join(outdir, f"{name}.npz"), config=json.dumps(kw), batch=batch, frames=frames, sigma=sigma,
                             weight_seed=wseed, input_seed=iseed, mel_crc32=zlib.crc32(np.ascontiguousarray(mel).tobytes()),
                             z_crc32=zlib.crc32(np.ascontiguousarray(z).tobytes()),
-                            inverse_ref_fp32=outs["fp32"], inverse_ref_fp64=outs["fp64"].astype(np.float64))
+                            n_samples=outs["fp64"].shape[1], sample_idx=idx,
+                            inverse_ref_fp32=outs["fp32"][:, idx], inverse_ref_fp64=outs["fp64"][:, idx].astype(np.float64))
 
 
 def main():

@@ -5,6 +5,8 @@ import os
 import subprocess
 import sys
 
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -26,19 +28,41 @@ def test_reference_arm_json_line():
     assert d["e2e"] == {"value": d["value"], "unit": "samples/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
 
 
+@pytest.mark.parametrize("argv", [["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]])
+def test_rejected_arguments(argv):
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=300, cwd=ROOT)
+    assert out.returncode == 2 and "error:" in out.stderr
+
+
+def test_dump_outputs_budget(tmp_path, monkeypatch):
+    """Within the budget the batch is written whole; beyond it, as the same seeded sample of its elements every time."""
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    import bench
+    audio = torch.randn(4, 1000, dtype=torch.float64)
+    bench.dump_outputs(str(tmp_path / "whole"), audio)
+    got = np.load(tmp_path / "whole" / "audio.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, audio.float().numpy())
+    monkeypatch.setattr(bench, "DUMP_BUDGET", 4096 + 4 * 1500)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), audio)
+    a, b = np.load(tmp_path / "a" / "audio.npy"), np.load(tmp_path / "b" / "audio.npy")
+    assert a.shape == (1500,) and np.array_equal(a, b) and np.isin(a, audio.float().numpy()).all()
+
+
 def test_default_precision_resolution():
     """`--precision` defaults to the fp32-path mode of the workload: f16f8 for the 256-channel WaveGlow, bf16x3 otherwise."""
     src = open(os.path.join(ROOT, "bench.py")).read()
     assert 'args.precision = "f16f8" if (args.workload == "waveglow" and args.channels == 256 and args.config in (0, 1, 2)) else "bf16x3"' in src
 
 
-import pytest
-
-
 @pytest.mark.gpu
-def test_gpu_arm_json_line():
-    """The driver's line at N=1 (short run): every key of the contract, a live roofline and a live accuracy check."""
-    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-cpu-baseline", "--no-extra"],
+def test_gpu_arm_json_line(tmp_path):
+    """The driver's line at N=1 (short run): every key of the contract, a live roofline and a live accuracy check; the
+    dumped waveforms are the batch of the timed path."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "3", "--no-cpu-baseline", "--no-extra",
+                          "--dump-outputs", str(tmp_path)],
                          capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
@@ -60,3 +84,20 @@ def test_gpu_arm_json_line():
     assert d["gpu_launches"] == 2 * 124
     a = d["accuracy"]
     assert a["max_abs"] <= 1e-3 and a["snr_db"] >= 60.0
+
+    # utterance 0 of the dump against a batch-1 call on bench.py's inputs (an utterance's bytes do not depend on its batch)
+    import numpy as np
+    import torch
+    sys.path.insert(0, ROOT)
+    from bench import MODEL_KW
+    from cookietts_b200 import WaveGlow
+    from cookietts_b200.synthetic import ModelConfig, synthetic_state_dict
+    dumped = np.load(tmp_path / "audio.npy")
+    assert dumped.dtype == np.float32 and dumped.shape == (16, 861 * 256) and np.isfinite(dumped).all()
+    g = torch.Generator().manual_seed(1000)
+    mel = (torch.randn(16, 80, 861, generator=g) * 2.0 - 5.0).clamp_(-11.5129, 2.0)
+    z = torch.randn(16, 861 * 256, generator=g)
+    m = WaveGlow(precision="f16f8", **MODEL_KW)
+    m.load_state_dict({k: torch.from_numpy(v) for k, v in synthetic_state_dict(ModelConfig(), 1234).items()})
+    one = m.cuda().eval().infer(mel[:1].cuda(), sigma=0.666, z=z[:1].cuda()).cpu().numpy()
+    assert np.array_equal(one[0], dumped[0])

@@ -41,7 +41,8 @@ def test_config2_and_config3_batches(precision, batch):
     assert out.shape == (batch, 861 * 256) and torch.isfinite(out).all()
     ref = g["audio_ref_fp64"]
     tol, snr = ((5e-2, 45.0) if precision == "bf16" else (1e-3, 60.0))
-    assert max_abs(out[:1].cpu().numpy(), ref) <= tol and snr_db(ref, out[:1].cpu().numpy()) >= snr
+    got = out[:1].cpu().numpy()[:, g["sample_idx"]]       # the golden holds the reference's waveform at these positions
+    assert max_abs(got, ref) <= tol and snr_db(ref, got) >= snr
     k = batch - 3
     alone = m.infer(mel[k:k + 1].cuda(), sigma=float(g["sigma"]), z=z[k:k + 1].cuda())
     assert torch.equal(alone[0], out[k])

@@ -92,7 +92,8 @@ def test_config2_length_matches_reference_golden(precision):
     model = model.cuda().eval()
     out = model.infer(torch.from_numpy(mel).cuda(), sigma=float(g["sigma"]), z=torch.from_numpy(z).cuda()).cpu().numpy()
     ref = g["audio_ref_fp64"]
-    assert out.shape == ref.shape and np.isfinite(out).all()
+    assert out.shape == (1, int(g["n_samples"])) and np.isfinite(out).all()
+    out = out[:, g["sample_idx"]]                     # the golden holds the reference's waveform at these positions
     assert max_abs(out, ref) <= TOL[precision]["max_abs"]
     assert snr_db(ref, out) >= TOL[precision]["snr"]
     if precision == "ffma":

@@ -127,9 +127,10 @@ def test_config5_full_length_matches_reference(precision):
     m = build(cfg, sd, precision)
     out, _ = m.inverse(torch.from_numpy(z).cuda() * float(g["sigma"]), torch.from_numpy(mel).cuda(), return_CPU=True)
     ref = g["inverse_ref_fp64"]
-    assert out.shape == ref.shape and torch.isfinite(out).all()
-    assert max_abs(out.numpy(), ref) <= TOL[precision]["max_abs"]
-    assert snr_db(ref, out.numpy()) >= TOL[precision]["snr"]
+    assert out.shape == (batch, int(g["n_samples"])) and torch.isfinite(out).all()
+    out = out.numpy()[:, g["sample_idx"]]             # the golden holds the reference's waveform at these positions
+    assert max_abs(out, ref) <= TOL[precision]["max_abs"]
+    assert snr_db(ref, out) >= TOL[precision]["snr"]
 
 
 def test_config5_batch_64_full_length_is_consistent():
@@ -151,8 +152,9 @@ def test_config5_batch_64_full_length_is_consistent():
     out, _ = m.inverse(z.cuda() * sigma, mel.cuda(), return_CPU=True)
     assert torch.isfinite(out).all()
     ref = g["inverse_ref_fp64"]
-    assert max_abs(out[:1].numpy(), ref) <= TOL["bf16x3"]["max_abs"]
-    assert snr_db(ref, out[:1].numpy()) >= TOL["bf16x3"]["snr"]
+    got = out[:1].numpy()[:, g["sample_idx"]]         # the golden holds the reference's waveform at these positions
+    assert max_abs(got, ref) <= TOL["bf16x3"]["max_abs"]
+    assert snr_db(ref, got) >= TOL["bf16x3"]["snr"]
     one, _ = m.inverse(z[37:38].cuda() * sigma, mel[37:38].cuda(), return_CPU=True)
     assert torch.equal(one[0], out[37])
 

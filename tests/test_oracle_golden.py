@@ -81,7 +81,8 @@ def test_oracle_port_matches_reference_at_config2_length():
     from tests.helpers import load_golden_regen
     cfg, sd, g, mel, z = load_golden_regen("config2_1x861")
     out = TorchPort(sd, cfg, torch.float32).infer(mel, z, float(g["sigma"]))
-    assert out.shape == g["audio_ref_fp64"].shape
+    assert out.shape == (1, int(g["n_samples"]))
+    out = out[:, g["sample_idx"]]                     # the golden holds the reference's waveform at these positions
     assert max_abs(out, g["audio_ref_fp64"]) < 5e-5
     assert max_abs(out, g["audio_ref_fp32"]) < 5e-5
     assert snr_db(g["audio_ref_fp64"], out) > 100.0
