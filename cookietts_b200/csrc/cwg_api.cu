@@ -93,27 +93,10 @@ void carve(const Dims& d, int mode, void* base, Workspace* ws) {
   ws->bytes = off;
 }
 
-// C = 256: the persistent sweep kernel (cwg_ps.cu) unless CWG_LAYER_PS=0 asks for the round-1 one-tile-per-CTA kernel
-int g_force_ps = -1;     // cwg_debug_set_layer_kernel: -1 = environment / default, 0 = round-1 kernel, 1 = persistent kernel
-// layer-0 fold (start conv folded into in_layers.0) unless CWG_FUSE_START=0
-bool use_fold() {
-  static const int v = [] { const char* e = getenv("CWG_FUSE_START"); return e ? (e[0] != '0') : 1; }();
-  return v != 0;
-}
-bool use_ps() {
-  static const int v = [] { const char* e = getenv("CWG_LAYER_PS"); return e ? (e[0] != '0') : 1; }();
-  return g_force_ps >= 0 ? g_force_ps != 0 : v != 0;
-}
-
-int layer_tc256(const Dims& d, const cwg_weights* w, int npass, int k, int i, const __nv_bfloat16* x_in,
-                __nv_bfloat16* x_out, const __nv_bfloat16* h2, float* eo, cudaStream_t s) {
-  if (use_ps()) return launch_layer_ps(d, w, npass, k, i, x_in, x_out, h2, eo, s);
-  return launch_layer_tc(d, w, npass, k, i, x_in, x_out, h2, eo, s);
-}
-
-// classic model, tensor-core modes: is layer 0 run from the (audio_0 | 1) planes instead of a materialised x_0 ?
+// tensor-core modes: is layer 0 run from the (audio_0 | 1) planes instead of a materialised x_0 (the start conv folded
+// into in_layers.0)?
 bool fold_active(const Dims& d, const cwg_weights* w) {
-  return d.C == 256 && d.L >= 2 && d.MG == 16 && w->w0_hi && w->w0_lo && use_ps() && use_fold();
+  return d.C == 256 && d.L >= 2 && d.MG == 16 && w->w0_hi && w->w0_lo;
 }
 
 int layer_tc(const cwg_config* cfg, const Dims& d, const cwg_weights* w, int npass, int k, int i, const Workspace& ws,
@@ -125,7 +108,7 @@ int layer_tc(const cwg_config* cfg, const Dims& d, const cwg_weights* w, int npa
     flow_channels(cfg, k, &n_rem, &n_half);
     return launch_layer_ps(d, w, npass, k, i, ws.xb[0], ws.xb[1], ws.h2b, ws.eo, s, ws.a0, audio, d.G - n_rem, n_half);
   }
-  return layer_tc256(d, w, npass, k, i, ws.xb[i & 1], ws.xb[(i + 1) & 1], ws.h2b, ws.eo, s);
+  return launch_layer_ps(d, w, npass, k, i, ws.xb[i & 1], ws.xb[(i + 1) & 1], ws.h2b, ws.eo, s);
 }
 
 int check_run(const cwg_config* cfg, const cwg_weights* w, int mode, int batch, int t_mel) {
@@ -172,10 +155,8 @@ extern "C" {
 
 int cwg_abi_version(void) { return CWG_ABI_VERSION; }
 
-// Debug only (not in cwg.h): the WN layer kernel writes 16 clock64 stamps per CTA into `buf`.
-void cwg_debug_set_timing(void* buf) { cwg::debug_set_timing((long long*)buf); }
-// Debug only: the persistent layer kernel writes {start, end, tiles, -} clock64 stamps per CTA (4 x int64 each).
-void cwg_debug_set_layer_kernel(int which) { cwg::g_force_ps = which; }
+// Debug only (not in cwg.h): the persistent layer kernel writes {start, end, tiles, -} clock64 stamps per CTA (4 x int64
+// each) into `buf`.
 void cwg_debug_set_ps_timing(void* buf) { cwg::debug_set_ps_timing((long long*)buf); }
 
 // Debug only: layer 0 of `flow` through the layer-0 fold (a0 planes built from `audio`, then the fused persistent kernel);
@@ -256,8 +237,8 @@ int cwg_wn_layer(const cwg_config* cfg, const cwg_weights* w, int mode, int flow
     return launch_layer_tc512(d, w, mode_npass(mode), flow, layer, (const __nv_bfloat16*)x_in,
                               (__nv_bfloat16*)x_out, (const __nv_bfloat16*)h2, ws.actsb, eo, s);
   }
-  return layer_tc256(d, w, mode_npass(mode), flow, layer, (const __nv_bfloat16*)x_in,
-                     (__nv_bfloat16*)x_out, (const __nv_bfloat16*)h2, eo, s);
+  return launch_layer_ps(d, w, mode_npass(mode), flow, layer, (const __nv_bfloat16*)x_in,
+                         (__nv_bfloat16*)x_out, (const __nv_bfloat16*)h2, eo, s);
 }
 
 int cwg_flow_boundary(const cwg_config* cfg, const cwg_weights* w, int mode,
@@ -396,7 +377,6 @@ int cwg_ax_infer(const cwg_config* cfg, const cwg_weights* w, int mode,
   CWG_REQUIRE(ws.bytes <= workspace_bytes, "workspace too small: need %zu, got %zu", ws.bytes, workspace_bytes);
   cudaStream_t s = (cudaStream_t)cuda_stream;
   const bool tc = mode != CWG_MODE_FFMA;
-  CWG_REQUIRE(!tc || use_ps() || (d.MG == 16 && !b1_batch), "n_group > 16 / per-utterance gate biases need the persistent layer kernel");
   const int npass = mode_npass(mode);
   const int xfmt = mode_xfmt(mode);
   const int F = cfg->n_flows, L = cfg->n_layers;

@@ -119,15 +119,11 @@ int launch_mel_up(int xfmt, const float* mel, void* out, int B, int M, int frame
                   int linear, cudaStream_t s);
 
 // ---- launchers implemented in cwg_tc.cu (tcgen05 / TMA path) ----
-void debug_set_timing(long long* buf);
 int launch_cond_tc(const Dims& d, const cwg_weights* w, int npass, int flow, const float* mel,
                    const float* cond_bias, __nv_bfloat16* h2_planes, __nv_bfloat16* mel4_planes,
                    cudaStream_t s);
-int launch_layer_tc(const Dims& d, const cwg_weights* w, int npass, int flow, int layer,
-                    const __nv_bfloat16* x_in, __nv_bfloat16* x_out, const __nv_bfloat16* h2,
-                    float* eo, cudaStream_t s);
 
-// persistent, epilogue-overlapped successor of launch_layer_tc for n_channels = 256 (cwg_ps.cu); the default
+// n_channels = 256: one persistent, epilogue-overlapped kernel per WN layer (cwg_ps.cu)
 int launch_layer_ps(const Dims& d, const cwg_weights* w, int npass, int flow, int layer,
                     const __nv_bfloat16* x_in, __nv_bfloat16* x_out, const __nv_bfloat16* h2,
                     float* eo, cudaStream_t s, const void* a0 = nullptr, const float* audio = nullptr,

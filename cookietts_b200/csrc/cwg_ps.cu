@@ -1,8 +1,7 @@
-// Persistent, epilogue-overlapped WN layer kernel (glow.py:201-220) for C = 256: the round-2 successor of
-// k_layer_tc<NPASS, TWO=true> (cwg_tc.cu), same math, same operand planes, same packed weights.
+// Persistent, epilogue-overlapped WN layer kernel (glow.py:201-220) for C = 256.
 //
-// Why: in k_layer_tc one tile's [128 x 512] fp32 pre-activation fills tensor memory, so the gate, the res/skip epilogue,
-// the stores and the per-tile prologue all run with the tensor pipe stopped (ncu r1e: 52 % active in f16f8).  Here
+// Why: when one tile's [128 x 512] fp32 pre-activation fills tensor memory, the gate, the res/skip epilogue, the stores
+// and the per-tile prologue all run with the tensor pipe stopped (ncu r1e: 52 % active in f16f8).  Here
 //   * a CTA PAIR (cta_group::2, M = 256) is persistent and loops over tile pairs: TMEM, barriers, biases and the
 //     folded-`end` weight tiles are set up once per CTA;
 //   * GEMM1 runs as two N = 256 SWEEPS over K.  Sweep g computes the tanh AND the sigmoid rows of channels

@@ -1,6 +1,6 @@
 // CUDA-core (fp32 FFMA) kernels of the WaveGlow inverse pass, plus the flow-boundary kernel
 // that both arithmetic modes share.  This path keeps exact fp32 semantics (CWG_MODE_FFMA) and
-// doubles as the on-device cross-check for the tcgen05 path in cwg_tc.cu.
+// doubles as the on-device cross-check for the tcgen05 path (cwg_tc.cu, cwg_ps.cu, cwg_tc512.cu).
 //
 // Reference lines implemented (CookieTTS/_4_mtw/waveglow/glow.py):
 //   cond GEMM        : upsample + squeeze + cond_layers[0..1]  :318-324, :198-199 (folded, see packing.py)

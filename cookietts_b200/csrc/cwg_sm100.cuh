@@ -124,22 +124,6 @@ __host__ __device__ constexpr uint32_t umma_idesc_f16(int m, int n) {
 __host__ __device__ constexpr uint32_t umma_idesc_e5m2(int m, int n) {
   return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(m >> 4) << 24);
 }
-__device__ __forceinline__ void umma_f8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-// Same with the A operand read from tensor memory ([M lanes] x [K/2 32-bit columns], two bf16 per column, the
-// even-k element in the low half): the ".ts" form.
-__device__ __forceinline__ void umma_bf16_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
 // 8 x 32-bit columns of this thread's TMEM lane (warp w may only touch lanes 32*(w%4) .. +31).
 __device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint32_t* r) {
   asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
@@ -197,6 +181,8 @@ __device__ __forceinline__ void tma_load_3d_2sm(void* smem_dst, const CUtensorMa
       ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(bar_cluster_addr), "r"(c0), "r"(c1), "r"(c2)
       : "memory");
 }
+// A operand read from tensor memory ([M lanes] x [K/2 32-bit columns], two bf16 per column, the even-k element in the
+// low half): the ".ts" form.
 __device__ __forceinline__ void umma_bf16_ts_2sm(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
   asm volatile(
       "{\n\t.reg .pred p;\n\t"

@@ -3,9 +3,6 @@
 //
 //   k_cond_tc   : folded upsample+squeeze+cond_layers[0..1] GEMM (glow.py:318-324,198-199)
 //                 H2[b, f*P+p, :] = mel4[b, f, :] @ cond_w[p*H:(p+1)*H, :]^T + bias
-//   k_layer_tc  : one WN layer (glow.py:201-220): dilated conv + cond_layers[2] slice as ONE
-//                 implicit GEMM (K = 3C + H), tanh*sigmoid gate in the TMEM epilogue, res_skip
-//                 GEMM from shared memory, residual update (TMA store) and folded-`end` skip sum.
 //
 // Operand precision: every fp32 quantity q that feeds an MMA is stored as two bf16 planes,
 // q ~= hi + lo.  NPASS = 1 issues hi*hi only (CWG_MODE_BF16); NPASS = 3 issues
@@ -181,711 +178,7 @@ k_cond_tc(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ C
   if (warp == 1) { __syncwarp(); tmem_dealloc(tmem, 256); }
 }
 
-// ------------------------------------------------------------------------------------------
-// cond GEMM as a 2-SM MMA (cta_group::2): a CTA pair computes 256 rows x 256 columns; each CTA stages its own A tile
-// and HALF of the weight tile, so the weight bytes every SM pulls through L2 halve.  Opt-in (CWG_COND_2SM=1): the
-// recipe the WN layer kernel needs next (DESIGN "Known limits" 1), validated here on the simplest GEMM of the path.
-// ------------------------------------------------------------------------------------------
-template <int NPASS>
-struct Cond2Cfg {
-  static constexpr int PL = NPASS != 1 ? 2 : 1;
-  static constexpr int STAGE = 2 * TILE_A * PL;                // per CTA: A 16 KB + B half 16 KB per plane
-  static constexpr int NST = 2;
-  static constexpr int STAGING = 4 * TILE_A;                   // epilogue staging, 128 columns at a time (64 KB)
-  static constexpr int SMEM = (NST * STAGE > STAGING ? NST * STAGE : STAGING) + 256 + 1024;
-};
-
-template <int NPASS>
-__global__ void __launch_bounds__(192, 1)
-k_cond_tc2(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ CUtensorMap tm_a_lo,
-           const __grid_constant__ CUtensorMap tm_b_hi, const __grid_constant__ CUtensorMap tm_b_lo,   // 128-row boxes
-           const __grid_constant__ CUtensorMap tm_c_hi, const __grid_constant__ CUtensorMap tm_c_lo,
-           const __grid_constant__ CUtensorMap tm_c_h8, CondArgs a) {
-  using Cfg = Cond2Cfg<NPASS>;
-  constexpr bool F8 = NPASS == 2;
-  constexpr uint32_t ID = F8 ? umma_idesc_f16(256, 256) : umma_idesc_bf16(256, 256);
-  constexpr int PIPE = Cfg::NST * Cfg::STAGE > Cfg::STAGING ? Cfg::NST * Cfg::STAGE : Cfg::STAGING;
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = align_1024(smem_raw);
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + PIPE);
-  uint64_t* empty = full + Cfg::NST;
-  uint64_t* acc_full = empty + Cfg::NST;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_full + 1);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();                      // 0 = leader (issues the MMAs), 1 = follower
-  const int p = blockIdx.y, m0 = blockIdx.x * 128;              // the pair = two neighbouring row tiles (cluster along x)
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < Cfg::NST; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-    mbar_init(acc_full, 1);
-    fence_barrier_init();
-  }
-  if (warp == 1) tmem_alloc_2sm(tmem_slot, 256);
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();                                           // both CTAs' barriers and TMEM exist
-  tc_fence_after_sync();
-  const uint32_t tmem = *tmem_slot;
-
-  if (warp == 0 && lane == 0) {
-    // each CTA loads its own A rows and its half of the weight rows; all bytes are counted on the LEADER's barrier
-    tma_prefetch_desc(&tm_a_hi); tma_prefetch_desc(&tm_b_hi);
-    int s = 0; uint32_t ph = 0;
-    for (int kb = 0; kb < a.nkb; ++kb) {
-      mbar_wait(&empty[s], ph ^ 1u);
-      uint8_t* st = smem + s * Cfg::STAGE;
-      const uint32_t lbar = mapa_shared(&full[s], 0);
-      if (rank == 0) mbar_arrive_expect_tx(&full[s], 2 * Cfg::STAGE);
-      tma_load_2d_2sm(st, &tm_a_hi, lbar, kb * 64, m0);
-      tma_load_2d_2sm(st + TILE_A, &tm_b_hi, lbar, kb * 64, a.w_row0 + p * 256 + (int)rank * 128);
-      if (NPASS != 1) {
-        tma_load_2d_2sm(st + 2 * TILE_A, &tm_a_lo, lbar, kb * 64, m0);
-        tma_load_2d_2sm(st + 3 * TILE_A, &tm_b_lo, lbar, kb * 64, a.w_row0 + p * 256 + (int)rank * 128);
-      }
-      ring_advance(s, ph, Cfg::NST);
-    }
-  } else if (warp == 1 && lane == 0 && rank == 0) {
-    int s = 0; uint32_t ph = 0;
-    auto kblock = [&](uint32_t a_addr, uint32_t b_addr, bool first) {
-#pragma unroll
-      for (int k = 0; k < 4; ++k)
-        umma_bf16_2sm(tmem, umma_desc_sw128(a_addr + 32 * k), umma_desc_sw128(b_addr + 32 * k), ID, (first && k == 0) ? 0u : 1u);
-    };
-    for (int kb = 0; kb < a.nkb; ++kb) {
-      mbar_wait(&full[s], ph);
-      tc_fence_after_sync();
-      const uint32_t st = smem_u32(smem + s * Cfg::STAGE);
-      kblock(st, st + TILE_A, kb == 0);
-      if (NPASS != 1) {
-        kblock(st + 2 * TILE_A, st + TILE_A, false);             // lo * hi
-        kblock(st, st + 3 * TILE_A, false);                      // hi * lo
-      }
-      umma_commit_2sm(&empty[s]);
-      ring_advance(s, ph, Cfg::NST);
-    }
-    umma_commit_2sm(acc_full);
-  } else if (warp >= 2) {
-    const int quarter = warp & 3, row = quarter * 32 + lane;
-    const uint32_t trow = tmem + ((uint32_t)(quarter * 32) << 16);
-    int m = m0 + row;
-    int b = min(m / a.Tm, a.B - 1);
-    const float4* bias4 = reinterpret_cast<const float4*>(a.bias + (size_t)b * a.bias_bstride);
-    mbar_wait(acc_full, 0);
-    tc_fence_after_sync();
-#pragma unroll 1
-    for (int half = 0; half < 2; ++half) {
-#pragma unroll 1
-      for (int c = 8 * half; c < 8 * half + 8; ++c) {
-        float v[16];
-        tmem_ld16_sync(trow + c * 16, v);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          float4 bb = __ldg(bias4 + c * 4 + q);
-          v[4 * q] += bb.x; v[4 * q + 1] += bb.y; v[4 * q + 2] += bb.z; v[4 * q + 3] += bb.w;
-        }
-        if (F8 && a.range_flag) {
-          float mx = 0.f;
-#pragma unroll
-          for (int q = 0; q < 16; ++q) mx = fmaxf(mx, fabsf(v[q]));
-          if (!(mx < 65504.f)) atomicOr(a.range_flag, 2);
-        }
-        uint8_t* thi = smem + ((c >> 2) & 1) * TILE_A;
-        if (F8) store_split16_f8(v, thi, nullptr, smem + 2 * TILE_A, smem + 3 * TILE_A, row, (c & 3) * 2, c & 7);
-        else store_split16<NPASS == 3>(v, thi, thi + 2 * TILE_A, row, (c & 3) * 2);
-      }
-      tc_fence_before_sync();
-      fence_proxy_async_smem();
-      asm volatile("bar.sync 1, 128;" ::: "memory");
-      if (warp == 2 && lane == 0) {
-        for (int j = 0; j < 2; ++j) {
-          tma_store_2d(&tm_c_hi, smem + j * TILE_A, p * 256 + (2 * half + j) * 64, m0);
-          if (NPASS == 3) tma_store_2d(&tm_c_lo, smem + (2 + j) * TILE_A, p * 256 + (2 * half + j) * 64, m0);
-        }
-        if (F8) {
-          tma_store_2d(&tm_c_lo, smem + 2 * TILE_A, p * 256 + half * 128, m0);
-          tma_store_2d(&tm_c_h8, smem + 3 * TILE_A, p * 256 + half * 128, m0);
-        }
-        tma_store_commit();
-        tma_store_wait_read();
-      }
-      asm volatile("bar.sync 1, 128;" ::: "memory");
-    }
-    if (warp == 2 && lane == 0) tma_store_wait_all();
-  }
-  tc_fence_before_sync();
-  __syncthreads();
-  cluster_sync_all();                                           // the pair releases TMEM together
-  if (warp == 1) { __syncwarp(); tmem_dealloc_2sm(tmem, 256); }
-}
-
-// ------------------------------------------------------------------------------------------
-// WN layer
-// ------------------------------------------------------------------------------------------
-struct LayerArgs {
-  const float* b1;        // [2C]
-  const float* b2;        // [C]
-  const float* eo_b;      // [16]
-  float* eo;              // [B*T'][16]
-  const __nv_bfloat16* x_hi;   // x_in planes (residual read)
-  const __nv_bfloat16* x_lo;
-  int Tp, dil;
-  int w1_row0, w2_row0;
-  int has_res, first;
-  long long* dbg;         // optional per-CTA clock64 stamps (cwg_debug_set_timing), 16 per CTA
-};
-
-long long* g_dbg_timing = nullptr;
-
-// Shared memory: a pool of twelve 16-KB units.
-//   GEMM1: activation (A) tiles [128 x 64] cycle through units 0..3; weight (B) tiles
-//          [256 rows x 64] = 32 KB cycle through the four unit pairs 4..11 (one N=256 MMA group each).
-//   gate : acts hi -> TENSOR MEMORY (bf16 pairs in the accumulator columns the gate has already consumed: channel
-//          chunk c of 16 at columns L_ACOL(c)), so GEMM2 reads its A operand from TMEM (".ts" MMA: the N=16
-//          folded-`end` MMAs are then no longer bound by the shared-memory A read); acts lo (bf16x3 only) ->
-//          units 4..7 (GEMM1 is complete by then).
-//   TMEM : GEMM1 accumulators in columns 0..511 (tanh half 0..255, sigmoid half 256..511); after the gate, acts hi
-//          in 0..63 and 128..191, GEMM2 res accumulator in 256..511, folded-`end` accumulator in 64..79.
-//   GEMM2: W2 res tiles [256 x 64] cycle through unit pairs (8,9) and (10,11); epilogue-2 stages
-//          x_new hi/lo in units 0..7.
-// Every tile slot has its own full/empty mbarrier pair and its own phase bit (kept in a bit mask
-// by the producer and by the consumer), so the slot sequences above need no common ring modulus.
-// Barrier index: A slot i -> i (0..3); B slot j -> 4 + j (j = 0..3, units 4+2j, 5+2j).
-constexpr int L_NS = 12, L_NA = 4, L_NBAR = 8;
-constexpr int L_OFF_WSE = L_NS * TILE_A;               // 196608
-constexpr int L_OFF_B1 = L_OFF_WSE + 16384;            // 212992
-constexpr int L_OFF_B2 = L_OFF_B1 + 2048;              // 215040
-constexpr int L_OFF_BAR = L_OFF_B2 + 1024;             // 216064
-constexpr int L_SMEM = L_OFF_BAR + 256 + 1024;         // 217344
-constexpr int L_EPI_WARPS = 8;                         // 2 per TMEM lane quarter, each owns 128 channels (16 warps measured no faster)
-constexpr int L_EPI_THREADS = 32 * L_EPI_WARPS;
-constexpr int L_THREADS = 128 + L_EPI_THREADS;         // warps 0-3: TMA-A, MMA, TMA-B, residual prefetch
-constexpr int L_CPG = 16 / (L_EPI_WARPS / 4);          // 16-channel chunks per epilogue column group
-constexpr uint32_t L_D2_RES = 256, L_D2_EO = 64;       // TMEM columns of the GEMM2 accumulators
-static_assert(L_CPG == 8, "f16f8 stages one 128-channel e5m2 tile per epilogue column group");
-// The N=16 folded-`end` MMAs cost ~110 cycles each - as much as an N=256 one.  Measured NOT to be the cause: the
-// shared-memory A read (A from TMEM: GEMM2 11.9 k instead of 13.0 k cycles in bf16x3, same in bf16) and the
-// accumulate dependency on the same 16 columns (L_EO_CHAINS = 4 independent accumulators summed in the epilogue:
-// no change).  L_EO_CHAINS is kept as a build-time experiment knob.
-#ifndef CWG_EO_CHAINS
-#define CWG_EO_CHAINS 1
-#endif
-constexpr int L_EO_CHAINS = CWG_EO_CHAINS;
-#ifndef CWG_ACTS_TMEM
-#define CWG_ACTS_TMEM 1
-#endif
-constexpr bool L_ACTS_TMEM = CWG_ACTS_TMEM != 0;
-// TMEM column of the packed bf16 acts of 16-channel chunk c: each column group writes behind its own read pointer
-__device__ __forceinline__ uint32_t L_ACOL(int c) { return (uint32_t)((c / L_CPG) * (16 * L_CPG) + (c % L_CPG) * 8); }
-
-template <int NPASS, bool TWO>
-__global__ void __launch_bounds__(L_THREADS, 1)
-k_layer_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ CUtensorMap tm_x_lo,
-           const __grid_constant__ CUtensorMap tm_h_hi, const __grid_constant__ CUtensorMap tm_h_lo,
-           const __grid_constant__ CUtensorMap tm_w1_hi, const __grid_constant__ CUtensorMap tm_w1_lo,
-           const __grid_constant__ CUtensorMap tm_w2_hi, const __grid_constant__ CUtensorMap tm_w2_lo,
-           const __grid_constant__ CUtensorMap tm_wse_hi, const __grid_constant__ CUtensorMap tm_wse_lo,
-           const __grid_constant__ CUtensorMap tm_xo_hi, const __grid_constant__ CUtensorMap tm_xo_lo,
-           // e5m2 planes, NPASS == 2 (CWG_MODE_F16F8) only: activations lo*2^P / hi*2^-Q, w1 hi*2^-P / lo*2^Q, x output
-           const __grid_constant__ CUtensorMap tm_x_l8, const __grid_constant__ CUtensorMap tm_x_h8,
-           const __grid_constant__ CUtensorMap tm_h_l8, const __grid_constant__ CUtensorMap tm_h_h8,
-           const __grid_constant__ CUtensorMap tm_w1_h8, const __grid_constant__ CUtensorMap tm_w1_l8,
-           const __grid_constant__ CUtensorMap tm_xo_l8, const __grid_constant__ CUtensorMap tm_xo_h8,
-           // f16f8: tm_w2_lo / tm_wse_lo are the e5m2 hi*2^-P planes of w2 (boxes of 256 / 16 rows), these the lo*2^Q ones
-           const __grid_constant__ CUtensorMap tm_w2_l8, const __grid_constant__ CUtensorMap tm_wse_l8, LayerArgs a) {
-  // NPASS: 1 = bf16 (hi planes only), 3 = bf16x3 (hi/lo bf16 planes, 3 MMAs), 2 = f16f8: fp16 hi/lo planes, GEMM1 =
-  // one fp16 pass + two e5m2 correction passes over K-blocks of 128 (same 16-KB tiles), GEMM2 = three fp16 passes.
-  constexpr bool F8 = NPASS == 2;
-  constexpr bool X3 = NPASS != 1;                 // lo planes exist (residual, GEMM2 cross terms)
-  constexpr int PL = NPASS == 3 ? 2 : 1;          // planes streamed per k-block in GEMM1 of the bf16 modes
-  constexpr int PL2 = X3 ? 2 : 1;                 // planes of the GEMM2 operands
-  // TWO: 2-SM MMAs (cta_group::2).  Two neighbouring tiles of one utterance form a CTA pair (cluster ranks 0 / 1); the
-  // leader issues every MMA with M = 256, each CTA supplies its own 128 rows of A and HALF of the N rows of every
-  // weight tile (16 KB instead of 32 KB per slot), all TMA completions are counted on the leader's barriers, slots and
-  // accumulators are released / published in both CTAs by multicast commits.
-  // The folded-`end` MMAs are N = 16; the 2-SM A-from-TMEM form needs N >= 32, so there N = 32: the leader stages the 16
-  // real rows, the follower the 16 rows that follow them in w2 (the next layer's first res rows, or TMA zero fill) - they
-  // only produce accumulator columns 16..31, which nobody reads.
-  constexpr int MM = TWO ? 256 : 128, NEO = TWO ? 32 : 16;
-  constexpr uint32_t ID256 = F8 ? umma_idesc_f16(MM, 256) : umma_idesc_bf16(MM, 256), ID16 = F8 ? umma_idesc_f16(MM, NEO) : umma_idesc_bf16(MM, NEO);
-  constexpr uint32_t IDF256 = umma_idesc_f16(MM, 256), IDF16 = umma_idesc_f16(MM, NEO);
-  constexpr uint32_t IDE256 = umma_idesc_e5m2(MM, 256), IDE16 = umma_idesc_e5m2(MM, NEO);
-  // shared-memory unit of the lo tile of 64-channel block kb of x (residual read / x_new staging).  f16f8: units 4..7
-  // hold the e5m2 acts tiles of the two 128-channel groups during GEMM2 (4 + g: lo*2^P, 6 + g: hi*2^-Q), and group g
-  // frees units 4 + g and 6 + g, so blocks 0, 1 (needed first) take units 4, 6 and blocks 2, 3 take 5, 7.
-  auto lo_unit = [](int kb) { return F8 ? 4 + ((kb & 1) << 1) + (kb >> 1) : 4 + kb; };
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = align_1024(smem_raw);
-  float* b1s = reinterpret_cast<float*>(smem + L_OFF_B1);
-  float* b2s = reinterpret_cast<float*>(smem + L_OFF_B2);
-  uint64_t* full = reinterpret_cast<uint64_t*>(smem + L_OFF_BAR);
-  uint64_t* empty = full + L_NBAR;
-  uint64_t* wse_full = empty + L_NBAR;
-  uint64_t* acc1_full = wse_full + 1;
-  uint64_t* acts_ready = acc1_full + 1;
-  uint64_t* acc2_full = acts_ready + 1;
-  uint64_t* xold_full = acc2_full + 1;      // [4]: x_old tiles of 64-channel block kb have landed
-  uint64_t* g2_done = xold_full + 4;        // [4]: GEMM2 no longer reads the acts tiles of block kb
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(g2_done + 4);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int t0 = blockIdx.x * 128, b = blockIdx.y;
-  auto slot = [&](int i) { return smem + i * TILE_A; };                 // 16-KB unit i
-  auto bslot = [&](int j) { return smem + (L_NA + 2 * j) * TILE_A; };   // 32-KB weight slot j (barrier 4 + j)
-  auto wse = [&](int plane, int kb) { return smem + L_OFF_WSE + plane * 8192 + kb * 2048; };
-
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < L_NBAR; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-    mbar_init(wse_full, 1); mbar_init(acc1_full, 1); mbar_init(acts_ready, (TWO ? 2 : 1) * L_EPI_THREADS); mbar_init(acc2_full, 1);
-    for (int i = 0; i < 4; ++i) { mbar_init(&xold_full[i], 1); mbar_init(&g2_done[i], 1); }
-    fence_barrier_init();
-  }
-  if (warp == 1) { if (TWO) tmem_alloc_2sm(tmem_slot, 512); else tmem_alloc(tmem_slot, 512); }
-  tc_fence_before_sync();
-  __syncthreads();
-  if (TWO) cluster_sync_all();                     // both CTAs' barriers and TMEM exist before anything targets them
-  tc_fence_after_sync();
-  const uint32_t tmem = *tmem_slot;
-  const uint32_t rank = TWO ? cluster_ctarank() : 0u;
-  const bool leader = rank == 0;
-  // pipeline helpers: in 2-SM mode loads complete on the leader's barrier (armed by the leader for both CTAs' bytes)
-  auto arm = [&](uint64_t* bar, uint32_t bytes) {
-    if (!TWO) mbar_arrive_expect_tx(bar, bytes); else if (leader) mbar_arrive_expect_tx(bar, 2 * bytes);
-  };
-  auto lda3 = [&](void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1, int c2) {
-    if (TWO) tma_load_3d_2sm(dst, m, mapa_shared(bar, 0), c0, c1, c2); else tma_load_3d(dst, m, bar, c0, c1, c2);
-  };
-  auto ldb2 = [&](void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int row, int half_rows) {
-    if (TWO) tma_load_2d_2sm(dst, m, mapa_shared(bar, 0), c0, row + (int)rank * half_rows); else tma_load_2d(dst, m, bar, c0, row);
-  };
-  auto commit = [&](uint64_t* bar) { if (TWO) umma_commit_2sm(bar); else umma_commit(bar); };
-  auto mma_ss = [&](uint32_t d, uint64_t ad, uint64_t bd, uint32_t id, uint32_t acc) { if (TWO) umma_bf16_2sm(d, ad, bd, id, acc); else umma_bf16(d, ad, bd, id, acc); };
-  auto mma_ts = [&](uint32_t d, uint32_t at, uint64_t bd, uint32_t id, uint32_t acc) { if (TWO) umma_bf16_ts_2sm(d, at, bd, id, acc); else umma_bf16_ts(d, at, bd, id, acc); };
-  auto mma_f8 = [&](uint32_t d, uint64_t ad, uint64_t bd, uint32_t id, uint32_t acc) { if (TWO) umma_f8_2sm(d, ad, bd, id, acc); else umma_f8(d, ad, bd, id, acc); };
-  auto kblk = [&](uint32_t a_addr, uint32_t b_addr, uint32_t d, uint32_t id, bool first) {
-    const uint64_t da = DESC_SW128_HI | (uint64_t)((a_addr & 0x3FFFF) >> 4), db = DESC_SW128_HI | (uint64_t)((b_addr & 0x3FFFF) >> 4);
-    mma_ss(d, da, db, id, first ? 0u : 1u); mma_ss(d, da + 2, db + 2, id, 1u); mma_ss(d, da + 4, db + 4, id, 1u); mma_ss(d, da + 6, db + 6, id, 1u);
-  };
-  auto kblk8 = [&](uint32_t a_addr, uint32_t b_addr, uint32_t d, uint32_t id) {
-    const uint64_t da = DESC_SW128_HI | (uint64_t)((a_addr & 0x3FFFF) >> 4), db = DESC_SW128_HI | (uint64_t)((b_addr & 0x3FFFF) >> 4);
-    mma_f8(d, da, db, id, 1u); mma_f8(d, da + 2, db + 2, id, 1u); mma_f8(d, da + 4, db + 4, id, 1u); mma_f8(d, da + 6, db + 6, id, 1u);
-  };
-  long long* dbg = a.dbg ? a.dbg + ((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 16 : nullptr;
-#define CWG_STAMP(i) do { if (dbg) dbg[i] = clock64(); } while (0)
-
-  if (warp == 0 && lane == 0) {
-    // ---------------- producer A: activation tiles (3 dilated taps of x, then the cond hidden H2)
-    tma_prefetch_desc(&tm_x_hi); tma_prefetch_desc(&tm_h_hi);
-    int s = 0; uint32_t pm = 0;
-    if (F8) {
-      // K in groups of 128 channels (taps 0..2 of x: groups 0..5, H2: groups 6, 7); per group two fp16 tiles of 64
-      // channels, then the e5m2 tile of lo*2^P and the e5m2 tile of hi*2^-Q (128 channels = 128 bytes per row)
-      tma_prefetch_desc(&tm_x_l8); tma_prefetch_desc(&tm_x_h8);
-      for (int G = 0; G < 8; ++G)
-        for (int it = 0; it < 4; ++it) {
-          mbar_wait(&empty[s], ((pm >> s) & 1u) ^ 1u);
-          pm ^= 1u << s;
-          arm(&full[s], TILE_A);
-          const bool cond = G >= 6;
-          const int tt = cond ? t0 : t0 + ((G >> 1) - 1) * a.dil;
-          const int c0 = (cond ? G - 6 : (G & 1)) * 128;
-          if (it < 2) lda3(slot(s), cond ? &tm_h_hi : &tm_x_hi, &full[s], c0 + it * 64, tt, b);
-          else if (it == 2) lda3(slot(s), cond ? &tm_h_l8 : &tm_x_l8, &full[s], c0, tt, b);
-          else lda3(slot(s), cond ? &tm_h_h8 : &tm_x_h8, &full[s], c0, tt, b);
-          s = (s + 1 == L_NA) ? 0 : s + 1;
-        }
-    }
-    for (int kb = 0; kb < (F8 ? 0 : 16); ++kb) {
-      for (int pl = 0; pl < PL; ++pl) {
-        mbar_wait(&empty[s], ((pm >> s) & 1u) ^ 1u);
-        pm ^= 1u << s;
-        arm(&full[s], TILE_A);
-        if (kb < 12) {
-          int tap = kb >> 2, cb = kb & 3;
-          lda3(slot(s), pl ? &tm_x_lo : &tm_x_hi, &full[s], cb * 64, t0 + (tap - 1) * a.dil, b);
-        } else {
-          lda3(slot(s), pl ? &tm_h_lo : &tm_h_hi, &full[s], (kb - 12) * 64, t0, b);
-        }
-        s = (s + 1 == L_NA) ? 0 : s + 1;
-      }
-    }
-  } else if (warp == 2 && lane == 0) {
-    // ---------------- producer B: weight tiles [256 rows x 64 k]
-    tma_prefetch_desc(&tm_w1_hi); tma_prefetch_desc(&tm_w2_hi);
-    int j = 0; uint32_t pm = 0;
-    if (F8) {
-      tma_prefetch_desc(&tm_w1_h8); tma_prefetch_desc(&tm_w1_l8);
-      for (int G = 0; G < 8; ++G)
-        for (int it = 0; it < 4; ++it)
-          for (int g = 0; g < 2; ++g) {
-            mbar_wait(&empty[4 + j], ((pm >> j) & 1u) ^ 1u);
-            pm ^= 1u << j;
-            arm(&full[4 + j], TWO ? TILE_A : 2 * TILE_A);
-            if (it < 2) ldb2(bslot(j), &tm_w1_hi, &full[4 + j], (2 * G + it) * 64, a.w1_row0 + g * 256, 128);
-            else ldb2(bslot(j), it == 2 ? &tm_w1_h8 : &tm_w1_l8, &full[4 + j], G * 128, a.w1_row0 + g * 256, 128);
-            j = (j + 1) & 3;
-          }
-    }
-    for (int kb = 0; kb < (F8 ? 0 : 16); ++kb)
-      for (int g = 0; g < 2; ++g)
-        for (int pl = 0; pl < PL; ++pl) {
-          mbar_wait(&empty[4 + j], ((pm >> j) & 1u) ^ 1u);
-          pm ^= 1u << j;
-          arm(&full[4 + j], TWO ? TILE_A : 2 * TILE_A);
-          ldb2(bslot(j), pl ? &tm_w1_lo : &tm_w1_hi, &full[4 + j], kb * 64, a.w1_row0 + g * 256, 128);
-          j = (j + 1) & 3;
-        }
-    if (a.has_res && F8) {
-      j = 2;
-      for (int grp = 0; grp < 2; ++grp)
-        for (int it = 0; it < 4; ++it) {          // two fp16 tiles, then the e5m2 hi*2^-P and lo*2^Q tiles of the group
-          mbar_wait(&empty[4 + j], ((pm >> j) & 1u) ^ 1u);
-          pm ^= 1u << j;
-          arm(&full[4 + j], TWO ? TILE_A : 2 * TILE_A);
-          if (it < 2) ldb2(bslot(j), &tm_w2_hi, &full[4 + j], (2 * grp + it) * 64, a.w2_row0, 128);
-          else ldb2(bslot(j), it == 2 ? &tm_w2_lo : &tm_w2_l8, &full[4 + j], grp * 128, a.w2_row0, 128);
-          j = j == 2 ? 3 : 2;
-        }
-    }
-    if (a.has_res && !F8) {
-      j = 2;
-      for (int kb = 0; kb < 4; ++kb)
-        for (int pl = 0; pl < PL2; ++pl) {
-          mbar_wait(&empty[4 + j], ((pm >> j) & 1u) ^ 1u);
-          pm ^= 1u << j;
-          arm(&full[4 + j], TWO ? TILE_A : 2 * TILE_A);
-          ldb2(bslot(j), pl ? &tm_w2_lo : &tm_w2_hi, &full[4 + j], kb * 64, a.w2_row0, 128);
-          j = j == 2 ? 3 : 2;
-        }
-    }
-  } else if (warp == 1 && lane == 0 && leader) {
-    // ---------------- MMA issuer (the leader CTA's thread in 2-SM mode)
-    int sa = 0, jb = 0; uint32_t cm = 0;
-    auto wait_full = [&](int bar) {               // bar: barrier index (A slot i -> i, B slot j -> 4 + j)
-      mbar_wait(&full[bar], (cm >> bar) & 1u);
-      cm ^= 1u << bar;
-    };
-    // GEMM1: pre[128 x 512] = [x taps | H2] (K = 1024) x W1^T, accumulators in TMEM columns 0..511
-    if (F8) {
-      for (int G = 0; G < 8; ++G)
-        for (int it = 0; it < 4; ++it) {
-          const int sa_cur = sa; wait_full(sa); sa = (sa + 1) & 3;
-          if (G == 0 && it == 0) CWG_STAMP(5);
-          for (int g = 0; g < 2; ++g) {
-            const int jb_cur = jb; wait_full(4 + jb); jb = (jb + 1) & 3;
-            tc_fence_after_sync();
-            const uint32_t d = tmem + g * 256;
-            if (it < 2) kblk(smem_u32(slot(sa_cur)), smem_u32(bslot(jb_cur)), d, IDF256, G == 0 && it == 0);
-            else kblk8(smem_u32(slot(sa_cur)), smem_u32(bslot(jb_cur)), d, IDE256);
-            commit(&empty[4 + jb_cur]);
-          }
-          commit(&empty[sa_cur]);
-        }
-    }
-    for (int kb = 0; kb < (F8 ? 0 : 16); ++kb) {
-      const int sa_hi = sa; wait_full(sa); sa = (sa + 1) & 3;
-      int sa_lo = 0;
-      if (NPASS == 3) { sa_lo = sa; wait_full(sa); sa = (sa + 1) & 3; }
-      if (kb == 0) CWG_STAMP(5);
-      for (int g = 0; g < 2; ++g) {
-        // Slots are waited for right before their first use and released right after their last one: with a B ring
-        // of one k-block (bf16x3) a weight slot must be refilled (~2 k cycles from free to full) inside the ~3 k
-        // cycles of MMA work of a k-block.
-        const int jb_hi = jb; wait_full(4 + jb); jb = (jb + 1) & 3;
-        tc_fence_after_sync();
-        const uint32_t d = tmem + g * 256;
-        kblk(smem_u32(slot(sa_hi)), smem_u32(bslot(jb_hi)), d, ID256, kb == 0);
-        if (NPASS == 3) {
-          kblk(smem_u32(slot(sa_lo)), smem_u32(bslot(jb_hi)), d, ID256, false);
-          commit(&empty[4 + jb_hi]);
-          if (g == 1) commit(&empty[sa_lo]);
-          const int jb_lo = jb; wait_full(4 + jb); jb = (jb + 1) & 3;
-          tc_fence_after_sync();
-          kblk(smem_u32(slot(sa_hi)), smem_u32(bslot(jb_lo)), d, ID256, false);
-          commit(&empty[4 + jb_lo]);
-        } else {
-          commit(&empty[4 + jb_hi]);
-        }
-      }
-      commit(&empty[sa_hi]);
-    }
-    commit(acc1_full);
-    CWG_STAMP(6);
-    // GEMM2: [res | folded end] = acts (smem units 0..3 hi / 4..7 lo) x W2^T
-    if (TWO) mbar_wait_cluster(acts_ready, 0); else mbar_wait(acts_ready, 0);
-    tc_fence_after_sync();
-    mbar_wait(wse_full, 0);
-    CWG_STAMP(7);
-    jb = 2;
-    int n_eo = 0;                                  // folded-`end` MMAs issued so far (round-robin over the chains)
-    auto mma_a_hi = [&](uint32_t d, int kb, int k, uint64_t bdesc, uint32_t idesc, uint32_t acc) {
-      if (L_ACTS_TMEM) mma_ts(d, tmem + L_ACOL(kb * 4 + k), bdesc, idesc, acc);     // A = acts hi in TMEM
-      else mma_ss(d, umma_desc_sw128(smem_u32(slot(kb)) + 32 * k), bdesc, idesc, acc);
-    };
-    auto eo_dst = [&](uint32_t* acc) {
-      const int j = n_eo % L_EO_CHAINS;
-      *acc = n_eo >= L_EO_CHAINS ? 1u : 0u;
-      ++n_eo;
-      return tmem + L_D2_EO + 16 * j;
-    };
-    if (F8) {
-      // f16f8 GEMM2: per 128-channel group two fp16 k-blocks (A = acts hi in TMEM) and two e5m2 k-blocks of 128
-      // (A = the e5m2 acts tiles in units 4 + grp / 6 + grp); the folded-`end` rows ride along as N=16 MMAs
-      const uint32_t dres = tmem + L_D2_RES, d16 = tmem + L_D2_EO;
-      for (int grp = 0; grp < 2; ++grp) {
-        for (int it = 0; it < 4; ++it) {
-          uint32_t r = 0; int jb_cur = 0;
-          if (a.has_res) { jb_cur = jb; wait_full(4 + jb); jb = jb == 2 ? 3 : 2; tc_fence_after_sync(); r = smem_u32(bslot(jb_cur)); }
-          if (it < 2) {
-            const int kb = 2 * grp + it;
-            const uint32_t wv = smem_u32(wse(0, kb));
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const uint32_t o = 32 * k, acc = (kb | k) ? 1u : 0u, a_t = tmem + L_ACOL(kb * 4 + k);
-              if (a.has_res) mma_ts(dres, a_t, umma_desc_sw128(r + o), IDF256, acc);
-              mma_ts(d16, a_t, umma_desc_sw128(wv + o), IDF16, acc);
-            }
-          } else {
-            const uint32_t av = smem_u32(slot(4 + 2 * (it - 2) + grp)), wv = smem_u32(wse(1, 2 * (it - 2) + grp));
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {
-              const uint32_t o = 32 * k;
-              if (a.has_res) mma_f8(dres, umma_desc_sw128(av + o), umma_desc_sw128(r + o), IDE256, 1u);
-              mma_f8(d16, umma_desc_sw128(av + o), umma_desc_sw128(wv + o), IDE16, 1u);
-            }
-          }
-          if (a.has_res) commit(&empty[4 + jb_cur]);
-        }
-        if (a.has_res) commit(&g2_done[grp]);
-      }
-    }
-    for (int kb = 0; kb < (F8 ? 0 : 4); ++kb) {
-      const uint32_t a_lo = smem_u32(slot(4 + kb));
-      const uint32_t w_hi = smem_u32(wse(0, kb)), w_lo = smem_u32(wse(1, kb));
-      const uint32_t dres = tmem + L_D2_RES;
-      uint32_t r_hi = 0, r_lo = 0;
-      int jb_hi = 0, jb_lo = 0;
-      if (a.has_res) {
-        jb_hi = jb; wait_full(4 + jb); jb = jb == 2 ? 3 : 2;
-        if (X3) { jb_lo = jb; wait_full(4 + jb); jb = jb == 2 ? 3 : 2; }
-        tc_fence_after_sync();
-        r_hi = smem_u32(bslot(jb_hi)); r_lo = smem_u32(bslot(jb_lo));
-      }
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        const uint32_t o = 32 * k, acc = (kb | k) ? 1u : 0u;
-        uint32_t eacc;
-        if (a.has_res) mma_a_hi(dres, kb, k, umma_desc_sw128(r_hi + o), ID256, acc);
-        { const uint32_t d16 = eo_dst(&eacc); mma_a_hi(d16, kb, k, umma_desc_sw128(w_hi + o), ID16, eacc); }
-        if (X3) {
-          if (a.has_res) mma_ss(dres, umma_desc_sw128(a_lo + o), umma_desc_sw128(r_hi + o), ID256, 1u);
-          { const uint32_t d16 = eo_dst(&eacc); mma_ss(d16, umma_desc_sw128(a_lo + o), umma_desc_sw128(w_hi + o), ID16, eacc); }
-          if (a.has_res) mma_a_hi(dres, kb, k, umma_desc_sw128(r_lo + o), ID256, 1u);
-          { const uint32_t d16 = eo_dst(&eacc); mma_a_hi(d16, kb, k, umma_desc_sw128(w_lo + o), ID16, eacc); }
-        }
-      }
-      if (a.has_res) {
-        commit(&empty[4 + jb_hi]);
-        if (X3) commit(&empty[4 + jb_lo]);
-        commit(&g2_done[kb]);
-      }
-    }
-    commit(acc2_full);
-    CWG_STAMP(8);
-  } else if (warp == 3 && lane == 0) {
-    // ---------------- folded-`end` weight tiles (kept off the activation producer: issuing them first
-    // delayed the first A tile by ~1 k cycles), then the residual prefetch: as soon as GEMM2 is done with
-    // the acts tiles of a 64-channel block, the x_old (centre tap) tiles of that block are TMA-loaded
-    // over them (units kb / 4+kb)
-    arm(wse_full, 4 * 2048 * PL2);
-    for (int kb = 0; kb < 4; ++kb) {
-      ldb2(wse(0, kb), &tm_wse_hi, wse_full, kb * 64, a.w2_row0 + 256, 16);
-      if (X3 && !F8) ldb2(wse(1, kb), &tm_wse_lo, wse_full, kb * 64, a.w2_row0 + 256, 16);
-    }
-    if (F8)       // e5m2 planes of the 16 folded-`end` rows: [16 rows x 128 B] per 128-channel group
-      for (int grp = 0; grp < 2; ++grp) {
-        ldb2(wse(1, grp), &tm_wse_lo, wse_full, grp * 128, a.w2_row0 + 256, 16);
-        ldb2(wse(1, 2 + grp), &tm_wse_l8, wse_full, grp * 128, a.w2_row0 + 256, 16);
-      }
-    if (a.has_res && F8) {
-      // acts hi live in TMEM, so the A-ring units 0..3 are free once GEMM1 has completed: the hi tiles of x_old go
-      // there right away; the lo tiles follow as GEMM2 releases the e5m2 acts tiles of each 128-channel group
-      static_assert(!F8 || L_ACTS_TMEM, "f16f8 keeps the fp16 acts plane in tensor memory");
-      tma_prefetch_desc(&tm_x_lo);
-      mbar_wait(acc1_full, 0);
-      for (int kb = 0; kb < 4; ++kb) {
-        mbar_arrive_expect_tx(&xold_full[kb], 2 * TILE_A);
-        tma_load_3d(slot(kb), &tm_x_hi, &xold_full[kb], kb * 64, t0, b);
-      }
-      for (int grp = 0; grp < 2; ++grp) {
-        mbar_wait(&g2_done[grp], 0);
-        for (int kb = 2 * grp; kb < 2 * grp + 2; ++kb)
-          tma_load_3d(slot(lo_unit(kb)), &tm_x_lo, &xold_full[kb], kb * 64, t0, b);
-      }
-    }
-    if (a.has_res && !F8) {
-      tma_prefetch_desc(&tm_x_lo);
-      for (int kb = 0; kb < 4; ++kb) {
-        mbar_wait(&g2_done[kb], 0);
-        mbar_arrive_expect_tx(&xold_full[kb], 2 * TILE_A);
-        tma_load_3d(slot(kb), &tm_x_hi, &xold_full[kb], kb * 64, t0, b);
-        tma_load_3d(slot(4 + kb), &tm_x_lo, &xold_full[kb], kb * 64, t0, b);
-      }
-    }
-  } else if (warp >= 4) {
-    // ---------------- epilogue warps: TMEM lane quarter = warp % 4 (one group-step per lane),
-    // column group = (warp - 4) / 4 (channels [16*L_CPG*grp, +16*L_CPG)).
-    const int quarter = warp & 3, grp = (warp - 4) >> 2, row = quarter * 32 + lane;
-    const uint32_t trow = tmem + ((uint32_t)(quarter * 32) << 16);
-    const bool valid = t0 + row < a.Tp;
-    const size_t m = (size_t)b * a.Tp + (size_t)min(t0 + row, a.Tp - 1);
-    const bool stamp = dbg && warp == 4 && lane == 0;
-    const float4* b1t = reinterpret_cast<const float4*>(b1s);
-    const float4* b1g = reinterpret_cast<const float4*>(b1s + 256);
-
-    {   // biases -> smem (read as broadcast float4 in the epilogues); off the prologue's critical path
-      const int e = threadIdx.x - 128;
-      if (e < 256) {     // gate biases pre-multiplied by the argument scales of gate_fused
-        b1s[e] = __ldg(a.b1 + e) * GateK<NPASS>::KA; b1s[256 + e] = __ldg(a.b1 + 256 + e) * GateK<NPASS>::KB;
-        b2s[e] = __ldg(a.b2 + e);
-      }
-      asm volatile("bar.sync 1, %0;" ::"n"(L_EPI_THREADS) : "memory");
-    }
-    // gate: acts = tanh(pre[:, :C]) * sigmoid(pre[:, C:]) -> bf16 planes in slots 0..7 (GEMM2's A operand)
-    if (stamp) dbg[0] = clock64();
-    mbar_wait(acc1_full, 0);
-    tc_fence_after_sync();
-    if (stamp) dbg[1] = clock64();
-    {
-      uint32_t buf[2][32];
-      const int c0 = grp * L_CPG;
-      tmem_issue16x2(trow + c0 * 16, trow + 256 + c0 * 16, buf[0]);
-#pragma unroll
-      for (int i = 0; i < L_CPG; ++i) {
-        const int c = c0 + i;
-        uint32_t* cur = buf[i & 1];
-        tmem_wait32(cur);
-        if (i + 1 < L_CPG) tmem_issue16x2(trow + (c + 1) * 16, trow + 256 + (c + 1) * 16, buf[(i + 1) & 1]);
-        float act[16];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const float4 bt = b1t[c * 4 + q], bs = b1g[c * 4 + q];
-          act[4 * q + 0] = gate_fused<NPASS>(__uint_as_float(cur[4 * q + 0]), __uint_as_float(cur[16 + 4 * q + 0]), bt.x, bs.x);
-          act[4 * q + 1] = gate_fused<NPASS>(__uint_as_float(cur[4 * q + 1]), __uint_as_float(cur[16 + 4 * q + 1]), bt.y, bs.y);
-          act[4 * q + 2] = gate_fused<NPASS>(__uint_as_float(cur[4 * q + 2]), __uint_as_float(cur[16 + 4 * q + 2]), bt.z, bs.z);
-          act[4 * q + 3] = gate_fused<NPASS>(__uint_as_float(cur[4 * q + 3]), __uint_as_float(cur[16 + 4 * q + 3]), bt.w, bs.w);
-        }
-        if (F8) store_split16_tmem_f8(act, trow + L_ACOL(c), slot(4 + (c >> 3)), slot(6 + (c >> 3)), row, c & 7);
-        else if (L_ACTS_TMEM) store_split16_tmem<X3, false>(act, trow + L_ACOL(c), slot(4 + (c >> 2)), row, (c & 3) * 2);
-        else store_split16<X3, false>(act, slot(c >> 2), slot(4 + (c >> 2)), row, (c & 3) * 2);
-      }
-    }
-    if (L_ACTS_TMEM) tmem_wait_st();
-    tc_fence_before_sync();
-    fence_proxy_async_smem();
-    if (TWO && !leader) mbar_arrive_cluster(mapa_shared(acts_ready, 0)); else mbar_arrive(acts_ready);
-    if (stamp) dbg[2] = clock64();
-
-    // prefetch this row's folded-`end` accumulator while GEMM2 runs
-    float4 eold[4];
-    if (grp == 0) {
-      const float4* e = reinterpret_cast<const float4*>(a.first ? a.eo_b : a.eo + m * CWG_EO_PAD);
-#pragma unroll
-      for (int q = 0; q < 4; ++q) eold[q] = __ldg(e + q);
-    }
-
-    // res / skip
-    mbar_wait(acc2_full, 0);
-    tc_fence_after_sync();
-    if (stamp) dbg[3] = clock64();
-    if (grp == 0) {
-      float4 v[4] = {eold[0], eold[1], eold[2], eold[3]};
-#pragma unroll
-      for (int j = 0; j < L_EO_CHAINS; ++j) {          // sum of the independent folded-`end` accumulators
-        uint32_t sk[16];
-        tmem_issue16(trow + L_D2_EO + 16 * j, sk);
-        tmem_wait16(sk);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          v[q].x += __uint_as_float(sk[4 * q]); v[q].y += __uint_as_float(sk[4 * q + 1]);
-          v[q].z += __uint_as_float(sk[4 * q + 2]); v[q].w += __uint_as_float(sk[4 * q + 3]);
-        }
-      }
-      if (valid) {
-        float4* e = reinterpret_cast<float4*>(a.eo + m * CWG_EO_PAD);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) e[q] = v[q];
-      }
-    }
-    if (stamp) dbg[9] = clock64();
-    if (a.has_res) {
-      const float4* b2v = reinterpret_cast<const float4*>(b2s);
-      uint32_t buf[2][16];
-      const int c0 = grp * L_CPG;
-      tmem_issue16(trow + L_D2_RES + c0 * 16, buf[0]);
-#pragma unroll
-      for (int i = 0; i < L_CPG; ++i) {
-        const int c = c0 + i;
-        uint32_t* cur = buf[i & 1];
-        if ((i & 3) == 0) mbar_wait(&xold_full[c >> 2], 0);   // x_old tiles of this 64-channel block have landed
-        tmem_wait16(cur);
-        if (i + 1 < L_CPG) tmem_issue16(trow + L_D2_RES + (c + 1) * 16, buf[(i + 1) & 1]);
-        uint8_t* thi = slot(c >> 2);
-        uint8_t* tlo = slot(lo_unit(c >> 2));
-        const uint32_t o0 = sw128_offset(row, (c & 3) * 2), o1 = sw128_offset(row, (c & 3) * 2 + 1);
-        const uint4 h0 = *reinterpret_cast<const uint4*>(thi + o0), h1 = *reinterpret_cast<const uint4*>(thi + o1);
-        const uint4 l0 = *reinterpret_cast<const uint4*>(tlo + o0), l1 = *reinterpret_cast<const uint4*>(tlo + o1);
-        const uint32_t hw[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
-        const uint32_t lw[8] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w};
-        float r[16];
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          const float4 bb = b2v[c * 4 + q];
-          r[4 * q] = __uint_as_float(cur[4 * q]) + bb.x; r[4 * q + 1] = __uint_as_float(cur[4 * q + 1]) + bb.y;
-          r[4 * q + 2] = __uint_as_float(cur[4 * q + 2]) + bb.z; r[4 * q + 3] = __uint_as_float(cur[4 * q + 3]) + bb.w;
-        }
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {   // x_new = x_old(hi + lo) + res, glow.py:217
-          float h0, h1, l0f, l1f;
-          unpack2<F8>(hw[j], h0, h1); unpack2<F8>(lw[j], l0f, l1f);
-          r[2 * j] += h0 + l0f;
-          r[2 * j + 1] += h1 + l1f;
-        }
-        // in place (same thread, same addresses); f16f8 adds the two e5m2 planes of this 128-channel group, staged
-        // in the idle W2 weight slots (units 8 + grp and 10 + grp)
-        if (F8) store_split16_f8(r, thi, tlo, slot(8 + grp), slot(10 + grp), row, (c & 3) * 2, c & 7);
-        else store_split16<true>(r, thi, tlo, row, (c & 3) * 2);
-        if ((i & 3) == 3) {
-          // one 64-channel tile (hi + lo) of this column group is final: store it while the rest computes
-          fence_proxy_async_smem();
-          asm volatile("bar.sync %0, 128;" ::"r"(2 + grp) : "memory");
-          if (quarter == 0 && lane == 0) {
-            const int kb = c >> 2;
-            tma_store_3d(&tm_xo_hi, slot(kb), kb * 64, t0, b);
-            tma_store_3d(&tm_xo_lo, slot(lo_unit(kb)), kb * 64, t0, b);
-            if (F8 && i == L_CPG - 1) {
-              tma_store_3d(&tm_xo_l8, slot(8 + grp), grp * 128, t0, b);
-              tma_store_3d(&tm_xo_h8, slot(10 + grp), grp * 128, t0, b);
-            }
-            tma_store_commit();
-          }
-        }
-      }
-      if (stamp) dbg[10] = clock64();
-      if (quarter == 0 && lane == 0) tma_store_wait_read();
-    }
-    tc_fence_before_sync();
-    if (stamp) dbg[4] = clock64();
-  }
-  __syncthreads();
-  if (TWO) cluster_sync_all();                     // the pair releases TMEM together; no CTA exits with peer traffic pending
-  if (warp == 1) { __syncwarp(); if (TWO) tmem_dealloc_2sm(tmem, 512); else tmem_dealloc(tmem, 512); }
-}
-
-
 }  // namespace
-
-void debug_set_timing(long long* buf) { g_dbg_timing = buf; }
 
 int launch_cond_tc(const Dims& d, const cwg_weights* w, int npass, int flow, const float* mel,
                    const float* cond_bias, __nv_bfloat16* h2_planes, __nv_bfloat16* mel4_planes,
@@ -916,28 +209,6 @@ int launch_cond_tc(const Dims& d, const cwg_weights* w, int npass, int flow, con
   a.M = (int)rows; a.Tm = d.Tm; a.B = d.B; a.w_row0 = flow * (int)ncol; a.nkb = d.KCp / 64;
   a.range_flag = npass == 2 ? range_flag() : nullptr;
   dim3 grid(d.P, (unsigned)((rows + 127) / 128));
-  static const int use_2sm = [] { const char* e = getenv("CWG_COND_2SM"); return e && e[0] == '1'; }();
-  if (use_2sm) {
-    CUtensorMap tb2_hi, tb2_lo;                                  // weight tiles in 128-row halves
-    if (int r = map_2d(&tb2_hi, w->cond_w_hi, d.KCp, (uint64_t)d.F * ncol, 128)) return r;
-    if (int r = map_2d(&tb2_lo, w->cond_w_lo, d.KCp, (uint64_t)d.F * ncol, 128)) return r;
-    // a row tile past the end is zero-filled / clipped by TMA
-    cudaLaunchConfig_t lc{};
-    lc.gridDim = dim3((grid.y + 1) & ~1u, grid.x); lc.blockDim = dim3(192); lc.stream = s;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension;
-    at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    lc.attrs = at; lc.numAttrs = 1;
-#define CWG_LAUNCH_COND2(NP)                                                                                     \
-    do {                                                                                                         \
-      lc.dynamicSmemBytes = Cond2Cfg<NP>::SMEM;                                                                  \
-      if (int r = set_smem(k_cond_tc2<NP>, Cond2Cfg<NP>::SMEM)) return r;                                        \
-      CWG_CHECK_CUDA(cudaLaunchKernelEx(&lc, k_cond_tc2<NP>, ta_hi, ta_lo, tb2_hi, tb2_lo, tc_hi, tc_lo, tc_h8, a)); \
-    } while (0)
-    if (npass == 3) CWG_LAUNCH_COND2(3); else if (npass == 2) CWG_LAUNCH_COND2(2); else CWG_LAUNCH_COND2(1);
-#undef CWG_LAUNCH_COND2
-    return 0;
-  }
   if (npass == 3) {
     if (int r = set_smem(k_cond_tc<3>, CondCfg<3>::SMEM)) return r;
     k_cond_tc<3><<<grid, 320, CondCfg<3>::SMEM, s>>>(ta_hi, ta_lo, tb_hi, tb_lo, tc_hi, tc_lo, tc_h8, a);
@@ -948,97 +219,6 @@ int launch_cond_tc(const Dims& d, const cwg_weights* w, int npass, int flow, con
     if (int r = set_smem(k_cond_tc<1>, CondCfg<1>::SMEM)) return r;
     k_cond_tc<1><<<grid, 320, CondCfg<1>::SMEM, s>>>(ta_hi, ta_lo, tb_hi, tb_lo, tc_hi, tc_lo, tc_h8, a);
   }
-  CWG_CHECK_CUDA(cudaGetLastError());
-  return 0;
-}
-
-int launch_layer_tc(const Dims& d, const cwg_weights* w, int npass, int flow, int layer,
-                    const __nv_bfloat16* x_in, __nv_bfloat16* x_out, const __nv_bfloat16* h2,
-                    float* eo, cudaStream_t s) {
-  CWG_REQUIRE(d.MG == 16 && d.b1_batch == nullptr,
-              "the one-tile-per-CTA layer kernel takes n_group <= 16 and a shared gate bias (unset CWG_LAYER_PS)");
-  const size_t plane = (size_t)d.BT * d.C, hplane = (size_t)d.BT * d.H;
-  const uint64_t fl = (uint64_t)d.F * d.L;
-  CUtensorMap tx_hi, tx_lo, th_hi, th_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo, tse_hi, tse_lo, to_hi, to_lo;
-  if (int r = map_act(&tx_hi, x_in, d.C, d.Tp, d.B)) return r;
-  if (int r = map_act(&tx_lo, x_in + plane, d.C, d.Tp, d.B)) return r;
-  if (int r = map_act(&th_hi, h2, d.H, d.Tp, d.B)) return r;
-  if (int r = map_act(&th_lo, h2 + hplane, d.H, d.Tp, d.B)) return r;
-  if (int r = map_2d(&tw1_hi, w->w1_hi, d.K1, fl * 2 * d.C, 256)) return r;
-  if (int r = map_2d(&tw1_lo, npass == 2 ? w->w1_hi : w->w1_lo, d.K1, fl * 2 * d.C, 256)) return r;   // f16f8 has no w1 lo plane
-  if (int r = map_2d(&tw2_hi, w->w2_hi, d.C, fl * d.N2, 256)) return r;
-  if (npass != 2) { if (int r = map_2d(&tw2_lo, w->w2_lo, d.C, fl * d.N2, 256)) return r; }
-  if (int r = map_2d(&tse_hi, w->w2_hi, d.C, fl * d.N2, 16)) return r;
-  if (npass != 2) { if (int r = map_2d(&tse_lo, w->w2_lo, d.C, fl * d.N2, 16)) return r; }
-  if (int r = map_act(&to_hi, x_out, d.C, d.Tp, d.B)) return r;
-  if (int r = map_act(&to_lo, x_out + plane, d.C, d.Tp, d.B)) return r;
-  // e5m2 planes (CWG_MODE_F16F8): x = [fp16 hi][fp16 lo][e5m2 lo*2^P][e5m2 hi*2^-Q], H2 = [fp16 hi][e5m2 lo*2^P][e5m2 hi*2^-Q]
-  CUtensorMap tx_l8 = tx_hi, tx_h8 = tx_hi, th_l8 = tx_hi, th_h8 = tx_hi, tw1_h8 = tx_hi, tw1_l8 = tx_hi, to_l8 = tx_hi, to_h8 = tx_hi;
-  CUtensorMap tw2_l8 = tx_hi, tse_l8 = tx_hi;
-  if (npass == 2) {
-    // the e5m2 planes of w2: hi*2^-P through the tw2_lo / tse_lo parameters, lo*2^Q through tw2_l8 / tse_l8
-    if (int r = map_2d8(&tw2_lo, w->w2_h8, d.C, fl * d.N2, 256)) return r;
-    if (int r = map_2d8(&tse_lo, w->w2_h8, d.C, fl * d.N2, 16)) return r;
-    if (int r = map_2d8(&tw2_l8, w->w2_l8, d.C, fl * d.N2, 256)) return r;
-    if (int r = map_2d8(&tse_l8, w->w2_l8, d.C, fl * d.N2, 16)) return r;
-    const uint8_t* xi8 = reinterpret_cast<const uint8_t*>(x_in) + 4 * plane;
-    uint8_t* xo8 = reinterpret_cast<uint8_t*>(x_out) + 4 * plane;
-    const uint8_t* h8 = reinterpret_cast<const uint8_t*>(h2) + 2 * hplane;
-    if (int r = map_act8(&tx_l8, xi8, d.C, d.Tp, d.B)) return r;
-    if (int r = map_act8(&tx_h8, xi8 + plane, d.C, d.Tp, d.B)) return r;
-    if (int r = map_act8(&th_l8, h8, d.H, d.Tp, d.B)) return r;
-    if (int r = map_act8(&th_h8, h8 + hplane, d.H, d.Tp, d.B)) return r;
-    if (int r = map_2d8(&tw1_h8, w->w1_h8, d.K1, fl * 2 * d.C, 256)) return r;
-    if (int r = map_2d8(&tw1_l8, w->w1_l8, d.K1, fl * 2 * d.C, 256)) return r;
-    if (int r = map_act8(&to_l8, xo8, d.C, d.Tp, d.B)) return r;
-    if (int r = map_act8(&to_h8, xo8 + plane, d.C, d.Tp, d.B)) return r;
-  }
-  const size_t idx = (size_t)flow * d.L + layer;
-  LayerArgs a{};
-  a.b1 = w->b1 + idx * 2 * d.C; a.b2 = w->b2 + idx * d.C; a.eo_b = w->eo_b + (size_t)flow * CWG_EO_PAD;
-  a.eo = eo; a.x_hi = x_in; a.x_lo = x_in + plane;
-  a.Tp = d.Tp; a.dil = 1 << layer;
-  a.w1_row0 = (int)(idx * 2 * d.C); a.w2_row0 = (int)(idx * d.N2);
-  a.has_res = layer < d.L - 1; a.first = layer == 0;
-  a.dbg = g_dbg_timing;
-  // 2-SM MMAs (cta_group::2).  CTA pairs = neighbouring tiles of one utterance (cluster along x); each
-  // CTA loads half of the N rows of every weight tile, so the weight maps get 128-row boxes.
-  // An odd tile count gets one tile fully past T' (TMA zero-fills its loads and clips its stores).
-  // Default: on for bf16x3 / f16f8 (measured +2.7 % / +0.9 % on config 2), off for bf16 (-0.5 %); CWG_LAYER_2SM=0/1 forces it.
-  static const int two_env = [] { const char* e = getenv("CWG_LAYER_2SM"); return e ? (e[0] == '1' ? 1 : 0) : -1; }();
-  const int two = two_env >= 0 ? two_env : (npass != 1);
-  unsigned tiles = (unsigned)((d.Tp + 127) / 128);
-  if (two) {
-    tiles = (tiles + 1) & ~1u;
-    if (int r = map_2d(&tw1_hi, w->w1_hi, d.K1, fl * 2 * d.C, 128)) return r;
-    if (int r = map_2d(&tw2_hi, w->w2_hi, d.C, fl * d.N2, 128)) return r;
-    if (npass == 2) {
-      if (int r = map_2d8(&tw1_h8, w->w1_h8, d.K1, fl * 2 * d.C, 128)) return r;
-      if (int r = map_2d8(&tw1_l8, w->w1_l8, d.K1, fl * 2 * d.C, 128)) return r;
-      if (int r = map_2d8(&tw2_lo, w->w2_h8, d.C, fl * d.N2, 128)) return r;
-      if (int r = map_2d8(&tw2_l8, w->w2_l8, d.C, fl * d.N2, 128)) return r;
-    } else {
-      if (int r = map_2d(&tw1_lo, w->w1_lo, d.K1, fl * 2 * d.C, 128)) return r;
-      if (int r = map_2d(&tw2_lo, w->w2_lo, d.C, fl * d.N2, 128)) return r;
-    }
-  }
-  dim3 grid(tiles, d.B);
-  cudaLaunchConfig_t lc{};
-  lc.gridDim = grid; lc.blockDim = dim3(L_THREADS); lc.dynamicSmemBytes = L_SMEM; lc.stream = s;
-  cudaLaunchAttribute lattr[1];
-  lattr[0].id = cudaLaunchAttributeClusterDimension;
-  lattr[0].val.clusterDim.x = 2; lattr[0].val.clusterDim.y = 1; lattr[0].val.clusterDim.z = 1;
-  lc.attrs = lattr; lc.numAttrs = two ? 1 : 0;
-#define CWG_LAUNCH_LAYER(NP, TW)                                                                                      \
-  do {                                                                                                                \
-    if (int r = set_smem(k_layer_tc<NP, TW>, L_SMEM)) return r;                                                       \
-    CWG_CHECK_CUDA(cudaLaunchKernelEx(&lc, k_layer_tc<NP, TW>, tx_hi, tx_lo, th_hi, th_lo, tw1_hi, tw1_lo, tw2_hi,    \
-                                      tw2_lo, tse_hi, tse_lo, to_hi, to_lo, tx_l8, tx_h8, th_l8, th_h8, tw1_h8,       \
-                                      tw1_l8, to_l8, to_h8, tw2_l8, tse_l8, a));                                      \
-  } while (0)
-  if (two) { if (npass == 3) CWG_LAUNCH_LAYER(3, true); else if (npass == 2) CWG_LAUNCH_LAYER(2, true); else CWG_LAUNCH_LAYER(1, true); }
-  else     { if (npass == 3) CWG_LAUNCH_LAYER(3, false); else if (npass == 2) CWG_LAUNCH_LAYER(2, false); else CWG_LAUNCH_LAYER(1, false); }
-#undef CWG_LAUNCH_LAYER
   CWG_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

@@ -8,7 +8,7 @@
 //   k_res512_tc  : grid.z = res channel half q.  acts [128 x 512] x W2[256q:256q+256]^T (8 k-blocks),
 //                  residual add + TMA store; the q = 0 CTAs also accumulate the folded `end` (N = 16).
 //
-// Same reference lines as cwg_tc.cu (glow.py:201-222).
+// Same reference lines as cwg_ps.cu (glow.py:201-222).
 #include "cwg_tc_common.cuh"
 
 namespace cwg {

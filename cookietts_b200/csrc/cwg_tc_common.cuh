@@ -67,16 +67,6 @@ inline int map_w0(CUtensorMap* m, const void* ptr, uint64_t rows) {
   return make_map(m, ptr, 2, dims, st, box, false, true);
 }
 
-// shared-tap tiles: the same maps with taller boxes (128 + 2 * dilation steps, <= 256)
-inline int map_act_rows(CUtensorMap* m, const void* ptr, uint64_t C, uint64_t Tp, uint64_t B, uint32_t rows) {
-  uint64_t dims[3] = {C, Tp, B}; uint64_t st[2] = {C * 2, Tp * C * 2}; uint32_t box[3] = {64, rows, 1};
-  return make_map(m, ptr, 3, dims, st, box);
-}
-inline int map_act8_rows(CUtensorMap* m, const void* ptr, uint64_t C, uint64_t Tp, uint64_t B, uint32_t rows) {
-  uint64_t dims[3] = {C, Tp, B}; uint64_t st[2] = {C, Tp * C}; uint32_t box[3] = {128, rows, 1};
-  return make_map(m, ptr, 3, dims, st, box, true);
-}
-
 // 8-bit (e5m2) planes: the same tiles measured in bytes - 128 channels x 128 steps / 128 k x box_rows rows = 16 KB units
 inline int map_2d8(CUtensorMap* m, const void* ptr, uint64_t cols, uint64_t rows, uint32_t box_rows) {
   uint64_t dims[2] = {cols, rows}; uint64_t st[1] = {cols}; uint32_t box[2] = {128, box_rows};
@@ -94,9 +84,6 @@ constexpr int TILE_A = 128 * 128;      // [128 rows][64 bf16] = 16 KB
 constexpr uint32_t IDESC_N256 = umma_idesc_bf16(128, 256);
 constexpr uint32_t IDESC_N16 = umma_idesc_bf16(128, 16);
 constexpr uint32_t IDESC_F16_N256 = umma_idesc_f16(128, 256);
-constexpr uint32_t IDESC_F16_N16 = umma_idesc_f16(128, 16);
-constexpr uint32_t IDESC_E5M2_N256 = umma_idesc_e5m2(128, 256);
-constexpr uint32_t IDESC_E5M2_N16 = umma_idesc_e5m2(128, 16);
 
 __device__ __forceinline__ uint8_t* align_1024(uint8_t* p) {
   uint32_t a = smem_u32(p);
@@ -276,15 +263,6 @@ __device__ __forceinline__ void issue_kblock_fast(uint32_t a_addr, uint32_t b_ad
   umma_bf16(tmem_d, da + 2, db + 2, idesc, 1u);
   umma_bf16(tmem_d, da + 4, db + 4, idesc, 1u);
   umma_bf16(tmem_d, da + 6, db + 6, idesc, 1u);
-}
-// One 128-deep k-block of e5m2 operands = 4 UMMA K-steps of 32 bytes along the swizzled 128-byte row.
-__device__ __forceinline__ void issue_kblock_fast_f8(uint32_t a_addr, uint32_t b_addr, uint32_t tmem_d, uint32_t idesc) {
-  const uint64_t da = DESC_SW128_HI | (uint64_t)((a_addr & 0x3FFFF) >> 4);
-  const uint64_t db = DESC_SW128_HI | (uint64_t)((b_addr & 0x3FFFF) >> 4);
-  umma_f8(tmem_d, da, db, idesc, 1u);
-  umma_f8(tmem_d, da + 2, db + 2, idesc, 1u);
-  umma_f8(tmem_d, da + 4, db + 4, idesc, 1u);
-  umma_f8(tmem_d, da + 6, db + 6, idesc, 1u);
 }
 
 // 2 x 16 TMEM columns, issued without waiting; pair with tmem_wait32.

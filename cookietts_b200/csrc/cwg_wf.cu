@@ -7,7 +7,7 @@
 //   efficient_modules.py:360-403   PermuteHeight.inverse         -> column bookkeeping on the host (no data movement)
 //
 // One autoregressive row step of one layer is the same fused kernel shape as the 1-D WN layer
-// (cwg_tc.cu): implicit GEMM over K = (kh rows) x (kw dilated taps) x C + padded mel, gate epilogue,
+// (cwg_ps.cu): implicit GEMM over K = (kh rows) x (kw dilated taps) x C + padded mel, gate epilogue,
 // res/skip GEMM, residual update.  The "conv queue" of the reference is a 3-slot ring of each
 // layer's input rows kept in HBM; rows that do not exist yet (zero queue) are simply skipped.
 #include "cwg_tc_common.cuh"

@@ -1,7 +1,7 @@
 """Drop-in for the reference's "ax" model `efficient_model_ax.py::WaveGlow` with `waveflow=False`
 (1-D WN + affine coupling + invertible 1x1 conv / PermuteHeight), inverse pass only.
 
-It runs on the SAME sm_100a layer / boundary kernels as the classic model (csrc/cwg_tc.cu,
+It runs on the SAME sm_100a layer / boundary kernels as the classic model (csrc/cwg_ps.cu,
 cwg_simple.cu): the cond vector is the F.interpolate'd mel (efficient_model_ax.py:171-182, computed
 once because `upsample_first=True`), zero-padded to the kernels' cond width, and the WN's single 1x1
 cond layer (glow_ax.py:297-312) rides as extra K columns of each in_layer GEMM; PermuteHeight is

@@ -39,7 +39,7 @@ def _mm(a, w, emulate):
     if emulate == "f16f8":
         a16 = _r16(a)
         a_lo = a - a16
-        if isinstance(w_lo, tuple):          # fp16 pass + two e5m2 correction passes (csrc/cwg_tc.cu, GEMM1)
+        if isinstance(w_lo, tuple):          # fp16 pass + two e5m2 correction passes (csrc/cwg_ps.cu, GEMM1)
             w_h8, w_l8 = w_lo
             return a16 @ w_hi.T + _r8(a_lo * 2.0 ** F8_P) @ w_h8.T + _r8(a16 * 2.0 ** -F8_Q) @ w_l8.T
         return a16 @ w_hi.T + _r16(a_lo) @ w_hi.T + a16 @ w_lo.T      # fp16 hi/lo, 3 passes

@@ -1,5 +1,5 @@
 #!/bin/bash
-# round-2 first GPU pass: stage parity of the persistent layer kernel, its timing against the round-1 kernel, full GPU suite, bench
+# round-2 first GPU pass: stage parity of the persistent layer kernel, its timing, full GPU suite, bench
 mkdir -p gpurun_out
 timeout 600 python -m pytest tests/test_gpu_stages.py -x -q > gpurun_out/r2a_stages.log 2>&1; rc=$?
 tail -15 gpurun_out/r2a_stages.log
@@ -12,5 +12,3 @@ timeout 1500 python -m pytest tests -m gpu -x -q > gpurun_out/r2a_gpu_tests.log 
 tail -8 gpurun_out/r2a_gpu_tests.log
 timeout 600 python bench.py > gpurun_out/r2a_bench.json 2> gpurun_out/r2a_bench.err
 tail -2 gpurun_out/r2a_bench.json
-CWG_LAYER_PS=0 timeout 600 python bench.py > gpurun_out/r2a_bench_ps0.json 2> gpurun_out/r2a_bench_ps0.err
-tail -2 gpurun_out/r2a_bench_ps0.json

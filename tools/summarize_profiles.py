@@ -34,7 +34,7 @@ def raw_rows(rep):
 
 
 lines = [f"# ncu summaries ({tag}) - extracted by tools/summarize_profiles.py from gpurun_out/*.ncu-rep",
-         "# capture: ncu --set full --clock-control none --import-source on (see tools/profile_r1.sh);",
+         "# capture: ncu --set full --clock-control none --import-source on (see tools/profile_r2b.sh);",
          "# per-launch values, cold-cache and serialised: compare shares, not absolutes.", ""]
 for name in sorted(os.listdir(os.path.join(ROOT, "gpurun_out"))):
     if not name.endswith(".ncu-rep"):

@@ -1,4 +1,4 @@
-"""Times the cond GEMM stage (cwg_cond) at BASELINE config-2 size; CWG_COND_2SM=1 selects the 2-SM MMA variant."""
+"""Times the cond GEMM stage (cwg_cond) at BASELINE config-2 size."""
 import os, sys
 import numpy as np, torch
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
@@ -23,4 +23,4 @@ for prec in sys.argv[1:] or ["bf16x3", "f16f8", "bf16"]:
     for _ in range(10):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize(); e0.record(); run(); e1.record(); torch.cuda.synchronize(); ts.append(e0.elapsed_time(e1))
-    print(prec, "2sm" if os.environ.get("CWG_COND_2SM") == "1" else "1sm", "cond stage median %.1f us (incl. im2col)" % (np.median(ts) * 1e3), "sum", float(out[:1000].float().sum()))
+    print(prec, "cond stage median %.1f us (incl. im2col)" % (np.median(ts) * 1e3), "sum", float(out[:1000].float().sum()))
