@@ -8,8 +8,14 @@
 //
 // One autoregressive row step of one layer is the same fused kernel shape as the 1-D WN layer
 // (cwg_ps.cu): implicit GEMM over K = (kh rows) x (kw dilated taps) x C + padded mel, gate epilogue,
-// res/skip GEMM, residual update.  The "conv queue" of the reference is a 3-slot ring of each
+// res/skip GEMM, residual update.  The "conv queue" of the reference is a kernel_h-slot ring of each
 // layer's input rows kept in HBM; rows that do not exist yet (zero queue) are simply skipped.
+//
+// Two in_layer layouts run on the tensor cores:
+//   dense 3x3 (k_wf_layer_tc; a separable 3x3 is folded into it at pack time): K = 9 x C + mel.
+//   depthwise-separable, kernel_h <= 7 x odd kernel_w <= 7 (k_wf_sep_tc; the layout of the reference author's
+//   trained checkpoints, glow_ax.py:525-531): the depthwise conv runs on the CUDA cores inside the layer kernel
+//   and writes its output straight into shared memory as the A operand of the pointwise GEMM, K = C + mel.
 #include "cwg_tc_common.cuh"
 
 namespace cwg {
@@ -22,11 +28,12 @@ namespace {
 constexpr int WF_C = 128, WF_KH = 3, WF_KW = 3, WF_HP = CWG_WF_COND_PAD;
 constexpr int WF_K1 = WF_KH * WF_KW * WF_C + WF_HP;     // 1280
 constexpr int WF_N2 = WF_C + CWG_EO_PAD;                // 144
-constexpr int WF_TC_MAX_GROUP = 16;                    // squeeze height of the tensor-core path (the fp32 path takes <= 32)
+constexpr int WF_TC_MAX_GROUP = 32;                    // squeeze height (only host arrays are sized by it)
+constexpr int WF_SEP_MAX_KH = 7, WF_SEP_MAX_KW = 7;     // separable in_layers: kernel_h <= 7, odd kernel_w <= 7
 constexpr uint32_t IDESC_N144 = umma_idesc_bf16(128, 144);
 
 struct WfDims {
-  int B, Tp, F, L, G, M;
+  int B, Tp, F, L, G, M, KH;
   long long BT;
 };
 
@@ -121,9 +128,15 @@ struct WfLayerArgs {
   int Tp, dil;
   int w1_row0, w2_row0;
   int ring_in, ring_out;  // 4th tensor-map coordinate base of the layer's input ring / next layer's ring
-  int row;                // AR row index (newest row), ring slot = row % 3
+  int row;                // AR row index (newest row), ring slot = row % 3 (row % kh when separable)
   int rows_valid;         // min(row + 1, 3): rows of the conv queue that exist
   int has_res, first;
+  // separable in_layers only (k_wf_sep_tc)
+  const __nv_bfloat16* x; // ring hi plane; the lo plane follows at x + xplane
+  long long xplane, BT;
+  const float* dw_w;      // [C][kh * kw] depthwise weights of this (flow, layer)
+  const float* dw_b;      // [C]
+  int kh, kw;
 };
 
 // Two CTAs per SM (each: 6 smem units = 96 KB, 256 TMEM columns), so one CTA's epilogues overlap
@@ -397,8 +410,364 @@ k_wf_layer_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant
   if (warp == 1) { __syncwarp(); tmem_dealloc(tmem, 256); }
 }
 
+// Separable layout (k_wf_sep_tc), one CTA per SM: the same pool (units 0..5), plus the depthwise output d - GEMM1's
+// x operand, hi in units 6,7 and lo in units 8,9 - and the depthwise weights transposed to [tap][C].
+constexpr int S_NS = W_NS + 4;
+constexpr int S_OFF_DW = S_NS * TILE_A;                                   // 163840
+constexpr int S_OFF_DWB = S_OFF_DW + WF_SEP_MAX_KH * WF_SEP_MAX_KW * WF_C * 4;
+constexpr int S_OFF_B1 = S_OFF_DWB + WF_C * 4;
+constexpr int S_OFF_B2 = S_OFF_B1 + 1024;
+constexpr int S_OFF_BAR = S_OFF_B2 + 512;
+constexpr int S_SMEM = S_OFF_BAR + 256 + 1024;                             // 192256
+
+// Depthwise part of a separable in_layer (glow_ax.py:525-528) for the 128 steps of this tile, by the 8 epilogue warps
+// while the mel k-blocks of GEMM1 run:
+//   d[t][c] = dw_b[c] + sum_{a,b} dw_w[c][a][b] * x[row - (kh-1-a)][t + (b - kw/2) * dil][c]     in fp32, x = hi + lo,
+// causal in height (rows that do not exist yet are the zero queue), zero-padded in width per utterance.  A lane owns 4
+// channels and a warp one step at a time, so each load is a 256-byte run of channels.  d is written as 128B-swizzled
+// bf16 hi (and lo) tiles, one per 64-channel k-block; it never goes to HBM.
+template <int NPASS>
+__device__ __forceinline__ void wf_depthwise_tile(const WfLayerArgs& a, const float* dws, const float* dwb, int b, int t0,
+                                                  int ew, int lane, uint8_t* d_hi, uint8_t* d_lo) {
+  // A warp handles 16 steps in two passes of S.  The loop is not bound by load latency (issuing two taps' loads at once
+  // was slower), so its instruction count is kept down: per bf16x2 word two FFMA2 (hi, then lo; no separate hi + lo add),
+  // and a pass checks the utterance bounds once when all S steps of a tap are inside (the common case).
+  constexpr int S = 8;
+  const int c = 4 * lane, chunk = (lane & 15) >> 1, sub = (lane & 1) * 8;
+  uint8_t* th = d_hi + (lane >> 4) * TILE_A;
+  uint8_t* tl = d_lo + (lane >> 4) * TILE_A;
+  const float4 bias = *reinterpret_cast<const float4*>(dwb + c);
+  auto lo2 = [](uint32_t v) { return make_float2(__uint_as_float(v << 16), __uint_as_float(v & 0xFFFF0000u)); };
+  for (int s0 = ew * 16; s0 < ew * 16 + 16; s0 += S) {
+    float2 acc[S][2];
+#pragma unroll
+    for (int i = 0; i < S; ++i) { acc[i][0] = make_float2(bias.x, bias.y); acc[i][1] = make_float2(bias.z, bias.w); }
+    for (int ah = 0; ah < a.kh; ++ah) {
+      const int r = a.row - (a.kh - 1 - ah);
+      if (r < 0) continue;
+      const __nv_bfloat16* xh = a.x + ((size_t)(a.ring_in + r % a.kh) * a.BT + (size_t)b * a.Tp) * WF_C + c;
+      const __nv_bfloat16* xl = xh + a.xplane;
+      for (int bw = 0; bw < a.kw; ++bw) {
+        const float4 w = *reinterpret_cast<const float4*>(dws + (ah * a.kw + bw) * WF_C + c);
+        const float2 w01 = make_float2(w.x, w.y), w23 = make_float2(w.z, w.w);
+        const int tt0 = t0 + s0 + (bw - a.kw / 2) * a.dil;
+        uint2 h[S], l[S];
+        if (tt0 >= 0 && tt0 + S <= a.Tp) {
+#pragma unroll
+          for (int i = 0; i < S; ++i) {
+            h[i] = __ldg(reinterpret_cast<const uint2*>(xh + (size_t)(tt0 + i) * WF_C));
+            l[i] = __ldg(reinterpret_cast<const uint2*>(xl + (size_t)(tt0 + i) * WF_C));
+          }
+        } else {
+#pragma unroll
+          for (int i = 0; i < S; ++i) {
+            const int tt = tt0 + i;
+            h[i] = l[i] = make_uint2(0u, 0u);
+            if (tt >= 0 && tt < a.Tp) {
+              h[i] = __ldg(reinterpret_cast<const uint2*>(xh + (size_t)tt * WF_C));
+              l[i] = __ldg(reinterpret_cast<const uint2*>(xl + (size_t)tt * WF_C));
+            }
+          }
+        }
+#pragma unroll
+        for (int i = 0; i < S; ++i) {
+          acc[i][0] = __ffma2_rn(w01, lo2(l[i].x), __ffma2_rn(w01, lo2(h[i].x), acc[i][0]));
+          acc[i][1] = __ffma2_rn(w23, lo2(l[i].y), __ffma2_rn(w23, lo2(h[i].y), acc[i][1]));
+        }
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < S; ++i) {
+      const uint32_t off = sw128_offset(s0 + i, chunk) + sub;
+      const float2 d01 = acc[i][0], d23 = acc[i][1];
+      const uint32_t h0 = pack_bf16x2(d01.x, d01.y), h1 = pack_bf16x2(d23.x, d23.y);
+      *reinterpret_cast<uint2*>(th + off) = make_uint2(h0, h1);
+      if (NPASS == 3) {
+        float e0, e1, e2, e3;
+        unpack2<false>(h0, e0, e1); unpack2<false>(h1, e2, e3);
+        *reinterpret_cast<uint2*>(tl + off) = make_uint2(pack_bf16x2(d01.x - e0, d01.y - e1), pack_bf16x2(d23.x - e2, d23.y - e3));
+      }
+    }
+  }
+}
+
+// The layer step with separable in_layers, one CTA per SM: GEMM1 runs over the 2 mel k-blocks (TMA, issued first), then
+// the 2 k-blocks of d, which the epilogue warps compute in the meantime (wf_depthwise_tile).  Gate, GEMM2 ([res | folded
+// end], N = 144), residual update and eo accumulation are those of k_wf_layer_tc, whose source is kept as it is.
+template <int NPASS>
+__global__ void __launch_bounds__(W_THREADS, 1)
+k_wf_sep_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ CUtensorMap tm_x_lo,
+            const __grid_constant__ CUtensorMap tm_m_hi, const __grid_constant__ CUtensorMap tm_m_lo,
+            const __grid_constant__ CUtensorMap tm_w1_hi, const __grid_constant__ CUtensorMap tm_w1_lo,
+            const __grid_constant__ CUtensorMap tm_w2_hi, const __grid_constant__ CUtensorMap tm_w2_lo, WfLayerArgs a) {
+  constexpr int PL = NPASS == 3 ? 2 : 1;
+  extern __shared__ uint8_t smem_raw[];
+  uint8_t* smem = align_1024(smem_raw);
+  float* b1s = reinterpret_cast<float*>(smem + S_OFF_B1);
+  float* b2s = reinterpret_cast<float*>(smem + S_OFF_B2);
+  uint64_t* full = reinterpret_cast<uint64_t*>(smem + S_OFF_BAR);
+  uint64_t* empty = full + W_NBAR;
+  uint64_t* acc1_full = empty + W_NBAR;
+  uint64_t* acts_ready = acc1_full + 1;
+  uint64_t* acc2_full = acts_ready + 1;
+  uint64_t* xold_full = acc2_full + 1;
+  uint64_t* d_ready = xold_full + 1;                 // depthwise tiles written
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(d_ready + 1);
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int t0 = blockIdx.x * 128, b = blockIdx.y;
+  auto slot = [&](int i) { return smem + i * TILE_A; };
+  auto bslot = [&](int j) { return smem + (W_NA + 2 * j) * TILE_A; };
+  constexpr int nkb = WF_HP / 64;                   // mel k-blocks through the A ring
+  constexpr int NKB_D = WF_C / 64;                  // k-blocks of d, after the mel ones
+  const int nslot = a.kh;                           // ring slots per layer
+
+  if (threadIdx.x == 0) {
+    for (int i = 0; i < W_NBAR; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
+    mbar_init(acc1_full, 1); mbar_init(acts_ready, W_EPI_THREADS); mbar_init(acc2_full, 1); mbar_init(xold_full, 1);
+    mbar_init(d_ready, W_EPI_THREADS);
+    fence_barrier_init();
+  }
+  if (warp == 1) tmem_alloc(tmem_slot, 256);
+  if (warp >= 4) {
+    const int e = threadIdx.x - 128;
+    b1s[e] = __ldg(a.b1 + e);
+    if (e < WF_C) b2s[e] = __ldg(a.b2 + e);
+    float* dws = reinterpret_cast<float*>(smem + S_OFF_DW);
+    const int ntap = a.kh * a.kw;
+    for (int i = e; i < ntap * WF_C; i += W_EPI_THREADS) dws[(i % ntap) * WF_C + i / ntap] = __ldg(a.dw_w + i);
+    if (e < WF_C) reinterpret_cast<float*>(smem + S_OFF_DWB)[e] = __ldg(a.dw_b + e);
+  }
+  tc_fence_before_sync();
+  __syncthreads();
+  tc_fence_after_sync();
+  const uint32_t tmem = *tmem_slot;
+
+  // k-block order of GEMM1: the 2 mel k-blocks (A ring), then the 2 channel k-blocks of d
+  if (warp == 0 && lane == 0) {
+    tma_prefetch_desc(&tm_x_hi); tma_prefetch_desc(&tm_m_hi);
+    int s = 0; uint32_t pm = 0;
+    for (int kb = 0; kb < nkb; ++kb) {
+      for (int pl = 0; pl < PL; ++pl) {
+        mbar_wait(&empty[s], ((pm >> s) & 1u) ^ 1u);
+        pm ^= 1u << s;
+        mbar_arrive_expect_tx(&full[s], TILE_A);
+        tma_load_3d(slot(s), pl ? &tm_m_lo : &tm_m_hi, &full[s], kb * 64, t0, b);
+        s = (s + 1 == W_NA) ? 0 : s + 1;
+      }
+    }
+  } else if (warp == 2 && lane == 0) {
+    tma_prefetch_desc(&tm_w1_hi); tma_prefetch_desc(&tm_w2_hi);
+    int j = 0; uint32_t pm = 0;
+    auto put = [&](const CUtensorMap* m, int c0, int r0, uint32_t bytes, bool only1) {
+      if (only1) j = 1;
+      mbar_wait(&empty[W_NA + j], ((pm >> j) & 1u) ^ 1u);
+      pm ^= 1u << j;
+      mbar_arrive_expect_tx(&full[W_NA + j], bytes);
+      tma_load_2d(bslot(j), m, &full[W_NA + j], c0, r0);
+      j ^= 1;
+    };
+    for (int kb = 0; kb < nkb + NKB_D; ++kb) {
+      const int col = kb < nkb ? WF_C + kb * 64 : (kb - nkb) * 64;          // w1 columns: pointwise (C) | mel
+      for (int pl = 0; pl < PL; ++pl) put(pl ? &tm_w1_lo : &tm_w1_hi, col, a.w1_row0, 2 * TILE_A, false);
+    }
+    for (int kb = 0; kb < 2; ++kb)
+      for (int pl = 0; pl < PL; ++pl) put(pl ? &tm_w2_lo : &tm_w2_hi, kb * 64, a.w2_row0, WF_N2 * 128, NPASS == 3);
+  } else if (warp == 1 && lane == 0) {
+    int sa = 0, jb = 0; uint32_t cm = 0;
+    auto wait_full = [&](int bar) { mbar_wait(&full[bar], (cm >> bar) & 1u); cm ^= 1u << bar; };
+    // GEMM1: pre[128 x 256] (tanh | sigmoid halves) in TMEM columns 0..255
+    for (int kb = 0; kb < nkb; ++kb) {
+      const int sa_hi = sa; wait_full(sa); sa ^= 1;
+      int sa_lo = 0;
+      if (NPASS == 3) { sa_lo = sa; wait_full(sa); sa ^= 1; }
+      const int jb_hi = jb; wait_full(W_NA + jb); jb ^= 1;     // slots: waited for just before first use, released after last use
+      tc_fence_after_sync();
+      issue_kblock_fast(smem_u32(slot(sa_hi)), smem_u32(bslot(jb_hi)), tmem, IDESC_N256, kb == 0);
+      if (NPASS == 3) {
+        issue_kblock_fast(smem_u32(slot(sa_lo)), smem_u32(bslot(jb_hi)), tmem, IDESC_N256, false);
+        umma_commit(&empty[W_NA + jb_hi]);
+        umma_commit(&empty[sa_lo]);
+        const int jb_lo = jb; wait_full(W_NA + jb); jb ^= 1;
+        tc_fence_after_sync();
+        issue_kblock_fast(smem_u32(slot(sa_hi)), smem_u32(bslot(jb_lo)), tmem, IDESC_N256, false);
+        umma_commit(&empty[W_NA + jb_lo]);
+      } else {
+        umma_commit(&empty[W_NA + jb_hi]);
+      }
+      umma_commit(&empty[sa_hi]);
+    }
+    mbar_wait(d_ready, 0);
+    tc_fence_after_sync();
+    for (int kd = 0; kd < NKB_D; ++kd) {
+      const uint32_t d_hi = smem_u32(slot(W_NS + kd)), d_lo = smem_u32(slot(W_NS + NKB_D + kd));
+      const int jb_hi = jb; wait_full(W_NA + jb); jb ^= 1;
+      tc_fence_after_sync();
+      issue_kblock_fast(d_hi, smem_u32(bslot(jb_hi)), tmem, IDESC_N256, false);
+      if (NPASS == 3) {
+        issue_kblock_fast(d_lo, smem_u32(bslot(jb_hi)), tmem, IDESC_N256, false);
+        umma_commit(&empty[W_NA + jb_hi]);
+        const int jb_lo = jb; wait_full(W_NA + jb); jb ^= 1;
+        tc_fence_after_sync();
+        issue_kblock_fast(d_hi, smem_u32(bslot(jb_lo)), tmem, IDESC_N256, false);
+        umma_commit(&empty[W_NA + jb_lo]);
+      } else {
+        umma_commit(&empty[W_NA + jb_hi]);
+      }
+    }
+    umma_commit(acc1_full);
+    // GEMM2: [res (128) | folded end (16)] = acts x W2^T, reusing TMEM columns 0..143
+    mbar_wait(acts_ready, 0);
+    tc_fence_after_sync();
+    for (int kb = 0; kb < 2; ++kb) {
+      const uint32_t a_hi = smem_u32(slot(kb)), a_lo = smem_u32(slot(2 + kb));
+      if (NPASS == 3) jb = 1;
+      const int jb_hi = jb; wait_full(W_NA + jb); jb ^= 1;
+      tc_fence_after_sync();
+      issue_kblock_fast(a_hi, smem_u32(bslot(jb_hi)), tmem, IDESC_N144, kb == 0);
+      if (NPASS == 3) {
+        issue_kblock_fast(a_lo, smem_u32(bslot(jb_hi)), tmem, IDESC_N144, false);
+        umma_commit(&empty[W_NA + jb_hi]);
+        wait_full(W_NA + 1);                 // W2 lo tile arrives in the same (only) slot
+        tc_fence_after_sync();
+        issue_kblock_fast(a_hi, smem_u32(bslot(1)), tmem, IDESC_N144, false);
+        umma_commit(&empty[W_NA + 1]);
+      } else {
+        umma_commit(&empty[W_NA + jb_hi]);
+      }
+    }
+    umma_commit(acc2_full);
+    if (a.has_res) {
+      // this row's input tiles (the conv's newest row, centre tap) -> units 0..3 for the residual add
+      mbar_wait(acc2_full, 0);
+      mbar_arrive_expect_tx(xold_full, 4 * TILE_A);
+      for (int kb = 0; kb < 2; ++kb)
+        for (int pl = 0; pl < 2; ++pl)
+          asm volatile(
+              "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
+              ::"r"(smem_u32(slot(2 * pl + kb))), "l"(reinterpret_cast<uint64_t>(pl ? &tm_x_lo : &tm_x_hi)), "r"(smem_u32(xold_full)),
+                "r"(kb * 64), "r"(t0), "r"(b), "r"(a.ring_in + a.row % nslot)
+              : "memory");
+    }
+  } else if (warp >= 4) {
+    const int quarter = warp & 3, half = (warp - 4) >> 2, row = quarter * 32 + lane;
+    const uint32_t trow = tmem + ((uint32_t)(quarter * 32) << 16);
+    const bool valid = t0 + row < a.Tp;
+    const size_t m = (size_t)b * a.Tp + (size_t)min(t0 + row, a.Tp - 1);
+    const float4* b1t = reinterpret_cast<const float4*>(b1s);
+    const float4* b1g = reinterpret_cast<const float4*>(b1s + WF_C);
+
+    // the mel k-blocks of GEMM1 run meanwhile
+    wf_depthwise_tile<NPASS>(a, reinterpret_cast<const float*>(smem + S_OFF_DW), reinterpret_cast<const float*>(smem + S_OFF_DWB),
+                             b, t0, warp - 4, lane, slot(W_NS), slot(W_NS + NKB_D));
+    tc_fence_before_sync();
+    fence_proxy_async_smem();
+    mbar_arrive(d_ready);
+    mbar_wait(acc1_full, 0);
+    tc_fence_after_sync();
+    {
+      uint32_t buf[2][32];
+      const int c0 = half * 4;
+      tmem_issue16x2(trow + c0 * 16, trow + WF_C + c0 * 16, buf[0]);
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int c = c0 + i;
+        uint32_t* cur = buf[i & 1];
+        tmem_wait32(cur);
+        if (i + 1 < 4) tmem_issue16x2(trow + (c + 1) * 16, trow + WF_C + (c + 1) * 16, buf[(i + 1) & 1]);
+        float act[16];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const float4 bt = b1t[c * 4 + q], bs = b1g[c * 4 + q];
+          act[4 * q + 0] = gate<NPASS>(__uint_as_float(cur[4 * q + 0]) + bt.x, __uint_as_float(cur[16 + 4 * q + 0]) + bs.x);
+          act[4 * q + 1] = gate<NPASS>(__uint_as_float(cur[4 * q + 1]) + bt.y, __uint_as_float(cur[16 + 4 * q + 1]) + bs.y);
+          act[4 * q + 2] = gate<NPASS>(__uint_as_float(cur[4 * q + 2]) + bt.z, __uint_as_float(cur[16 + 4 * q + 2]) + bs.z);
+          act[4 * q + 3] = gate<NPASS>(__uint_as_float(cur[4 * q + 3]) + bt.w, __uint_as_float(cur[16 + 4 * q + 3]) + bs.w);
+        }
+        store_split16<NPASS == 3>(act, slot(c >> 2), slot(2 + (c >> 2)), row, (c & 3) * 2);
+      }
+    }
+    tc_fence_before_sync();
+    fence_proxy_async_smem();
+    mbar_arrive(acts_ready);
+
+    float4 eold[4];
+    if (half == 0) {
+      const float4* e = reinterpret_cast<const float4*>(a.first ? a.eo_b : a.eo + m * CWG_EO_PAD);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) eold[q] = __ldg(e + q);
+    }
+    mbar_wait(acc2_full, 0);
+    tc_fence_after_sync();
+    if (half == 0) {
+      uint32_t sk[16];
+      tmem_issue16(trow + WF_C, sk);
+      tmem_wait16(sk);
+      if (valid) {
+        float4* e = reinterpret_cast<float4*>(a.eo + m * CWG_EO_PAD);
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          float4 v = eold[q];
+          v.x += __uint_as_float(sk[4 * q]); v.y += __uint_as_float(sk[4 * q + 1]);
+          v.z += __uint_as_float(sk[4 * q + 2]); v.w += __uint_as_float(sk[4 * q + 3]);
+          e[q] = v;
+        }
+      }
+    }
+    if (a.has_res) {
+      const float4* b2v = reinterpret_cast<const float4*>(b2s);
+      uint32_t buf[2][16];
+      const int c0 = half * 4;
+      tmem_issue16(trow + c0 * 16, buf[0]);
+      mbar_wait(xold_full, 0);
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int c = c0 + i;
+        uint32_t* cur = buf[i & 1];
+        tmem_wait16(cur);
+        if (i + 1 < 4) tmem_issue16(trow + (c + 1) * 16, buf[(i + 1) & 1]);
+        uint8_t* thi = slot(c >> 2);
+        uint8_t* tlo = slot(2 + (c >> 2));
+        const uint32_t o0 = sw128_offset(row, (c & 3) * 2), o1 = sw128_offset(row, (c & 3) * 2 + 1);
+        const uint4 h0 = *reinterpret_cast<const uint4*>(thi + o0), h1 = *reinterpret_cast<const uint4*>(thi + o1);
+        const uint4 l0 = *reinterpret_cast<const uint4*>(tlo + o0), l1 = *reinterpret_cast<const uint4*>(tlo + o1);
+        const uint32_t hw[8] = {h0.x, h0.y, h0.z, h0.w, h1.x, h1.y, h1.z, h1.w};
+        const uint32_t lw[8] = {l0.x, l0.y, l0.z, l0.w, l1.x, l1.y, l1.z, l1.w};
+        float r[16];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const float4 bb = b2v[c * 4 + q];
+          r[4 * q] = __uint_as_float(cur[4 * q]) + bb.x; r[4 * q + 1] = __uint_as_float(cur[4 * q + 1]) + bb.y;
+          r[4 * q + 2] = __uint_as_float(cur[4 * q + 2]) + bb.z; r[4 * q + 3] = __uint_as_float(cur[4 * q + 3]) + bb.w;
+        }
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {   // audio += res_skip_acts[:, :C], glow_ax.py:615-620
+          r[2 * j] += __uint_as_float(hw[j] << 16) + __uint_as_float(lw[j] << 16);
+          r[2 * j + 1] += __uint_as_float(hw[j] & 0xFFFF0000u) + __uint_as_float(lw[j] & 0xFFFF0000u);
+        }
+        store_split16<true>(r, thi, tlo, row, (c & 3) * 2);
+      }
+      // each column half owns one 64-channel tile (hi + lo)
+      fence_proxy_async_smem();
+      asm volatile("bar.sync %0, 128;" ::"r"(2 + half) : "memory");
+      if (quarter == 0 && lane == 0) {
+        for (int pl = 0; pl < 2; ++pl)
+          asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
+                       ::"l"(reinterpret_cast<uint64_t>(pl ? &tm_x_lo : &tm_x_hi)), "r"(smem_u32(slot(2 * pl + half))),
+                         "r"(half * 64), "r"(t0), "r"(b), "r"(a.ring_out + a.row % nslot)
+                       : "memory");
+        tma_store_commit();
+        tma_store_wait_read();
+      }
+    }
+    tc_fence_before_sync();
+  }
+  __syncthreads();
+  if (warp == 1) { __syncwarp(); tmem_dealloc(tmem, 256); }
+}
+
 struct WfWorkspace {
-  __nv_bfloat16* x;      // hi plane then lo plane, each [L][3][B][T'][C]
+  __nv_bfloat16* x;      // hi plane then lo plane, each [L][KH][B][T'][C] (KH = kernel_h: 3 for the dense layout)
   __nv_bfloat16* mel_up; // hi, lo planes [B][T'][128]
   float* eo;             // [B*T'][16]
   float* state;          // [B*T'][G] scratch audio state (flows F-1 .. 1)
@@ -411,15 +780,19 @@ void wf_carve(const WfDims& d, void* base, WfWorkspace* ws) {
   ws->eo = (float*)take((size_t)d.BT * CWG_EO_PAD * 4);
   ws->state = (float*)take((size_t)d.BT * d.G * 4);
   ws->mel_up = (__nv_bfloat16*)take((size_t)d.BT * WF_HP * 2 * 2);
-  ws->x = (__nv_bfloat16*)take((size_t)d.L * 3 * d.BT * WF_C * 2 * 2);
+  ws->x = (__nv_bfloat16*)take((size_t)d.L * d.KH * d.BT * WF_C * 2 * 2);
   ws->bytes = off;
 }
 
 int wf_check(const cwg_wf_config* c, int mode, int batch, int t_samples) {
   CWG_REQUIRE(c != nullptr, "cfg is NULL");
   CWG_REQUIRE(mode == CWG_MODE_BF16X3 || mode == CWG_MODE_BF16, "WaveFlow supports the tensor-core modes only");
-  CWG_REQUIRE(c->n_channels == WF_C && c->kernel_h == WF_KH && c->kernel_w == WF_KW,
-              "WaveFlow kernels are built for n_channels=128 and a 3x3 kernel (got %d, %dx%d)", c->n_channels, c->kernel_h, c->kernel_w);
+  CWG_REQUIRE(c->n_channels == WF_C && ((c->kernel_h == WF_KH && c->kernel_w == WF_KW) ||
+                                        (c->kernel_h >= 1 && c->kernel_h <= WF_SEP_MAX_KH && c->kernel_w >= 1 &&
+                                         c->kernel_w <= WF_SEP_MAX_KW && c->kernel_w % 2 == 1)),
+              "the tensor-core WaveFlow kernels take n_channels=128 with a dense or separable 3x3 kernel, or separable in_layers "
+              "of kernel_h <= %d and odd kernel_w <= %d (got %d, %dx%d)", WF_SEP_MAX_KH, WF_SEP_MAX_KW, c->n_channels, c->kernel_h,
+              c->kernel_w);
   CWG_REQUIRE(c->n_group >= 2 && c->n_group <= WF_TC_MAX_GROUP, "n_group must be in [2, %d]", WF_TC_MAX_GROUP);
   CWG_REQUIRE(c->n_mel >= 1 && c->n_mel <= WF_HP, "n_mel must be <= %d", WF_HP);
   CWG_REQUIRE(c->n_flows >= 1 && c->n_layers >= 1 && c->n_layers <= 16, "bad n_flows / n_layers");
@@ -437,6 +810,7 @@ WfDims wf_dims(const cwg_wf_config* c, int batch, int t_samples) {
   WfDims d;
   d.B = batch; d.Tp = t_samples / c->n_group; d.F = c->n_flows; d.L = c->n_layers; d.G = c->n_group; d.M = c->n_mel;
   d.BT = (long long)batch * d.Tp;
+  d.KH = c->kernel_h;
   return d;
 }
 
@@ -452,13 +826,23 @@ void wf_perm(int k, int h, int* idx) {
   }
 }
 
+// Separable in_layers (cwg_wf_weights.dw_w set) run k_wf_sep_tc, everything else the dense 3x3 kernel.
+int wf_check_weights(const cwg_wf_config* c, const cwg_wf_weights* w) {
+  CWG_REQUIRE(w->dw_w != nullptr || (c->kernel_h == WF_KH && c->kernel_w == WF_KW),
+              "a %dx%d WaveFlow in_layer runs on the tensor cores only as a depthwise-separable conv (cwg_wf_weights.dw_w)",
+              c->kernel_h, c->kernel_w);
+  CWG_REQUIRE(w->dw_w == nullptr || w->dw_b != nullptr, "dw_b missing");
+  return 0;
+}
+
 int wf_launch_layer(const cwg_wf_config* cfg, const WfDims& d, const cwg_wf_weights* w, int npass, int flow, int layer,
                     int row, __nv_bfloat16* x, const __nv_bfloat16* mel_up, float* eo, cudaStream_t s) {
-  const size_t xplane = (size_t)d.L * 3 * d.BT * WF_C, mplane = (size_t)d.BT * WF_HP;
+  const bool sep = w->dw_w != nullptr;
+  const size_t xplane = (size_t)d.L * d.KH * d.BT * WF_C, mplane = (size_t)d.BT * WF_HP;
   const uint64_t fl = (uint64_t)d.F * d.L;
   CUtensorMap tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo;
   {
-    uint64_t dims[4] = {WF_C, (uint64_t)d.Tp, (uint64_t)d.B, (uint64_t)d.L * 3};
+    uint64_t dims[4] = {WF_C, (uint64_t)d.Tp, (uint64_t)d.B, (uint64_t)d.L * d.KH};
     uint64_t st[3] = {WF_C * 2, (uint64_t)d.Tp * WF_C * 2, (uint64_t)d.BT * WF_C * 2};
     uint32_t box[4] = {64, 128, 1, 1};
     if (int r = make_map(&tx_hi, x, 4, dims, st, box)) return r;
@@ -466,8 +850,9 @@ int wf_launch_layer(const cwg_wf_config* cfg, const WfDims& d, const cwg_wf_weig
   }
   if (int r = map_act(&tm_hi, mel_up, WF_HP, d.Tp, d.B)) return r;
   if (int r = map_act(&tm_lo, mel_up + mplane, WF_HP, d.Tp, d.B)) return r;
-  if (int r = map_2d(&tw1_hi, w->w1_hi, WF_K1, fl * 2 * WF_C, 256)) return r;
-  if (int r = map_2d(&tw1_lo, w->w1_lo, WF_K1, fl * 2 * WF_C, 256)) return r;
+  const uint64_t k1 = sep ? WF_C + WF_HP : WF_K1;               // separable: pointwise columns | mel
+  if (int r = map_2d(&tw1_hi, w->w1_hi, k1, fl * 2 * WF_C, 256)) return r;
+  if (int r = map_2d(&tw1_lo, w->w1_lo, k1, fl * 2 * WF_C, 256)) return r;
   if (int r = map_2d(&tw2_hi, w->w2_hi, WF_C, fl * WF_N2, WF_N2)) return r;
   if (int r = map_2d(&tw2_lo, w->w2_lo, WF_C, fl * WF_N2, WF_N2)) return r;
   const size_t idx = (size_t)flow * d.L + layer;
@@ -475,11 +860,22 @@ int wf_launch_layer(const cwg_wf_config* cfg, const WfDims& d, const cwg_wf_weig
   a.b1 = w->b1 + idx * 2 * WF_C; a.b2 = w->b2 + idx * WF_C; a.eo_b = w->eo_b + (size_t)flow * CWG_EO_PAD;
   a.eo = eo; a.Tp = d.Tp; a.dil = 1 << layer;
   a.w1_row0 = (int)(idx * 2 * WF_C); a.w2_row0 = (int)(idx * WF_N2);
-  a.ring_in = layer * 3; a.ring_out = (layer + 1) * 3;
+  a.ring_in = layer * d.KH; a.ring_out = (layer + 1) * d.KH;
   a.row = row; a.rows_valid = row + 1 < WF_KH ? row + 1 : WF_KH;
   a.has_res = layer < d.L - 1; a.first = layer == 0;
   dim3 grid((unsigned)((d.Tp + 127) / 128), d.B);
-  if (npass == 3) {
+  if (sep) {
+    a.x = x; a.xplane = (long long)xplane; a.BT = d.BT;
+    a.kh = cfg->kernel_h; a.kw = cfg->kernel_w;
+    a.dw_w = w->dw_w + idx * WF_C * a.kh * a.kw; a.dw_b = w->dw_b + idx * WF_C;
+    if (npass == 3) {
+      if (int r = set_smem(k_wf_sep_tc<3>, S_SMEM)) return r;
+      k_wf_sep_tc<3><<<grid, W_THREADS, S_SMEM, s>>>(tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo, a);
+    } else {
+      if (int r = set_smem(k_wf_sep_tc<1>, S_SMEM)) return r;
+      k_wf_sep_tc<1><<<grid, W_THREADS, S_SMEM, s>>>(tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo, a);
+    }
+  } else if (npass == 3) {
     if (int r = set_smem(k_wf_layer_tc<3>, W_SMEM)) return r;
     k_wf_layer_tc<3><<<grid, W_THREADS, W_SMEM, s>>>(tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo, a);
   } else {
@@ -516,6 +912,7 @@ int cwg_wf_layer(const cwg_wf_config* cfg, const cwg_wf_weights* w, int mode, in
                  void* x_rings, const void* mel_up, float* eo, int batch, int t_samples, void* cuda_stream) {
   if (int r = wf_check(cfg, mode, batch, t_samples)) return r;
   CWG_REQUIRE(w && w->w1_hi && w->w1_lo && w->w2_hi && w->w2_lo && w->b1 && w->b2 && w->eo_b, "missing weight arrays");
+  if (int r = wf_check_weights(cfg, w)) return r;
   CWG_REQUIRE(flow >= 0 && flow < cfg->n_flows && layer >= 0 && layer < cfg->n_layers && row >= 0 && row < cfg->n_group - 1,
               "flow/layer/row out of range");
   WfDims d = wf_dims(cfg, batch, t_samples);
@@ -548,6 +945,7 @@ int cwg_wf_infer_profiled(const cwg_wf_config* cfg, const cwg_wf_weights* w, int
   int ev = 0;
   CWG_REQUIRE(w && w->w1_hi && w->w1_lo && w->w2_hi && w->w2_lo && w->b1 && w->b2 && w->eo_b && w->start_w && w->start_b,
               "missing weight arrays");
+  if (int r = wf_check_weights(cfg, w)) return r;
   CWG_REQUIRE(mel && z && audio && frames >= 1 && pad_frames >= 0, "bad tensor arguments");
   CWG_REQUIRE(workspace != nullptr && ((uintptr_t)workspace % 1024) == 0, "workspace must be 1024-byte aligned");
   WfDims d = wf_dims(cfg, batch, t_samples);
@@ -557,7 +955,7 @@ int cwg_wf_infer_profiled(const cwg_wf_config* cfg, const cwg_wf_weights* w, int
   cudaStream_t s = (cudaStream_t)cuda_stream;
   const int npass = mode == CWG_MODE_BF16X3 ? 3 : 1;
   const int h = d.G, F = d.F, L = d.L;
-  const size_t xplane = (size_t)L * 3 * d.BT * WF_C, slot_elems = (size_t)d.BT * WF_C, mplane = (size_t)d.BT * WF_HP;
+  const size_t xplane = (size_t)L * d.KH * d.BT * WF_C, slot_elems = (size_t)d.BT * WF_C, mplane = (size_t)d.BT * WF_HP;
 
   {   // cond = interpolate(mel) once; every flow's cond layer rides in its W1 columns
     long long n = d.BT * WF_HP;
@@ -589,7 +987,7 @@ int cwg_wf_infer_profiled(const cwg_wf_config* cfg, const cwg_wf_weights* w, int
       p.eo = ws.eo; p.do_couple = i >= 0;
       p.start_w = w->start_w + (size_t)k * WF_C; p.start_b = w->start_b + (size_t)k * WF_C;
       if (j < h - 1) {
-        p.x_hi = ws.x + (size_t)(j % 3) * slot_elems;                   // ring of layer 0
+        p.x_hi = ws.x + (size_t)(j % d.KH) * slot_elems;                // ring of layer 0
         p.x_lo = p.x_hi + xplane;
       }
       k_wf_row<<<row_grid, 256, 0, s>>>(p);

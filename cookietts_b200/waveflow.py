@@ -1,6 +1,7 @@
 """Drop-in for the reference's "ax" model `CookieTTS/_4_mtw/waveglow/efficient_model_ax.py::WaveGlow`
 in its WaveFlow configuration (`waveflow=True`, `WN_2d`, `PermuteHeight`; BASELINE config 5),
-inverse pass only, on sm_100a tensor-core kernels (csrc/cwg_wf.cu).
+inverse pass only, on sm_100a tensor-core kernels (csrc/cwg_wf.cu): the dense 3x3 WN_2d of config 5, and the
+depthwise-separable in_layers (kernel_h <= 7 x odd kernel_w <= 7) of the reference author's trained checkpoints.
 
 Interface mirrored: the ax constructor keywords (efficient_model_ax.py:19-20), the state_dict layout
 (`WN.{k}.WN.{start,end,cond_layers.0,in_layers.i,res_skip_layers.i}`; probe-printed, pinned by
@@ -61,7 +62,8 @@ class WaveFlowPackConfig:
     mix_first: bool = True
     mixing_conv: bool = False    # channel_mixing='1x1conv'
     cond_external: bool = False  # the WN cond path is evaluated by the module (cwg_wf_weights.c_all): no cond columns in w1
-    sep_dw: bool = False         # fp32 mode: separable in_layers stay separable (cwg_wf_weights.dw_w / dw_b + a 1x1 GEMM)
+    sep_dw: bool = False         # separable in_layers stay separable (cwg_wf_weights.dw_w / dw_b + a 1x1 GEMM); the tensor-core
+                                 # modes fold a separable 3x3 into the dense 3x3 kernel instead
 
     @property
     def kx(self) -> int:
@@ -275,8 +277,7 @@ class WaveFlow(nn.Module, AxFrontEndMixin):
             gate=v["gate"], dilations_w=v["dilations_w"], dilations_h=v["dilations_h"], res_skip=v["res_skip"],
             merge_res_skip=v["merge"], wn_speaker_dim=v["speaker_dim"], n_early_every=v["n_early_every"],
             n_early_size=v["n_early_size"], mix_first=v["mix_first"], mixing_conv=v["mixing_conv"],
-            cond_external=v["cond_external"],
-            sep_dw=bool(wn.get("seperable_conv")) and precision == "ffma" and (wn["kernel_size_h"], wn["kernel_size_w"]) != (1, 1))
+            cond_external=v["cond_external"], sep_dw=self._sep_dw(wn, precision))
         self.WN = nn.ModuleList([_Coupling(n_layers=wn["n_layers"], n_channels=wn["n_channels"],
                                            kernel_h=wn["kernel_size_h"], kernel_w=wn["kernel_size_w"],
                                            cond_in_channels=self.wn_cond_in_channels,
@@ -297,6 +298,13 @@ class WaveFlow(nn.Module, AxFrontEndMixin):
         self._packed = None
         self._packed_key = None
         self._workspace = None
+
+    @staticmethod
+    def _sep_dw(wn, precision):
+        """Separable in_layers stay separable (depthwise kernel + pointwise GEMM), except a 1x1 (not separable in the
+        reference, glow_ax.py:520) and, in the tensor-core modes, a 3x3, which is folded into the dense 3x3 kernel."""
+        kernel = (wn["kernel_size_h"], wn["kernel_size_w"])
+        return bool(wn.get("seperable_conv")) and kernel != (1, 1) and (precision == "ffma" or kernel != (3, 3))
 
     def _check_supported(self, a, wn, precision="bf16x3"):
         """Raises for what is not built; returns the precision the model runs in (WN_config variants force "ffma")."""
@@ -360,10 +368,12 @@ class WaveFlow(nn.Module, AxFrontEndMixin):
                  "precision='ffma' takes even n_channels, kernel_size_h <= 16 and odd kernel_size_w <= 15")
             need(a["hop_length"] % a["n_group"] == 0 and a["n_group"] <= 32, "hop_length % n_group == 0 and n_group <= 32")
             need(L <= 16, "n_layers <= 16")
-        else:
-            need(wn["n_channels"] == 128 and wn["kernel_size_h"] == 3 and wn["kernel_size_w"] == 3,
-                 "the tensor-core kernels are built for n_channels=128, kernel 3x3 (precision='ffma' runs other shapes)")
-            need(a["hop_length"] % a["n_group"] == 0 and a["n_group"] <= 16, "hop_length % n_group == 0 and n_group <= 16 (32 with precision='ffma')")
+        else:                        # tensor-core kernels (csrc/cwg_wf.cu): dense 3x3, or separable kernel_h <= 7 x odd kernel_w <= 7
+            kh, kw = wn["kernel_size_h"], wn["kernel_size_w"]
+            need(wn["n_channels"] == 128 and ((kh, kw) == (3, 3) or (self._sep_dw(wn, precision) and kh <= 7 and kw % 2 == 1 and kw <= 7)),
+                 "the tensor-core kernels are built for n_channels=128 with a dense or separable 3x3 kernel, or depthwise-separable "
+                 "in_layers of kernel_size_h <= 7 and odd kernel_size_w <= 7 (precision='ffma' runs other shapes)")
+            need(a["hop_length"] % a["n_group"] == 0 and a["n_group"] <= 32, "hop_length % n_group == 0 and n_group <= 32")
         need(wn.get("upsample_mode", "linear") in ("linear", "nearest"), "upsample_mode must be 'linear' or 'nearest'")
         return precision
 

@@ -241,19 +241,21 @@ int cwg_ax_speaker_bias(const cwg_config* cfg, const float* b1, const float* spk
  * WaveFlow (BASELINE config 5): the reference's "ax" model with waveflow=True
  *   efficient_model_ax.py:279-357  WaveGlow.inverse      efficient_modules.py:42-65  WaveFlowCoupling.inverse
  *   glow_ax.py:556-635             WN_2d.forward          efficient_modules.py:360-403 PermuteHeight
- * Supported subset: channel_mixing='permuteheight', mix_first, upsample_first (model-level
- * F.interpolate of the mel), WN_2d with one 1x1 cond layer, kernel (3,3), dilation_h 1,
- * dilation_w 2^i, n_channels 128, GTU gate, res_skip without merge.  Tensor-core modes only.
+ * Tensor-core modes (CWG_MODE_BF16X3 / CWG_MODE_BF16): channel_mixing='permuteheight', mix_first, upsample_first
+ * (model-level F.interpolate of the mel), WN_2d with one 1x1 cond layer, dilation_h 1, dilation_w 2^i, n_channels 128,
+ * GTU gate, res_skip without merge, n_group <= 32, and either a dense 3x3 in_layer or a depthwise-separable one
+ * (glow_ax.py:525-531) of kernel_h <= 7 x odd kernel_w <= 7 (cwg_wf_weights.dw_w set; the trained checkpoints' 7x7).
+ * CWG_MODE_FFMA runs general shapes and the WN_config variants.
  * ===================================================================================== */
 #define CWG_WF_COND_PAD 128  /* mel channels padded to two 64-wide k-blocks */
 
 typedef struct cwg_wf_config {
   int32_t n_mel;
   int32_t n_flows;
-  int32_t n_group;        /* squeeze height h (<= 16 in the tensor-core modes, <= 32 in CWG_MODE_FFMA) */
+  int32_t n_group;        /* squeeze height h, 2 .. 32 */
   int32_t n_layers;
   int32_t n_channels;     /* 128 */
-  int32_t kernel_h, kernel_w;   /* 3, 3 */
+  int32_t kernel_h, kernel_w;   /* tensor-core modes: 3 x 3, or separable kernel_h <= 7 x odd kernel_w <= 7 */
   int32_t hop_length;
   int32_t upsample_linear;      /* 1: F.interpolate(mode='linear', align_corners=True); 0: 'nearest' */
   /* ABI 5 - WN_config variants of WN_2d, CWG_MODE_FFMA only (the tensor-core kernels take the defaults: all zero) */
@@ -267,9 +269,9 @@ typedef struct cwg_wf_config {
                                 /*    :269-286; cwg_wf_weights.winv); 0: PermuteHeight                                        */
 } cwg_wf_config;
 
-/* K1 = kernel_h*kernel_w*C + CWG_WF_COND_PAD, N2 = C + CWG_EO_PAD */
+/* K1 = kernel_h*kernel_w*C + CWG_WF_COND_PAD (dense in_layers) or C + CWG_WF_COND_PAD (separable), N2 = C + CWG_EO_PAD */
 typedef struct cwg_wf_weights {
-  const uint16_t* w1_hi;   /* [F][L][2C][K1]  col (kh*kw_n + kw)*C + c | 9C + mel channel   */
+  const uint16_t* w1_hi;   /* [F][L][2C][K1]  col (kh*kw_n + kw)*C + c | 9C + mel channel; separable: c | C + mel channel */
   const uint16_t* w1_lo;
   const float*    b1;      /* [F][L][2C]      in_layer bias + cond layer bias slice          */
   const uint16_t* w2_hi;   /* [F][L][N2][C]   rows <C res (0 for last layer; all 0 with merge_res_skip, where the hidden
@@ -294,10 +296,12 @@ typedef struct cwg_wf_weights {
    * cond stacks, a WN-level TransposedUpsampleNet (glow_ax.py:476-505,:565-579) - as [F][batch][2*C*L][T'] fp32.  When set,
    * w1_f32 has no cond columns (K1 = kernel_h*kernel_w*C), b1 holds the in_layer biases only and `mel` is not read. */
   const float*    c_all;
-  /* ABI 5, CWG_MODE_FFMA, optional: depthwise-separable in_layers (glow_ax.py:525-531) kept separable instead of folded to a
-   * dense kernel_h x kernel_w conv (the layout of the reference author's trained checkpoints: 7x7 -> 49x fewer MACs).
-   * dw_w [F][L][C][kernel_h*kernel_w], dw_b [F][L][C]: the depthwise conv; w1_f32 is then [F][L][2C][C + n_mel]
-   * (pointwise weights | cond layer), b1 the pointwise + cond biases. */
+  /* ABI 5, optional: depthwise-separable in_layers (glow_ax.py:525-531) kept separable instead of folded to a dense
+   * kernel_h x kernel_w conv (the layout of the reference author's trained checkpoints: 7x7 -> 49x fewer MACs).
+   * dw_w [F][L][C][kernel_h*kernel_w], dw_b [F][L][C]: the depthwise conv (fp32 in every mode); w1_f32 is then
+   * [F][L][2C][C + n_mel] and w1_hi / w1_lo [F][L][2C][C + CWG_WF_COND_PAD] (pointwise weights | cond layer), b1 the
+   * pointwise + cond biases.  The tensor-core modes run it in one kernel per layer step (k_wf_sep_tc: the depthwise conv
+   * on the CUDA cores feeds the pointwise GEMM through shared memory); NULL there means a dense 3x3 in_layer. */
   const float*    dw_w;
   const float*    dw_b;
 } cwg_wf_weights;
@@ -307,8 +311,9 @@ size_t cwg_wf_workspace_bytes(const cwg_wf_config* cfg, int mode, int batch, int
 /* WaveGlow.inverse of the ax model (explicit latent): mel [batch][n_mel][frames] fp32, zero-extended
  * to frames + pad_frames (infer's artifact_trimming pad, efficient_model_ax.py:370-371) and
  * interpolated to T' = t_samples / n_group steps; z [batch][t_samples] standard normal (scaled by
- * sigma inside); audio [batch][t_samples] out.  mode: CWG_MODE_BF16X3 or CWG_MODE_BF16 (tcgen05 kernels: C = 128, 3x3,
- * n_group <= 16, n_mel <= 128), or CWG_MODE_FFMA (exact fp32 on the CUDA cores, general shapes; csrc/cwg_wf_ffma.cu). */
+ * sigma inside); audio [batch][t_samples] out.  mode: CWG_MODE_BF16X3 or CWG_MODE_BF16 (tcgen05 kernels: C = 128, dense
+ * 3x3 or separable kernel_h <= 7 x odd kernel_w <= 7, n_group <= 32, n_mel <= 128), or CWG_MODE_FFMA (exact fp32 on the
+ * CUDA cores, general shapes; csrc/cwg_wf_ffma.cu). */
 int cwg_wf_infer(const cwg_wf_config* cfg, const cwg_wf_weights* w, int mode,
                  const float* mel, int frames, int pad_frames, const float* z, float sigma,
                  float* audio, void* workspace, size_t workspace_bytes,
@@ -324,9 +329,9 @@ int cwg_wf_infer_profiled(const cwg_wf_config* cfg, const cwg_wf_weights* w, int
 
 int cwg_wf_launch_count(const cwg_wf_config* cfg);
 
-/* Stage entry point (tests): one WN_2d layer of one autoregressive row step.
- * x_rings: bf16 planes (hi then lo), each [L][3][batch][T'][C]; mel_up planes [batch][T'][128];
- * reads ring slots of rows row, row-1, row-2 of layer `layer`, writes slot row%3 of layer+1. */
+/* Stage entry point (tests): one WN_2d layer of one autoregressive row step, either layout (tensor-core modes).
+ * x_rings: bf16 planes (hi then lo), each [L][kernel_h][batch][T'][C]; mel_up planes [batch][T'][128];
+ * reads ring slots of rows row .. row-kernel_h+1 (those >= 0) of layer `layer`, writes slot row%kernel_h of layer+1. */
 int cwg_wf_layer(const cwg_wf_config* cfg, const cwg_wf_weights* w, int mode, int flow, int layer, int row,
                  void* x_rings, const void* mel_up, float* eo, int batch, int t_samples, void* cuda_stream);
 
