@@ -49,7 +49,8 @@ EXPORTS = ("cwg_abi_version", "cwg_last_error", "cwg_workspace_bytes", "cwg_laun
            "cwg_denoise_workspace_bytes", "cwg_denoise_out_samples", "cwg_stft_mean_magnitude", "cwg_denoise", "cwg_pcm16",
            "cwg_conv1d", "cwg_conv_transpose1d", "cwg_resample1d", "cwg_deemphasis",
            "cwg_fd_workspace_bytes", "cwg_fd_launch_count", "cwg_fd_inverse",
-           "cwg_axg_workspace_bytes", "cwg_axg_launch_count", "cwg_axg_flow", "cwg_group_transpose")
+           "cwg_axg_workspace_bytes", "cwg_axg_launch_count", "cwg_axg_flow", "cwg_group_transpose",
+           "cwg_pack_forward", "cwg_forward_workspace_bytes", "cwg_forward_launch_count", "cwg_forward")
 
 
 class CwgError(RuntimeError):
@@ -113,6 +114,16 @@ def load():
                                       C.c_int, C.c_int, C.c_void_p, C.c_float,
                                       C.c_void_p, C.c_void_p, C.c_void_p,
                                       C.c_int, C.c_int, C.c_void_p]
+    lib.cwg_pack_forward.restype = C.c_int
+    lib.cwg_pack_forward.argtypes = [C.POINTER(CwgConfig), C.POINTER(CwgTensor), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.cwg_forward_workspace_bytes.restype = C.c_size_t
+    lib.cwg_forward_workspace_bytes.argtypes = [C.POINTER(CwgConfig), C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.cwg_forward_launch_count.restype = C.c_int
+    lib.cwg_forward_launch_count.argtypes = [C.POINTER(CwgConfig), C.c_int]
+    lib.cwg_forward.restype = C.c_int
+    lib.cwg_forward.argtypes = [C.POINTER(CwgConfig), C.POINTER(CwgWeights), C.c_void_p, C.c_void_p, C.c_int,
+                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p]
     lib.cwg_denoise_workspace_bytes.restype = C.c_size_t
     lib.cwg_denoise_workspace_bytes.argtypes = [C.c_int] * 4
     lib.cwg_denoise_out_samples.restype = C.c_int

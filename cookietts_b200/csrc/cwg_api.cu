@@ -328,6 +328,149 @@ int cwg_infer_profiled(const cwg_config* cfg, const cwg_weights* w, int mode,
 }
 
 // ---------------------------------------------------------------------------------------------
+// Forward direction (audio -> z, log_s, log det W): NVIDIA's WaveGlow.forward, of which glow.py is derived.  Flows run
+// k = 0 .. F-1; flow k mixes with W_k, runs WN_k on audio_0 and applies audio_1 = exp(log_s) * audio_1 + b.  The WN work
+// is the launch sequence of cwg_infer; the flow boundaries are cwg_forward.cu's.
+// ---------------------------------------------------------------------------------------------
+namespace {
+struct FwdLayout {
+  Dims d;           // layer dims: T' = t_samples / n_group per utterance (Tm = tf, the frames the cond GEMM runs on)
+  Dims dc;          // cond GEMM dims: tf = ceil(t_samples / hop) frames, tf * P group-steps per utterance
+  size_t ls_part, z2_part, cond, mel, bytes;   // byte offsets of the extra regions (cond / mel: 0 = not needed)
+};
+
+int fwd_check(const cwg_config* cfg, int mode, int batch, int t_mel, int t_samples) {
+  if (int r = check_config(cfg)) return r;
+  if (int r = check_mode(cfg, mode)) return r;
+  CWG_REQUIRE(batch >= 1 && t_mel >= 1, "batch and t_mel must be >= 1");
+  CWG_REQUIRE(t_samples >= cfg->n_group && t_samples % cfg->n_group == 0,
+              "t_samples must be a positive multiple of n_group = %d (got %d)", cfg->n_group, t_samples);
+  CWG_REQUIRE((long long)t_samples <= (long long)t_mel * cfg->hop_length,
+              "t_samples = %d exceeds t_mel * hop_length = %lld: the upsampled mel must cover the audio", t_samples,
+              (long long)t_mel * cfg->hop_length);
+  CWG_REQUIRE((long long)batch * ((t_samples + cfg->hop_length - 1) / cfg->hop_length) * (cfg->hop_length / cfg->n_group) <
+              (1ll << 31) / 4, "batch * T' too large for one call; split the batch");
+  return 0;
+}
+
+FwdLayout fwd_layout(const cwg_config* cfg, int mode, int batch, int t_mel, int t_samples) {
+  FwdLayout l;
+  const int tf = (t_samples + cfg->hop_length - 1) / cfg->hop_length;
+  l.dc = make_dims(cfg, batch, tf);
+  l.d = l.dc;
+  l.d.Tp = t_samples / cfg->n_group;
+  l.d.BT = (long long)batch * l.d.Tp;
+  Workspace ws;
+  carve(l.d, mode, nullptr, &ws);
+  size_t off = ws.bytes;
+  auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 1024); return o; };
+  const size_t nblk = (size_t)fwd_blocks(l.d);
+  l.ls_part = take((size_t)l.d.F * batch * nblk * sizeof(double));
+  l.z2_part = take((size_t)batch * nblk * sizeof(double));
+  l.cond = l.dc.Tp != l.d.Tp ? take((size_t)l.dc.BT * l.d.H * 4) : 0;     // every cond format is 4 bytes per element
+  l.mel = t_mel != tf ? take((size_t)batch * l.d.M * tf * sizeof(float)) : 0;
+  l.bytes = off;
+  return l;
+}
+}  // namespace
+
+size_t cwg_forward_workspace_bytes(const cwg_config* cfg, int mode, int batch, int t_mel, int t_samples) {
+  if (fwd_check(cfg, mode, batch, t_mel, t_samples)) return 0;
+  return fwd_layout(cfg, mode, batch, t_mel, t_samples).bytes + 1024;
+}
+
+int cwg_forward_launch_count(const cwg_config* cfg, int mode) {
+  const int n = cwg_launch_count(cfg, mode);
+  return n < 0 ? n : n + 1;       // the inverse pass's sequence (one boundary per flow plus one) + the final reduction
+}
+
+int cwg_forward(const cwg_config* cfg, const cwg_weights* w, const float* w_fwd, const double* logdet, int mode,
+                const float* mel, const float* cond_bias, const float* audio, int t_samples,
+                float* z, float* log_s, double* logp_terms,
+                void* workspace, size_t workspace_bytes, int batch, int t_mel, void* cuda_stream) {
+  if (int r = fwd_check(cfg, mode, batch, t_mel, t_samples)) return r;
+  if (int r = check_run(cfg, w, mode, batch, (t_samples + cfg->hop_length - 1) / cfg->hop_length)) return r;
+  CWG_REQUIRE(w_fwd && logdet && mel && cond_bias && audio && z && logp_terms, "NULL tensor argument");
+  CWG_REQUIRE(workspace != nullptr && ((uintptr_t)workspace % 1024) == 0, "workspace must be 1024-byte aligned");
+  const FwdLayout l = fwd_layout(cfg, mode, batch, t_mel, t_samples);
+  CWG_REQUIRE(l.bytes <= workspace_bytes, "workspace too small: need %zu, got %zu", l.bytes, workspace_bytes);
+  const Dims& d = l.d;
+  Workspace ws;
+  carve(d, mode, workspace, &ws);
+  char* base = (char*)workspace;
+  double* ls_part = (double*)(base + l.ls_part);
+  double* z2_part = (double*)(base + l.z2_part);
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  const bool tc = mode != CWG_MODE_FFMA;
+  const int npass = mode_npass(mode), xfmt = mode_xfmt(mode);
+  const int F = cfg->n_flows, L = cfg->n_layers, tf = l.dc.Tm;
+  const size_t nblk = (size_t)fwd_blocks(d);
+
+  CWG_CHECK_CUDA(cudaMemsetAsync(ws.status, 0, sizeof(int), s));     // status word as in cwg_infer (cwg_infer_status)
+  set_range_flag(mode == CWG_MODE_F16F8 ? ws.status : nullptr);
+  auto run = [&]() -> int {
+  // the cond GEMM reads [B][n_mel][tf]: a longer mel is cut to the tf frames the audio needs (ConvTranspose1d is causal
+  // in frames: sample o depends on frames <= o / hop only)
+  const float* melc = mel;
+  if (l.mel) {
+    melc = (const float*)(base + l.mel);
+    CWG_CHECK_CUDA(cudaMemcpy2DAsync((void*)melc, (size_t)tf * 4, mel, (size_t)t_mel * 4, (size_t)tf * 4,
+                                     (size_t)batch * d.M, cudaMemcpyDeviceToDevice, s));
+  }
+  void* h2 = tc ? (void*)ws.h2b : (void*)ws.h2;
+  void* h2c = l.cond ? (void*)(base + l.cond) : h2;       // T % hop != 0: cond of tf * P steps, compacted to T' below
+  // One fp32 plane of one utterance already holds its first T' rows in place; every other layout needs the compaction
+  // (the offsets of the lo / e5m2 planes and of utterance b > 0 depend on the row count)
+  const bool compact = l.cond && (tc || batch > 1);
+  const float* h2f = compact ? ws.h2 : (const float*)h2c;  // cond rows of the fp32 layers
+  void* x0 = tc ? (void*)ws.xb[0] : (void*)ws.x[0];
+  void* a0 = (tc && fold_active(d, w)) ? ws.a0 : nullptr;
+  // z = audio, then W_0 and the start conv of flow 0
+  if (int r = launch_fwd_boundary(cfg, d, w, w_fwd, xfmt, -1, 0, audio, z, nullptr, nullptr, nullptr, nullptr, x0, a0, s)) return r;
+  size_t ls_off = 0;
+  for (int k = 0; k < F; ++k) {
+    if (tc) {
+      if (int r = launch_cond_tc(l.dc, w, npass, k, k == 0 ? melc : nullptr, cond_bias, (__nv_bfloat16*)h2c, ws.mel4, s)) return r;
+    } else {
+      if (int r = launch_cond_ffma(l.dc, w, k, melc, cond_bias, (float*)h2c, s)) return r;
+    }
+    if (compact) {
+      // per plane: the first T' of the tf * P rows of every utterance (planes: fp32 | bf16 hi, lo | fp16, e5m2, e5m2)
+      const int ne[3] = {xfmt == 0 ? 4 : 2, xfmt == 0 ? 0 : (xfmt == 1 ? 2 : 1), xfmt == 2 ? 1 : 0};
+      size_t so = 0, dof = 0;
+      for (int q = 0; q < 3 && ne[q]; ++q) {
+        const size_t row = (size_t)d.H * ne[q];
+        CWG_CHECK_CUDA(cudaMemcpy2DAsync((char*)h2 + dof, (size_t)d.Tp * row, (const char*)h2c + so, (size_t)l.dc.Tp * row,
+                                         (size_t)d.Tp * row, (size_t)batch, cudaMemcpyDeviceToDevice, s));
+        so += (size_t)l.dc.BT * row;
+        dof += (size_t)d.BT * row;
+      }
+    }
+    for (int i = 0; i < L; ++i) {
+      if (tc) {
+        if (int r = layer_tc(cfg, d, w, npass, k, i, ws, z, s)) return r;
+      } else {
+        if (int r = launch_layer_ffma(d, w, k, i, ws.x[i & 1], ws.x[(i + 1) & 1], h2f, ws.eo, ws.pre, ws.acts, s)) return r;
+      }
+    }
+    int n_rem, n_half;
+    flow_channels(cfg, k, &n_rem, &n_half);
+    float* ls_k = log_s ? log_s + ls_off : nullptr;
+    ls_off += (size_t)batch * n_half * d.Tp;
+    // coupling of flow k, then W_{k+1} and the start conv of flow k+1 (the last boundary reduces z^2 instead)
+    if (int r = launch_fwd_boundary(cfg, d, w, w_fwd, xfmt, k, k + 1 < F ? k + 1 : -1, nullptr, z, ws.eo, ls_k,
+                                    ls_part + (size_t)k * batch * nblk, z2_part, x0, a0, s)) return r;
+  }
+  return launch_fwd_reduce(d, ls_part, z2_part, logdet + F, logp_terms, s);
+  };
+  const int rc = run();
+  set_range_flag(nullptr);
+  if (rc) return rc;
+  if (mode == CWG_MODE_F16F8) return launch_nonfinite(z, (size_t)batch * t_samples, ws.status, s, false);
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
 // ax WaveGlow (waveflow=False): efficient_model_ax.py:279-357 with AffineCouplingBlock.inverse
 // (efficient_modules.py:94-105), glow_ax.WN.forward (:375-418), InvertibleConv1x1.inverse (:269-286)
 // or PermuteHeight as the channel mixing (packed as a permutation matrix in `winv`).

@@ -215,6 +215,38 @@ __global__ void k_winv(const float* __restrict__ W, int n, int mg, float* __rest
     for (int j = 0; j < mg; ++j) out[i * mg + j] = (i < n && j < n) ? (float)a[i][n + j] : 0.f;
 }
 
+// Forward direction: W itself zero-padded to [mg][mg], and log det W from an fp64 LU with partial pivoting.
+// logdet[flow] follows torch.logdet (NaN for det < 0, -inf for det = 0); logdet[n_flows + flow] = log|det W|.
+__global__ void k_wfwd(const float* __restrict__ W, int n, int mg, int flow, int n_flows, float* __restrict__ out,
+                       double* __restrict__ logdet) {
+  __shared__ double a[CWG_MAX_GROUP][CWG_MAX_GROUP];
+  if (threadIdx.x != 0) return;
+  for (int i = 0; i < mg; ++i)
+    for (int j = 0; j < mg; ++j) out[i * mg + j] = (i < n && j < n) ? W[i * n + j] : 0.f;
+  for (int i = 0; i < n; ++i)
+    for (int j = 0; j < n; ++j) a[i][j] = (double)W[i * n + j];
+  double logabs = 0.0;
+  int neg = 0;
+  for (int col = 0; col < n; ++col) {
+    int piv = col;
+    for (int r = col + 1; r < n; ++r) if (fabs(a[r][col]) > fabs(a[piv][col])) piv = r;
+    if (a[piv][col] == 0.0) { logabs = -INFINITY; neg = 0; break; }
+    if (piv != col) {
+      neg ^= 1;
+      for (int j = col; j < n; ++j) { const double t = a[col][j]; a[col][j] = a[piv][j]; a[piv][j] = t; }
+    }
+    const double d = a[col][col];
+    if (d < 0.0) neg ^= 1;
+    logabs += log(fabs(d));
+    for (int r = col + 1; r < n; ++r) {
+      const double f = a[r][col] / d;
+      if (f != 0.0) for (int j = col; j < n; ++j) a[r][j] -= f * a[col][j];
+    }
+  }
+  logdet[flow] = neg ? (double)NAN : logabs;
+  logdet[n_flows + flow] = logabs;
+}
+
 // cond_bias[b][f][h] = cond_b_base[f][h] + sum_e cond_w_spk[f][h][e] * speaker_embed_f[ids[b]][e]   (glow.py:193-196)
 __global__ void k_cond_bias(const float* __restrict__ base, const float* __restrict__ wspk, const float* __restrict__ emb,
                             const long long* __restrict__ ids, int F, int H, int E, int S, float* __restrict__ out) {
@@ -501,6 +533,25 @@ int cwg_pack_weights(const cwg_config* cfg, int mode, const cwg_tensor* sd, int 
     CWG_CHECK_CUDA(cudaGetLastError());
   }
   *out = w;
+  return 0;
+}
+
+int cwg_pack_forward(const cwg_config* cfg, const cwg_tensor* sd, int n_tensors, float* w_fwd, double* logdet,
+                     void* cuda_stream) {
+  CWG_REQUIRE(cfg && sd && w_fwd && logdet, "cwg_pack_forward: NULL argument");
+  CWG_REQUIRE(cfg->n_group % 2 == 0 && cfg->n_group >= 2 && cfg->n_group <= CWG_MAX_GROUP && cfg->n_flows >= 1 &&
+              cfg->n_early_every >= 1, "bad configuration");
+  const int F = cfg->n_flows, mg = CWG_GROUP_PAD(cfg->n_group);
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  char nm[160];
+  for (int k = 0; k < F; ++k) {
+    int n_rem, n_half;
+    flow_channels(cfg, k, &n_rem, &n_half);
+    const float* Wm;
+    snprintf(nm, sizeof(nm), "convinv.%d.conv.weight", k); if (int r = need(sd, n_tensors, nm, (long long)n_rem * n_rem, &Wm)) return r;
+    k_wfwd<<<1, 32, 0, s>>>(Wm, n_rem, mg, k, F, w_fwd + (size_t)k * mg * mg, logdet);
+  }
+  CWG_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
 

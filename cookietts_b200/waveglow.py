@@ -4,8 +4,10 @@ Mirrors the interface of the reference class `CookieTTS/_4_mtw/waveglow/glow.py:
 same constructor kwargs (`WaveGlow(**waveglow_config)`, glow.py:226-227 and `WN_config`
 :116-117), same parameter names/shapes (so `load_state_dict(checkpoint['model'])` of a
 reference checkpoint works unchanged, SURVEY Appendix A), same
-`infer(spect, speaker_id=None, sigma=1.0)` call.  Only the inverse pass is implemented
-(north_star scope): `forward` (the training direction) raises.
+`infer(spect, speaker_id=None, sigma=1.0)` call.  `forward((spect, audio))` runs the other direction
+(audio -> z, log_s per flow, log_det_W per flow) without gradients, for scoring and encoding audio;
+`encode` and `log_prob` are its flat-latent and per-utterance-likelihood forms.  Training (a backward
+pass) is not implemented: `forward` raises when autograd would need one.
 
 There is no CPU or PyTorch fallback: `infer` needs a CUDA device and the in-tree
 `libcwg.so`; otherwise it raises.
@@ -150,8 +152,134 @@ class WaveGlow(nn.Module):
         time here, so this is a no-op kept for call-site compatibility."""
         return model
 
-    def forward(self, *a, **kw):
-        raise NotImplementedError("only the inverse pass (infer) is in scope of this implementation")
+    # ------------------------------------------------------------------ forward direction (audio -> z), no grad
+    def forward(self, forward_input, *, speaker_ids=None):
+        """`glow.py`'s `WaveGlow.forward` for evaluation: `forward_input` = (spect, audio) or (spect, audio, speaker_ids),
+        spect [B, n_mel, T_mel], audio [B, T] with T % n_group == 0 and 0 < T <= T_mel*hop.  Returns the reference's tuple
+        (z [B, n_group, T'], log_s_list with log_s_list[k] [B, n_half_k, T'], log_det_W_list with 0-dim
+        log_det_W_list[k] = B*T'*torch.logdet(W_k)), fp32 on the module's device.
+
+        There is no backward pass: with grad mode on and a parameter that requires grad this raises instead of returning
+        tensors a training loop would silently not learn from; wrap the call in torch.no_grad() / torch.inference_mode()."""
+        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
+            raise RuntimeError("cookietts_b200.WaveGlow.forward has no backward pass (training is not implemented); "
+                               "call it under torch.no_grad() or torch.inference_mode()")
+        if len(forward_input) == 3:
+            spect, audio, ids = forward_input
+            speaker_ids = ids if speaker_ids is None else speaker_ids
+        elif len(forward_input) == 2:
+            spect, audio = forward_input
+        else:
+            raise ValueError("forward_input must be (spect, audio) or (spect, audio, speaker_ids)")
+        z, log_s, _, logdet = self._forward(spect, audio, speaker_ids, want_log_s=True)
+        pc = self.pack_config
+        B, T = z.shape
+        tp = T // pc.n_group
+        out = z.view(B, tp, pc.n_group).transpose(1, 2).contiguous()
+        log_s_list, off = [], 0
+        for _, n_half in pc.flow_channels():
+            log_s_list.append(log_s[off:off + B * n_half * tp].view(B, n_half, tp))
+            off += B * n_half * tp
+        log_det_W_list = [(B * tp * logdet[k]).float() for k in range(pc.n_flows)]
+        return out, log_s_list, log_det_W_list
+
+    @torch.no_grad()
+    def encode(self, spect, audio, speaker_id=None, *, speaker_ids=None) -> torch.Tensor:
+        """audio [B, T] -> z [B, T] in this repo's latent layout (z[b, s*n_group + c], the layout `infer(z=...)` takes):
+        `infer(spect, z=encode(spect, x), sigma=1.0)` reproduces x.  The forward pass without storing log_s."""
+        z, _, _, _ = self._forward(spect, audio, speaker_id if speaker_id is not None else speaker_ids, want_log_s=False)
+        return z
+
+    @torch.no_grad()
+    def log_prob(self, spect, audio, sigma=1.0, speaker_id=None, *, speaker_ids=None) -> torch.Tensor:
+        """Log-density of each utterance in nats, float64 [B]:
+            sum_i -z_i^2 / (2 sigma^2) - (T/2) log(2 pi sigma^2) + sum_k sum log_s_k + T' * sum_k log|det W_k|
+        with every sum reduced on the device in a fixed order (identical calls give identical results).  It relates to
+        the reference's loss by
+            WaveGlowLoss(sigma)(forward(...)) == (-sum_b log_prob_b - B * (T/2) * log(2 pi sigma^2)) / (B * T).
+        `forward`'s log_det_W_list follows torch.logdet, which is NaN for det W < 0; this uses log|det W|.  The two agree
+        for every W the reference's initialisation (det W = +1) and training (det W never crosses 0) can reach."""
+        z, _, terms, _ = self._forward(spect, audio, speaker_id if speaker_id is not None else speaker_ids, want_log_s=False)
+        T = z.shape[1]
+        s2 = float(sigma) ** 2
+        return -terms[:, 0] / (2.0 * s2) - 0.5 * T * np.log(2.0 * np.pi * s2) + terms[:, 1] + terms[:, 2]
+
+    def forward_launch_count(self) -> int:
+        """Kernels launched by one `encode` / `forward` / `log_prob` call in the current precision mode."""
+        lib = _cabi.load()
+        # cwg_forward's kernels + the k_cond_bias launch of cwg_cond_bias that waveglow_forward issues before it
+        return int(lib.cwg_forward_launch_count(_cabi.make_config(self.pack_config), _cabi.MODES[self.precision])) + 1
+
+    def _ensure_packed_forward(self) -> torch.Tensor:
+        """W_k padded [F][MG][MG] fp32 + logdet [2][F] fp64 in one device blob (cwg_pack_forward).  It lives in the same
+        cache as the packed weights (key "forward"), so a weight change and `invalidate()` drop it together with them."""
+        self._ensure_packed()
+        if "forward" not in self._packs:
+            sd = self.state_dict()
+            names = [k for k in sd.keys() if k.startswith("convinv.")]
+            self._packs["forward"] = _torch_ops.load().waveglow_pack_forward([sd[k] for k in names], "\n".join(names),
+                                                                             self._cfg_list)
+        return self._packs["forward"]
+
+    def _forward(self, spect, audio, speaker_id, want_log_s):
+        """-> (z [B, T], log_s flat (empty unless want_log_s), logp_terms [B, 3] fp64, logdet [F] fp64 (torch.logdet))"""
+        dev = self._device()
+        if dev.type != "cuda":
+            raise RuntimeError("cookietts_b200.WaveGlow.forward needs the module on a CUDA device (no CPU fallback)")
+        if self.precision not in _cabi.MODES:
+            raise ValueError(f"precision must be one of {list(_cabi.MODES)}")
+        pc = self.pack_config
+        if spect.dim() != 3 or spect.shape[1] != pc.n_mel or spect.shape[0] == 0 or spect.shape[2] == 0:
+            raise ValueError(f"spect must be [B, {pc.n_mel}, T_mel] with B, T_mel > 0, got {tuple(spect.shape)}")
+        batch, t_mel = int(spect.shape[0]), int(spect.shape[2])
+        if audio.dim() != 2 or audio.shape[0] != batch:
+            raise ValueError(f"audio must be [B = {batch}, T], got {tuple(audio.shape)}")
+        T = int(audio.shape[1])
+        if T <= 0 or T % pc.n_group or T > t_mel * pc.hop_length:
+            raise ValueError(f"audio length T = {T} must be a positive multiple of n_group = {pc.n_group} and at most "
+                             f"T_mel * hop_length = {t_mel * pc.hop_length}")
+        speaker_id = self._check_speaker_ids(batch, speaker_id)
+        mode = _cabi.MODES[self.precision]
+        mel = spect.to(device=dev, dtype=torch.float32).contiguous()
+        x = audio.to(device=dev, dtype=torch.float32).contiguous()
+        with torch.cuda.device(dev):
+            ops = _torch_ops.load()
+            fwd = self._ensure_packed_forward()
+            z, log_s, terms, status = ops.waveglow_forward(self._packed, fwd, self._cfg_list, mode, self._embed_dim,
+                                                           self._n_speakers, mel, speaker_id, x, want_log_s)
+            if self.precision == "f16f8" and self.range_guard and not torch.cuda.is_current_stream_capturing():
+                # as in infer: the fp16 planes' range flag (or a NaN / Inf in z) re-runs the call in bf16x3
+                self.last_status = int(status.item())
+                if self.last_status:
+                    import warnings
+                    warnings.warn(f"cookietts_b200.WaveGlow: f16f8 range guard tripped (status {self.last_status}); "
+                                  "re-running this call in bf16x3", RuntimeWarning)
+                    self.fallbacks += 1
+                    self._ensure_packed("bf16x3")
+                    z, log_s, terms, _ = ops.waveglow_forward(self._packs["bf16x3"][0], fwd, self._cfg_list,
+                                                              _cabi.MODES["bf16x3"], self._embed_dim, self._n_speakers,
+                                                              mel, speaker_id, x, want_log_s)
+        mg = 16 if pc.n_group <= 16 else 32
+        logdet = fwd[pc.n_flows * mg * mg * 4:].view(torch.float64)[:pc.n_flows]
+        return z, log_s, terms, logdet
+
+    def _check_speaker_ids(self, batch: int, speaker_id):
+        """Host-side speaker-id checks shared by infer and forward: None for single-speaker models, else int64 [batch]."""
+        if self.multispeaker and speaker_id is None:
+            # the reference fails on a shape mismatch in cond_layers[0] here (glow.py:193-199)
+            raise ValueError("this model has speaker embeddings: pass speaker_id / speaker_ids")
+        if not self.multispeaker:
+            return None
+        speaker_id = torch.as_tensor(speaker_id).reshape(-1).cpu()          # host copy: the range check costs no kernel
+        if speaker_id.numel() not in (1, batch):
+            # glow.py:195 concatenates the embedding onto the mel along channels: one id per utterance
+            raise ValueError(f"speaker_id must hold 1 or batch = {batch} entries, got {speaker_id.numel()}")
+        n_spk = self.WN[0].speaker_embed.weight.shape[0]
+        if int(speaker_id.min()) < 0 or int(speaker_id.max()) >= n_spk:
+            raise IndexError(f"speaker_id out of range for an embedding table of {n_spk} rows")   # nn.Embedding raises too
+        if speaker_id.numel() == 1 and batch > 1:
+            speaker_id = speaker_id.expand(batch)
+        return speaker_id.long().contiguous()
 
     # ------------------------------------------------------------------ packing cache
     def _weights_key(self):
@@ -270,22 +398,7 @@ class WaveGlow(nn.Module):
         mode = _cabi.MODES[self.precision]
         if speaker_id is None:
             speaker_id = speaker_ids
-        if self.multispeaker and speaker_id is None:
-            # the reference fails on a shape mismatch in cond_layers[0] here (glow.py:193-199)
-            raise ValueError("this model has speaker embeddings: pass speaker_id / speaker_ids")
-        if self.multispeaker:
-            speaker_id = torch.as_tensor(speaker_id).reshape(-1).cpu()          # host copy: the range check costs no kernel
-            if speaker_id.numel() not in (1, spect.shape[0]):
-                # glow.py:195 concatenates the embedding onto the mel along channels: one id per utterance
-                raise ValueError(f"speaker_id must hold 1 or batch = {spect.shape[0]} entries, got {speaker_id.numel()}")
-            n_spk = self.WN[0].speaker_embed.weight.shape[0]
-            if int(speaker_id.min()) < 0 or int(speaker_id.max()) >= n_spk:
-                raise IndexError(f"speaker_id out of range for an embedding table of {n_spk} rows")   # nn.Embedding raises too
-            if speaker_id.numel() == 1 and spect.shape[0] > 1:
-                speaker_id = speaker_id.expand(spect.shape[0])
-            speaker_id = speaker_id.long().contiguous()
-        else:
-            speaker_id = None
+        speaker_id = self._check_speaker_ids(spect.shape[0], speaker_id)
         pc = self.pack_config
         if spect.dim() != 3 or spect.shape[1] != pc.n_mel:
             raise ValueError(f"spect must be [B, {pc.n_mel}, T_mel], got {tuple(spect.shape)}")

@@ -211,6 +211,36 @@ int cwg_flow_boundary(const cwg_config* cfg, const cwg_weights* w, int mode,
                       float* audio, const float* eo, void* x_out,
                       int batch, int t_mel, void* cuda_stream);
 
+/* ---- forward direction: audio -> z, log_s, log det W (no-grad evaluation; NVIDIA WaveGlow.forward) ----------------
+ * Flows run k = 0 .. F-1: early channels leave at k % n_early_every == 0, k > 0 (they stay in their columns of the
+ * [batch][T'][n_group] audio state, which ends as z in the repo's layout z[b, s*n_group + c]); audio = W_k audio;
+ * (b, log_s) = WN_k(audio_0, cond); audio_1 = exp(log_s) * audio_1 + b.  The cond is the upsampled mel cut to t_samples.
+ *
+ * Mixing matrices for the forward direction, from the state_dict's convinv.{k}.conv.weight (device fp32):
+ *   w_fwd  [F][MG][MG] fp32 device out: W_k zero-padded (MG = CWG_GROUP_PAD(n_group))
+ *   logdet [2][F] fp64 device out: logdet[k] = log det W_k as torch.logdet gives it (NaN for det < 0, -inf for det = 0),
+ *          logdet[F + k] = log|det W_k|; fp64 LU with partial pivoting. */
+int cwg_pack_forward(const cwg_config* cfg, const cwg_tensor* sd, int n_tensors, float* w_fwd, double* logdet,
+                     void* cuda_stream);
+
+/* Bytes of device workspace cwg_forward needs. 0 on error (cwg_last_error says why). */
+size_t cwg_forward_workspace_bytes(const cwg_config* cfg, int mode, int batch, int t_mel, int t_samples);
+
+/* Kernels cwg_forward launches (device-to-device copies not counted). */
+int cwg_forward_launch_count(const cwg_config* cfg, int mode);
+
+/* Forward pass.  mel [batch][n_mel][t_mel] fp32, cond_bias as in cwg_infer (cwg_cond_bias), audio [batch][t_samples]
+ * fp32 with t_samples a positive multiple of n_group and <= t_mel * hop_length (need not be a multiple of hop_length).
+ *   z          [batch][t_samples] fp32 out (may alias audio)
+ *   log_s      NULL, or fp32 out: for k = 0 .. F-1 one [batch][n_half_k][T'] block after the other (T' = t_samples / n_group)
+ *   logp_terms [batch][3] fp64 out: sum z^2, sum_k sum log_s_k, T' * sum_k log|det W_k| per utterance
+ * Sums are reduced in a fixed order: identical calls give identical bytes.  The status word (cwg_infer_status) works as
+ * for cwg_infer, with z in place of the waveform. */
+int cwg_forward(const cwg_config* cfg, const cwg_weights* w, const float* w_fwd, const double* logdet, int mode,
+                const float* mel, const float* cond_bias, const float* audio, int t_samples,
+                float* z, float* log_s, double* logp_terms,
+                void* workspace, size_t workspace_bytes, int batch, int t_mel, void* cuda_stream);
+
 /* ax WaveGlow with waveflow=False (efficient_model_ax.py:279-357; AffineCouplingBlock.inverse
  * efficient_modules.py:94-105; glow_ax.WN.forward :375-418; InvertibleConv1x1.inverse :269-286 or
  * PermuteHeight, packed as a permutation matrix in `winv`).  Uses cwg_config / cwg_weights:
