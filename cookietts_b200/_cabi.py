@@ -46,6 +46,7 @@ EXPORTS = ("cwg_abi_version", "cwg_last_error", "cwg_workspace_bytes", "cwg_laun
            "cwg_cond_bias", "cwg_nonfinite", "cwg_infer_status", "cwg_infer", "cwg_infer_profiled", "cwg_cond", "cwg_wn_layer", "cwg_flow_boundary",
            "cwg_ax_workspace_bytes", "cwg_ax_infer", "cwg_ax_speaker_bias",
            "cwg_wf_workspace_bytes", "cwg_wf_infer", "cwg_wf_infer_profiled", "cwg_wf_launch_count", "cwg_wf_layer",
+           "cwg_wf_forward_workspace_bytes", "cwg_wf_forward_launch_count", "cwg_wf_forward", "cwg_wf_forward_layer",
            "cwg_denoise_workspace_bytes", "cwg_denoise_out_samples", "cwg_stft_mean_magnitude", "cwg_denoise", "cwg_pcm16",
            "cwg_conv1d", "cwg_conv_transpose1d", "cwg_resample1d", "cwg_deemphasis",
            "cwg_fd_workspace_bytes", "cwg_fd_launch_count", "cwg_fd_inverse",

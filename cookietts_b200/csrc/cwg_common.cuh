@@ -129,6 +129,16 @@ int launch_fwd_boundary(const cwg_config* cfg, const Dims& d, const cwg_weights*
 // terms [B][3] = {sum z^2, sum log_s, T' * sum_k log|det W_k|} from the partials (ls_part [F][B][fwd_blocks])
 int launch_fwd_reduce(const Dims& d, const double* ls_part, const double* z2_part, const double* logabsdet, double* terms,
                       cudaStream_t s);
+int launch_fwd_reduce(int F, int B, int nblk, int Tp, const double* ls_part, const double* z2_part, const double* logabsdet,
+                      double* terms, cudaStream_t s);
+// WaveFlow (cwg_wf_forward): one launch per flow boundary, k_wf_fwd_boundary in cwg_forward.cu.  phys_done: column map of
+// the flow just run (NULL: first launch, which reads audio_in and zeroes ld_zero [F]); phys_next / start_*: the flow to
+// prepare (NULL: last launch, z in logical order and z^2 partials).  Partials are [B][wf_fwd_blocks(Tp)].
+int wf_fwd_blocks(int Tp);
+int launch_wf_fwd_boundary(int B, int Tp, int G, int F, const float* audio_in, float* z, const float* eo,
+                           const int* phys_done, const int* phys_next, const float* start_w, const float* start_b,
+                           __nv_bfloat16* x0, long long xplane, double* ls_part, double* z2_part, double* ld_zero,
+                           cudaStream_t s);
 
 // ---- launchers implemented in cwg_tc.cu (tcgen05 / TMA path) ----
 int launch_cond_tc(const Dims& d, const cwg_weights* w, int npass, int flow, const float* mel,

@@ -243,6 +243,93 @@ __global__ void __launch_bounds__(TBF) k_fwd_reduce(const double* __restrict__ l
   }
 }
 
+// ------------------------------------------------------------------------------------------
+// WaveFlow's forward direction (cwg_wf_forward): one launch per flow boundary, a thread per group-step of the state
+// [B*T'][G] (z), whose columns are read and written through the host's phys[] maps: PermuteHeight moves no data.
+//   flow done: x[phys[r+1]] = x[phys[r+1]] * exp(log_s_r) + t_r, r = 0 .. G-2 (eo [G-1][B*T'][16]: log_s, t)
+//   flow next: x0[r] = start(x[phys'[r]]), r = 0 .. G-2, as bf16 hi / lo planes [G-1][B*T'][128]
+//   last     : z[c] = x[phys[c]] in logical order, and the block's sum of z^2
+// ------------------------------------------------------------------------------------------
+constexpr int WF_FWD_MAXG = 32, WF_FWD_C = 128;
+
+struct WfFwdP {
+  int Tp, G, nblk, F;
+  long long BT, xplane;
+  const float* audio_in;          // first launch: the waveform [B*T'][G]; NULL afterwards
+  float* z;                       // the state, physical columns; the last launch leaves z in logical order
+  const float* eo;                // coupling of the flow done, or NULL (first launch)
+  double* ls_part;                // [B][nblk] sums of log_s of the flow done
+  double* z2_part;                // [B][nblk] sums of z^2 (last launch), or NULL
+  double* ld_zero;                // first launch: zeroes the [F] log|det| array k_fwd_reduce adds (PermuteHeight: 0)
+  const float* start_w;           // [C] start conv of the next flow, or NULL (last launch)
+  const float* start_b;
+  __nv_bfloat16* x0;              // hi plane; the lo plane at x0 + xplane
+  int phys_done[WF_FWD_MAXG], phys_next[WF_FWD_MAXG];
+};
+
+__global__ void __launch_bounds__(TBF) k_wf_fwd_boundary(WfFwdP p) {
+  __shared__ float v_s[WF_FWD_MAXG - 1][TBF];
+  __shared__ double red[TBF / 32];
+  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, b = blockIdx.y;
+  const int t0 = blockIdx.x * TBF, t = t0 + tid;
+  const long long m0 = (long long)b * p.Tp + t0, m = m0 + tid;
+  const bool next = p.start_w != nullptr;
+  if (p.ld_zero && blockIdx.x == 0 && b == 0)
+    for (int k = tid; k < p.F; k += TBF) p.ld_zero[k] = 0.0;
+  double lsum = 0.0, z2 = 0.0;
+  if (t < p.Tp) {
+    float a[WF_FWD_MAXG];
+    const float* src = (p.audio_in ? p.audio_in : p.z) + m * p.G;
+    for (int g = 0; g < p.G; ++g) a[g] = src[g];
+    if (p.eo) {                                                    // efficient_modules.py:42-65 run forward
+      for (int r = 0; r + 1 < p.G; ++r) {
+        const float2 e = __ldcs(reinterpret_cast<const float2*>(p.eo + ((size_t)r * p.BT + m) * CWG_EO_PAD));
+        const int c = p.phys_done[r + 1];
+        a[c] = fmaf(expf(e.x), a[c], e.y);
+        lsum += (double)e.x;
+      }
+    }
+    float* dst = p.z + m * p.G;
+    if (next) {
+      for (int r = 0; r + 1 < p.G; ++r) v_s[r][tid] = a[p.phys_next[r]];
+      for (int g = 0; g < p.G; ++g) dst[g] = a[g];
+    } else {
+      for (int c = 0; c < p.G; ++c) {
+        const float v = a[p.phys_done[c]];
+        z2 = fma((double)v, (double)v, z2);
+        dst[c] = v;
+      }
+    }
+  }
+  if (p.eo) {
+    const double s = block_sum(lsum, red);
+    if (tid == 0) p.ls_part[(size_t)b * p.nblk + blockIdx.x] = s;
+  }
+  if (!next) {
+    const double s = block_sum(z2, red);
+    if (tid == 0) p.z2_part[(size_t)b * p.nblk + blockIdx.x] = s;
+    return;
+  }
+  __syncthreads();
+  // start conv (glow_ax.py:558): warp -> group-step, lane -> 4 consecutive channels
+  const int nrow = min(TBF, p.Tp - t0), c = 4 * lane;
+  const float4 w4 = __ldg(reinterpret_cast<const float4*>(p.start_w + c));
+  const float4 b4 = __ldg(reinterpret_cast<const float4*>(p.start_b + c));
+  for (int r = 0; r + 1 < p.G; ++r) {
+    for (int i = warp; i < nrow; i += TBF / 32) {
+      const float v = v_s[r][i];
+      const float x0 = fmaf(w4.x, v, b4.x), x1 = fmaf(w4.y, v, b4.y), x2 = fmaf(w4.z, v, b4.z), x3 = fmaf(w4.w, v, b4.w);
+      const __nv_bfloat162 h01 = __floats2bfloat162_rn(x0, x1), h23 = __floats2bfloat162_rn(x2, x3);
+      const __nv_bfloat162 l01 = __floats2bfloat162_rn(x0 - __low2float(h01), x1 - __high2float(h01));
+      const __nv_bfloat162 l23 = __floats2bfloat162_rn(x2 - __low2float(h23), x3 - __high2float(h23));
+      const size_t idx = ((size_t)r * p.BT + m0 + i) * WF_FWD_C + c;
+      *reinterpret_cast<uint2*>(p.x0 + idx) = make_uint2(*reinterpret_cast<const uint32_t*>(&h01), *reinterpret_cast<const uint32_t*>(&h23));
+      *reinterpret_cast<uint2*>(p.x0 + p.xplane + idx) =
+          make_uint2(*reinterpret_cast<const uint32_t*>(&l01), *reinterpret_cast<const uint32_t*>(&l23));
+    }
+  }
+}
+
 template <int XFMT, int MG>
 void launch_fb(dim3 grid, bool vec, const FwdP& p, cudaStream_t s) {
   if (vec) k_fwd_boundary<XFMT, MG, true><<<grid, TBF, 0, s>>>(p);
@@ -295,7 +382,35 @@ int launch_fwd_boundary(const cwg_config* cfg, const Dims& d, const cwg_weights*
 
 int launch_fwd_reduce(const Dims& d, const double* ls_part, const double* z2_part, const double* logabsdet, double* terms,
                       cudaStream_t s) {
-  k_fwd_reduce<<<d.B, TBF, 0, s>>>(ls_part, z2_part, logabsdet, d.F, d.B, fwd_blocks(d), d.Tp, terms);
+  return launch_fwd_reduce(d.F, d.B, fwd_blocks(d), d.Tp, ls_part, z2_part, logabsdet, terms, s);
+}
+
+int launch_fwd_reduce(int F, int B, int nblk, int Tp, const double* ls_part, const double* z2_part, const double* logabsdet,
+                      double* terms, cudaStream_t s) {
+  k_fwd_reduce<<<B, TBF, 0, s>>>(ls_part, z2_part, logabsdet, F, B, nblk, Tp, terms);
+  CWG_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
+int wf_fwd_blocks(int Tp) { return (Tp + TBF - 1) / TBF; }
+
+int launch_wf_fwd_boundary(int B, int Tp, int G, int F, const float* audio_in, float* z, const float* eo,
+                           const int* phys_done, const int* phys_next, const float* start_w, const float* start_b,
+                           __nv_bfloat16* x0, long long xplane, double* ls_part, double* z2_part, double* ld_zero,
+                           cudaStream_t s) {
+  CWG_REQUIRE(G >= 2 && G <= WF_FWD_MAXG, "forward boundary: n_group must be in [2, %d]", WF_FWD_MAXG);
+  CWG_REQUIRE((eo == nullptr) == (phys_done == nullptr) && (start_w == nullptr) == (phys_next == nullptr),
+              "forward boundary: inconsistent arguments");
+  CWG_REQUIRE(start_w || (phys_done && z2_part), "forward boundary: the last launch needs the flow done and z^2 partials");
+  WfFwdP p{};
+  p.Tp = Tp; p.G = G; p.F = F; p.BT = (long long)B * Tp; p.nblk = wf_fwd_blocks(Tp); p.xplane = xplane;
+  p.audio_in = audio_in; p.z = z; p.eo = eo; p.ls_part = ls_part; p.z2_part = z2_part; p.ld_zero = ld_zero;
+  p.start_w = start_w; p.start_b = start_b; p.x0 = x0;
+  for (int c = 0; c < G; ++c) {
+    p.phys_done[c] = phys_done ? phys_done[c] : c;
+    p.phys_next[c] = phys_next ? phys_next[c] : c;
+  }
+  k_wf_fwd_boundary<<<dim3((unsigned)p.nblk, (unsigned)B), TBF, 0, s>>>(p);
   CWG_CHECK_CUDA(cudaGetLastError());
   return 0;
 }

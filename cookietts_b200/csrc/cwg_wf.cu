@@ -130,6 +130,8 @@ struct WfLayerArgs {
   int ring_in, ring_out;  // 4th tensor-map coordinate base of the layer's input ring / next layer's ring
   int row;                // AR row index (newest row), ring slot = row % 3 (row % kh when separable)
   int rows_valid;         // min(row + 1, 3): rows of the conv queue that exist
+                          // full-height form (FULL): row = blockIdx.z, set in the kernel with rows_valid and eo's row; x rows
+                          // are absolute (ring_in + row), eo is [G-1][B*T'][16]
   int has_res, first;
   // separable in_layers only (k_wf_sep_tc)
   const __nv_bfloat16* x; // ring hi plane; the lo plane follows at x + xplane
@@ -151,7 +153,7 @@ constexpr int W_OFF_BAR = W_OFF_B2 + 512;
 constexpr int W_SMEM = W_OFF_BAR + 256 + 1024;
 constexpr int W_THREADS = 384, W_EPI_THREADS = 256;
 
-template <int NPASS>
+template <int NPASS, bool FULL = false>
 __global__ void __launch_bounds__(W_THREADS, 2)
 k_wf_layer_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ CUtensorMap tm_x_lo,
               const __grid_constant__ CUtensorMap tm_m_hi, const __grid_constant__ CUtensorMap tm_m_lo,
@@ -170,6 +172,11 @@ k_wf_layer_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant
   uint64_t* xold_full = acc2_full + 1;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(xold_full + 1);
 
+  if constexpr (FULL) {                              // full-height form: one CTA row per height row
+    a.row = blockIdx.z;
+    a.rows_valid = min(a.row + 1, WF_KH);
+    a.eo += (size_t)a.row * a.BT * CWG_EO_PAD;
+  }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int t0 = blockIdx.x * 128, b = blockIdx.y;
   auto slot = [&](int i) { return smem + i * TILE_A; };
@@ -210,7 +217,7 @@ k_wf_layer_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant
           asm volatile(
               "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
               ::"r"(smem_u32(slot(s))), "l"(reinterpret_cast<uint64_t>(pl ? &tm_x_lo : &tm_x_hi)), "r"(smem_u32(&full[s])),
-                "r"(cb * 64), "r"(t0 + (kw - 1) * a.dil), "r"(b), "r"(a.ring_in + r % 3)
+                "r"(cb * 64), "r"(t0 + (kw - 1) * a.dil), "r"(b), "r"(a.ring_in + (FULL ? r : r % 3))
               : "memory");
         } else {
           tma_load_3d(slot(s), pl ? &tm_m_lo : &tm_m_hi, &full[s], (kb - nkb_x) * 64, t0, b);
@@ -296,7 +303,7 @@ k_wf_layer_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant
           asm volatile(
               "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
               ::"r"(smem_u32(slot(2 * pl + kb))), "l"(reinterpret_cast<uint64_t>(pl ? &tm_x_lo : &tm_x_hi)), "r"(smem_u32(xold_full)),
-                "r"(kb * 64), "r"(t0), "r"(b), "r"(a.ring_in + a.row % 3)
+                "r"(kb * 64), "r"(t0), "r"(b), "r"(a.ring_in + (FULL ? a.row : a.row % 3))
               : "memory");
     }
   } else if (warp >= 4) {
@@ -398,7 +405,7 @@ k_wf_layer_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant
         for (int pl = 0; pl < 2; ++pl)
           asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
                        ::"l"(reinterpret_cast<uint64_t>(pl ? &tm_x_lo : &tm_x_hi)), "r"(smem_u32(slot(2 * pl + half))),
-                         "r"(half * 64), "r"(t0), "r"(b), "r"(a.ring_out + a.row % 3)
+                         "r"(half * 64), "r"(t0), "r"(b), "r"(a.ring_out + (FULL ? a.row : a.row % 3))
                        : "memory");
         tma_store_commit();
         tma_store_wait_read();
@@ -426,7 +433,7 @@ constexpr int S_SMEM = S_OFF_BAR + 256 + 1024;                             // 19
 // causal in height (rows that do not exist yet are the zero queue), zero-padded in width per utterance.  A lane owns 4
 // channels and a warp one step at a time, so each load is a 256-byte run of channels.  d is written as 128B-swizzled
 // bf16 hi (and lo) tiles, one per 64-channel k-block; it never goes to HBM.
-template <int NPASS>
+template <int NPASS, bool FULL>
 __device__ __forceinline__ void wf_depthwise_tile(const WfLayerArgs& a, const float* dws, const float* dwb, int b, int t0,
                                                   int ew, int lane, uint8_t* d_hi, uint8_t* d_lo) {
   // A warp handles 16 steps in two passes of S.  The loop is not bound by load latency (issuing two taps' loads at once
@@ -445,7 +452,7 @@ __device__ __forceinline__ void wf_depthwise_tile(const WfLayerArgs& a, const fl
     for (int ah = 0; ah < a.kh; ++ah) {
       const int r = a.row - (a.kh - 1 - ah);
       if (r < 0) continue;
-      const __nv_bfloat16* xh = a.x + ((size_t)(a.ring_in + r % a.kh) * a.BT + (size_t)b * a.Tp) * WF_C + c;
+      const __nv_bfloat16* xh = a.x + ((size_t)(a.ring_in + (FULL ? r : r % a.kh)) * a.BT + (size_t)b * a.Tp) * WF_C + c;
       const __nv_bfloat16* xl = xh + a.xplane;
       for (int bw = 0; bw < a.kw; ++bw) {
         const float4 w = *reinterpret_cast<const float4*>(dws + (ah * a.kw + bw) * WF_C + c);
@@ -494,7 +501,7 @@ __device__ __forceinline__ void wf_depthwise_tile(const WfLayerArgs& a, const fl
 // The layer step with separable in_layers, one CTA per SM: GEMM1 runs over the 2 mel k-blocks (TMA, issued first), then
 // the 2 k-blocks of d, which the epilogue warps compute in the meantime (wf_depthwise_tile).  Gate, GEMM2 ([res | folded
 // end], N = 144), residual update and eo accumulation are those of k_wf_layer_tc, whose source is kept as it is.
-template <int NPASS>
+template <int NPASS, bool FULL = false>
 __global__ void __launch_bounds__(W_THREADS, 1)
 k_wf_sep_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ CUtensorMap tm_x_lo,
             const __grid_constant__ CUtensorMap tm_m_hi, const __grid_constant__ CUtensorMap tm_m_lo,
@@ -514,6 +521,10 @@ k_wf_sep_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__
   uint64_t* d_ready = xold_full + 1;                 // depthwise tiles written
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(d_ready + 1);
 
+  if constexpr (FULL) {                              // full-height form: one CTA row per height row
+    a.row = blockIdx.z;
+    a.eo += (size_t)a.row * a.BT * CWG_EO_PAD;
+  }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int t0 = blockIdx.x * 128, b = blockIdx.y;
   auto slot = [&](int i) { return smem + i * TILE_A; };
@@ -646,7 +657,7 @@ k_wf_sep_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__
           asm volatile(
               "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2];"
               ::"r"(smem_u32(slot(2 * pl + kb))), "l"(reinterpret_cast<uint64_t>(pl ? &tm_x_lo : &tm_x_hi)), "r"(smem_u32(xold_full)),
-                "r"(kb * 64), "r"(t0), "r"(b), "r"(a.ring_in + a.row % nslot)
+                "r"(kb * 64), "r"(t0), "r"(b), "r"(a.ring_in + (FULL ? a.row : a.row % nslot))
               : "memory");
     }
   } else if (warp >= 4) {
@@ -658,7 +669,7 @@ k_wf_sep_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__
     const float4* b1g = reinterpret_cast<const float4*>(b1s + WF_C);
 
     // the mel k-blocks of GEMM1 run meanwhile
-    wf_depthwise_tile<NPASS>(a, reinterpret_cast<const float*>(smem + S_OFF_DW), reinterpret_cast<const float*>(smem + S_OFF_DWB),
+    wf_depthwise_tile<NPASS, FULL>(a, reinterpret_cast<const float*>(smem + S_OFF_DW), reinterpret_cast<const float*>(smem + S_OFF_DWB),
                              b, t0, warp - 4, lane, slot(W_NS), slot(W_NS + NKB_D));
     tc_fence_before_sync();
     fence_proxy_async_smem();
@@ -754,7 +765,7 @@ k_wf_sep_tc(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__
         for (int pl = 0; pl < 2; ++pl)
           asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];"
                        ::"l"(reinterpret_cast<uint64_t>(pl ? &tm_x_lo : &tm_x_hi)), "r"(smem_u32(slot(2 * pl + half))),
-                         "r"(half * 64), "r"(t0), "r"(b), "r"(a.ring_out + a.row % nslot)
+                         "r"(half * 64), "r"(t0), "r"(b), "r"(a.ring_out + (FULL ? a.row : a.row % nslot))
                        : "memory");
         tma_store_commit();
         tma_store_wait_read();
@@ -781,6 +792,30 @@ void wf_carve(const WfDims& d, void* base, WfWorkspace* ws) {
   ws->state = (float*)take((size_t)d.BT * d.G * 4);
   ws->mel_up = (__nv_bfloat16*)take((size_t)d.BT * WF_HP * 2 * 2);
   ws->x = (__nv_bfloat16*)take((size_t)d.L * d.KH * d.BT * WF_C * 2 * 2);
+  ws->bytes = off;
+}
+
+// Forward direction (cwg_wf_forward): all G-1 height rows of a flow are known before it runs.
+struct WfFwdWorkspace {
+  __nv_bfloat16* x;      // hi plane then lo plane, each two full-height buffers [2][G-1][B][T'][C] (layers ping-pong)
+  __nv_bfloat16* mel_up; // hi, lo planes [B][T'][128]
+  float* eo;             // [G-1][B*T'][16]
+  double* ls_part;       // [F][B][nblk] block sums of log_s
+  double* z2_part;       // [B][nblk] block sums of z^2
+  double* ld_zero;       // [F] zeros: the log|det| of PermuteHeight that k_fwd_reduce adds
+  size_t bytes;
+};
+
+void wf_fwd_carve(const WfDims& d, void* base, WfFwdWorkspace* ws) {
+  size_t off = 0;
+  auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 1024); return (char*)base + o; };
+  const size_t nblk = (size_t)wf_fwd_blocks(d.Tp);
+  ws->eo = (float*)take((size_t)(d.G - 1) * d.BT * CWG_EO_PAD * 4);
+  ws->ls_part = (double*)take((size_t)d.F * d.B * nblk * 8);
+  ws->z2_part = (double*)take((size_t)d.B * nblk * 8);
+  ws->ld_zero = (double*)take((size_t)d.F * 8);
+  ws->mel_up = (__nv_bfloat16*)take((size_t)d.BT * WF_HP * 2 * 2);
+  ws->x = (__nv_bfloat16*)take((size_t)2 * (d.G - 1) * d.BT * WF_C * 2 * 2);
   ws->bytes = off;
 }
 
@@ -835,14 +870,26 @@ int wf_check_weights(const cwg_wf_config* c, const cwg_wf_weights* w) {
   return 0;
 }
 
+template <bool FULL>
+void wf_go(bool sep, int npass, dim3 grid, const CUtensorMap* m, const WfLayerArgs& a, cudaStream_t s) {
+  if (sep && npass == 3) k_wf_sep_tc<3, FULL><<<grid, W_THREADS, S_SMEM, s>>>(m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7], a);
+  else if (sep) k_wf_sep_tc<1, FULL><<<grid, W_THREADS, S_SMEM, s>>>(m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7], a);
+  else if (npass == 3) k_wf_layer_tc<3, FULL><<<grid, W_THREADS, W_SMEM, s>>>(m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7], a);
+  else k_wf_layer_tc<1, FULL><<<grid, W_THREADS, W_SMEM, s>>>(m[0], m[1], m[2], m[3], m[4], m[5], m[6], m[7], a);
+}
+
+// One WN_2d layer.  row >= 0: the step of AR row `row`, x = the conv-queue rings [L][KH][B][T'][C] (hi plane, then lo).
+// row < 0 (forward direction): all G-1 height rows in one launch, x = two full-height buffers [2][G-1][B][T'][C] per plane;
+// layer l reads buffer l % 2 and writes buffer (l + 1) % 2, eo is [G-1][B*T'][16].
 int wf_launch_layer(const cwg_wf_config* cfg, const WfDims& d, const cwg_wf_weights* w, int npass, int flow, int layer,
                     int row, __nv_bfloat16* x, const __nv_bfloat16* mel_up, float* eo, cudaStream_t s) {
-  const bool sep = w->dw_w != nullptr;
-  const size_t xplane = (size_t)d.L * d.KH * d.BT * WF_C, mplane = (size_t)d.BT * WF_HP;
+  const bool sep = w->dw_w != nullptr, full = row < 0;
+  const uint64_t xrows = full ? 2ull * (d.G - 1) : (uint64_t)d.L * d.KH;
+  const size_t xplane = (size_t)xrows * d.BT * WF_C, mplane = (size_t)d.BT * WF_HP;
   const uint64_t fl = (uint64_t)d.F * d.L;
   CUtensorMap tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo;
   {
-    uint64_t dims[4] = {WF_C, (uint64_t)d.Tp, (uint64_t)d.B, (uint64_t)d.L * d.KH};
+    uint64_t dims[4] = {WF_C, (uint64_t)d.Tp, (uint64_t)d.B, xrows};
     uint64_t st[3] = {WF_C * 2, (uint64_t)d.Tp * WF_C * 2, (uint64_t)d.BT * WF_C * 2};
     uint32_t box[4] = {64, 128, 1, 1};
     if (int r = make_map(&tx_hi, x, 4, dims, st, box)) return r;
@@ -860,28 +907,31 @@ int wf_launch_layer(const cwg_wf_config* cfg, const WfDims& d, const cwg_wf_weig
   a.b1 = w->b1 + idx * 2 * WF_C; a.b2 = w->b2 + idx * WF_C; a.eo_b = w->eo_b + (size_t)flow * CWG_EO_PAD;
   a.eo = eo; a.Tp = d.Tp; a.dil = 1 << layer;
   a.w1_row0 = (int)(idx * 2 * WF_C); a.w2_row0 = (int)(idx * WF_N2);
-  a.ring_in = layer * d.KH; a.ring_out = (layer + 1) * d.KH;
-  a.row = row; a.rows_valid = row + 1 < WF_KH ? row + 1 : WF_KH;
+  if (full) {
+    a.ring_in = (layer & 1) * (d.G - 1); a.ring_out = ((layer + 1) & 1) * (d.G - 1);
+  } else {
+    a.ring_in = layer * d.KH; a.ring_out = (layer + 1) * d.KH;
+    a.row = row; a.rows_valid = row + 1 < WF_KH ? row + 1 : WF_KH;
+  }
   a.has_res = layer < d.L - 1; a.first = layer == 0;
-  dim3 grid((unsigned)((d.Tp + 127) / 128), d.B);
+  a.x = x; a.xplane = (long long)xplane; a.BT = d.BT;
+  dim3 grid((unsigned)((d.Tp + 127) / 128), d.B, full ? d.G - 1 : 1);
   if (sep) {
-    a.x = x; a.xplane = (long long)xplane; a.BT = d.BT;
     a.kh = cfg->kernel_h; a.kw = cfg->kernel_w;
     a.dw_w = w->dw_w + idx * WF_C * a.kh * a.kw; a.dw_b = w->dw_b + idx * WF_C;
-    if (npass == 3) {
-      if (int r = set_smem(k_wf_sep_tc<3>, S_SMEM)) return r;
-      k_wf_sep_tc<3><<<grid, W_THREADS, S_SMEM, s>>>(tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo, a);
-    } else {
-      if (int r = set_smem(k_wf_sep_tc<1>, S_SMEM)) return r;
-      k_wf_sep_tc<1><<<grid, W_THREADS, S_SMEM, s>>>(tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo, a);
-    }
-  } else if (npass == 3) {
-    if (int r = set_smem(k_wf_layer_tc<3>, W_SMEM)) return r;
-    k_wf_layer_tc<3><<<grid, W_THREADS, W_SMEM, s>>>(tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo, a);
-  } else {
-    if (int r = set_smem(k_wf_layer_tc<1>, W_SMEM)) return r;
-    k_wf_layer_tc<1><<<grid, W_THREADS, W_SMEM, s>>>(tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo, a);
   }
+  if (full) {
+    if (int r = sep ? (npass == 3 ? set_smem(k_wf_sep_tc<3, true>, S_SMEM) : set_smem(k_wf_sep_tc<1, true>, S_SMEM))
+                    : (npass == 3 ? set_smem(k_wf_layer_tc<3, true>, W_SMEM) : set_smem(k_wf_layer_tc<1, true>, W_SMEM)))
+      return r;
+  } else {
+    if (int r = sep ? (npass == 3 ? set_smem(k_wf_sep_tc<3>, S_SMEM) : set_smem(k_wf_sep_tc<1>, S_SMEM))
+                    : (npass == 3 ? set_smem(k_wf_layer_tc<3>, W_SMEM) : set_smem(k_wf_layer_tc<1>, W_SMEM)))
+      return r;
+  }
+  const CUtensorMap maps[8] = {tx_hi, tx_lo, tm_hi, tm_lo, tw1_hi, tw1_lo, tw2_hi, tw2_lo};
+  if (full) wf_go<true>(sep, npass, grid, maps, a, s);
+  else wf_go<false>(sep, npass, grid, maps, a, s);
   CWG_CHECK_CUDA(cudaGetLastError());
   return 0;
 }
@@ -997,6 +1047,88 @@ int cwg_wf_infer_profiled(const cwg_wf_config* cfg, const cwg_wf_weights* w, int
     for (int c = 0; c < h; ++c) phys[c] = nxt[c];
   }
   return 0;
+}
+
+static int wf_fwd_check(const cwg_wf_config* cfg, int mode, int batch, int t_samples) {
+  CWG_REQUIRE(cfg != nullptr, "cfg is NULL");
+  CWG_REQUIRE(mode != CWG_MODE_FFMA, "the WaveFlow forward direction runs in CWG_MODE_BF16X3 / CWG_MODE_BF16 only, not CWG_MODE_FFMA");
+  return wf_check(cfg, mode, batch, t_samples);
+}
+
+size_t cwg_wf_forward_workspace_bytes(const cwg_wf_config* cfg, int mode, int batch, int frames, int t_samples) {
+  if (wf_fwd_check(cfg, mode, batch, t_samples)) return 0;
+  if (frames < 1) { set_error("frames must be >= 1"); return 0; }
+  WfDims d = wf_dims(cfg, batch, t_samples);
+  WfFwdWorkspace ws;
+  wf_fwd_carve(d, nullptr, &ws);
+  return ws.bytes + 1024;
+}
+
+int cwg_wf_forward_launch_count(const cwg_wf_config* cfg) {
+  if (!cfg) return -1;
+  return cfg->n_flows * (cfg->n_layers + 1) + 3;      // mel, F + 1 boundaries, F * L full-height layers, reduction
+}
+
+int cwg_wf_forward_layer(const cwg_wf_config* cfg, const cwg_wf_weights* w, int mode, int flow, int layer, void* x_bufs,
+                         const void* mel_up, float* eo, int batch, int t_samples, void* cuda_stream) {
+  if (int r = wf_fwd_check(cfg, mode, batch, t_samples)) return r;
+  CWG_REQUIRE(w && w->w1_hi && w->w1_lo && w->w2_hi && w->w2_lo && w->b1 && w->b2 && w->eo_b, "missing weight arrays (NULL)");
+  if (int r = wf_check_weights(cfg, w)) return r;
+  CWG_REQUIRE(x_bufs && mel_up && eo, "NULL tensor argument");
+  CWG_REQUIRE(flow >= 0 && flow < cfg->n_flows && layer >= 0 && layer < cfg->n_layers, "flow/layer out of range");
+  WfDims d = wf_dims(cfg, batch, t_samples);
+  return wf_launch_layer(cfg, d, w, mode == CWG_MODE_BF16X3 ? 3 : 1, flow, layer, -1, (__nv_bfloat16*)x_bufs,
+                         (const __nv_bfloat16*)mel_up, eo, (cudaStream_t)cuda_stream);
+}
+
+int cwg_wf_forward(const cwg_wf_config* cfg, const cwg_wf_weights* w, int mode, const float* mel, int frames,
+                   const float* audio, int t_samples, float* z, double* logp_terms, void* workspace, size_t workspace_bytes,
+                   int batch, void* cuda_stream) {
+  if (int r = wf_fwd_check(cfg, mode, batch, t_samples)) return r;
+  CWG_REQUIRE(w && w->w1_hi && w->w1_lo && w->w2_hi && w->w2_lo && w->b1 && w->b2 && w->eo_b && w->start_w && w->start_b,
+              "missing weight arrays (NULL)");
+  if (int r = wf_check_weights(cfg, w)) return r;
+  CWG_REQUIRE(mel && audio && z && logp_terms, "NULL tensor argument");
+  CWG_REQUIRE(frames >= 1, "frames must be >= 1");
+  CWG_REQUIRE(workspace != nullptr && ((uintptr_t)workspace % 1024) == 0, "workspace must be 1024-byte aligned (NULL)");
+  WfDims d = wf_dims(cfg, batch, t_samples);
+  WfFwdWorkspace ws;
+  wf_fwd_carve(d, workspace, &ws);
+  CWG_REQUIRE(ws.bytes <= workspace_bytes, "workspace too small: need %zu, got %zu", ws.bytes, workspace_bytes);
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  const int npass = mode == CWG_MODE_BF16X3 ? 3 : 1;
+  const int h = d.G, F = d.F, L = d.L, nblk = wf_fwd_blocks(d.Tp);
+  const long long xplane = 2ll * (h - 1) * d.BT * WF_C;
+  {
+    const long long n = d.BT * WF_HP, mplane = n;
+    k_wf_mel_up<<<(unsigned)((n + 255) / 256), 256, 0, s>>>(mel, ws.mel_up, ws.mel_up + mplane, d.B, d.M, frames, frames,
+                                                           d.Tp, cfg->upsample_linear);
+    CWG_CHECK_CUDA(cudaGetLastError());
+  }
+  // phys[c]: physical column of logical height row c in z; x = permute_height(x, k) before flow k's coupling
+  int phys[WF_TC_MAX_GROUP], perm[WF_TC_MAX_GROUP], nxt[WF_TC_MAX_GROUP];
+  for (int c = 0; c < h; ++c) phys[c] = c;
+  auto permute = [&](int k) {
+    wf_perm(k, h, perm);
+    for (int c = 0; c < h; ++c) nxt[c] = phys[perm[c]];
+    for (int c = 0; c < h; ++c) phys[c] = nxt[c];
+  };
+  permute(0);
+  if (int r = launch_wf_fwd_boundary(d.B, d.Tp, h, F, audio, z, nullptr, nullptr, phys, w->start_w, w->start_b, ws.x, xplane,
+                                     nullptr, nullptr, ws.ld_zero, s)) return r;
+  for (int k = 0; k < F; ++k) {
+    for (int l = 0; l < L; ++l)
+      if (int r = wf_launch_layer(cfg, d, w, npass, k, l, -1, ws.x, ws.mel_up, ws.eo, s)) return r;
+    int done[WF_TC_MAX_GROUP];
+    for (int c = 0; c < h; ++c) done[c] = phys[c];
+    const bool last = k + 1 == F;
+    if (!last) permute(k + 1);
+    if (int r = launch_wf_fwd_boundary(d.B, d.Tp, h, F, nullptr, z, ws.eo, done, last ? nullptr : phys,
+                                       last ? nullptr : w->start_w + (size_t)(k + 1) * WF_C,
+                                       last ? nullptr : w->start_b + (size_t)(k + 1) * WF_C, ws.x, xplane,
+                                       ws.ls_part + (size_t)k * d.B * nblk, last ? ws.z2_part : nullptr, nullptr, s)) return r;
+  }
+  return launch_fwd_reduce(F, d.B, nblk, d.Tp, ws.ls_part, ws.z2_part, ws.ld_zero, logp_terms, s);
 }
 
 }  // extern "C"

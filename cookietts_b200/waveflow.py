@@ -1,6 +1,6 @@
 """Drop-in for the reference's "ax" model `CookieTTS/_4_mtw/waveglow/efficient_model_ax.py::WaveGlow`
 in its WaveFlow configuration (`waveflow=True`, `WN_2d`, `PermuteHeight`; BASELINE config 5),
-inverse pass only, on sm_100a tensor-core kernels (csrc/cwg_wf.cu): the dense 3x3 WN_2d of config 5, and the
+inverse pass, plus the no-grad forward direction (`encode`, `log_prob`) in the tensor-core modes, on sm_100a tensor-core kernels (csrc/cwg_wf.cu): the dense 3x3 WN_2d of config 5, and the
 depthwise-separable in_layers (kernel_h <= 7 x odd kernel_w <= 7) of the reference author's trained checkpoints.
 
 Interface mirrored: the ax constructor keywords (efficient_model_ax.py:19-20), the state_dict layout
@@ -185,6 +185,16 @@ def _bind(lib):
     lib.cwg_wf_layer.restype = C.c_int
     lib.cwg_wf_layer.argtypes = [C.POINTER(CwgWfConfig), C.POINTER(CwgWfWeights), C.c_int, C.c_int, C.c_int, C.c_int,
                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
+    lib.cwg_wf_forward_workspace_bytes.restype = C.c_size_t
+    lib.cwg_wf_forward_workspace_bytes.argtypes = [C.POINTER(CwgWfConfig), C.c_int, C.c_int, C.c_int, C.c_int]
+    lib.cwg_wf_forward_launch_count.restype = C.c_int
+    lib.cwg_wf_forward_launch_count.argtypes = [C.POINTER(CwgWfConfig)]
+    lib.cwg_wf_forward.restype = C.c_int
+    lib.cwg_wf_forward.argtypes = [C.POINTER(CwgWfConfig), C.POINTER(CwgWfWeights), C.c_int, C.c_void_p, C.c_int,
+                                   C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_void_p]
+    lib.cwg_wf_forward_layer.restype = C.c_int
+    lib.cwg_wf_forward_layer.argtypes = [C.POINTER(CwgWfConfig), C.POINTER(CwgWfWeights), C.c_int, C.c_int, C.c_int,
+                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]
     lib._wf_bound = True
 
 
@@ -237,7 +247,8 @@ class _Coupling(nn.Module):
 
 
 class WaveFlow(nn.Module, AxFrontEndMixin):
-    """`efficient_model_ax.WaveGlow(..., waveflow=True)` - inverse pass on B200."""
+    """`efficient_model_ax.WaveGlow(..., waveflow=True)` - inverse pass on B200, plus the no-grad forward direction
+    (`encode`, `log_prob`) in the tensor-core modes."""
     GRAPH_MAX_FRAMES = 4096
 
     def __init__(self, n_mel_channels, n_flows, n_group, n_early_every, n_early_size, memory_efficient,
@@ -600,6 +611,79 @@ class WaveFlow(nn.Module, AxFrontEndMixin):
         if artifact_trimming > 0:
             audio = audio[:, :-artifact_trimming * self.hop_length]
         return audio.to(in_dtype)
+
+    def _forward_terms(self, spect, audio, speaker_ids):
+        """audio -> (z [B, T], logp_terms [B, 3] fp64 {sum z^2, sum log_s, 0}) on the device (csrc/cwg_wf.cu,
+        cwg_wf_forward)."""
+        if self.precision == "ffma":
+            raise NotImplementedError("cookietts_b200.WaveFlow: the forward direction (encode / log_prob) runs in the tensor-core "
+                                      "modes 'bf16x3' and 'bf16' only; this model runs in 'ffma' (its precision or a WN_config "
+                                      "variant)")
+        if self.vol_scaling or self.preempthasis:
+            raise NotImplementedError("cookietts_b200.WaveFlow: the forward direction is not built for preceived_vol_scaling / "
+                                      "preempthasis models (their post-filter's forward map and Jacobian are not pinned)")
+        if spect.dim() == 2:
+            spect = spect[None]
+        if audio.dim() == 1:
+            audio = audio[None]
+        B, T = audio.shape
+        if T < self.n_group or T % self.n_group:
+            raise ValueError(f"audio length {T} must be a positive multiple of n_group = {self.n_group}")
+        if spect.shape[0] != B:
+            raise ValueError(f"batch mismatch: spect has {spect.shape[0]} utterances, audio {B}")
+        dev = self._device()
+        if dev.type != "cuda":
+            raise RuntimeError("cookietts_b200.WaveFlow needs the module on a CUDA device (no CPU fallback)")
+        lib = _cabi.load()
+        _bind(lib)
+        mode = _cabi.MODES[self.precision]
+        cond = spect.to(device=dev, dtype=torch.float32)
+        if self.shift_spect != 0.:
+            cond = cond + self.shift_spect
+        if self.scale_spect != 1.:
+            cond = cond * self.scale_spect
+        audio = audio.to(device=dev, dtype=torch.float32).contiguous()
+        with torch.cuda.device(dev):
+            self._ensure_packed()
+            cond = self._fe_apply(cond.contiguous(), speaker_ids, T // self.n_group).contiguous()   # as `inverse` does
+            frames = cond.shape[2]
+            nbytes = lib.cwg_wf_forward_workspace_bytes(self._ccfg, mode, B, frames, T)
+            if nbytes == 0:
+                raise _cabi.CwgError(lib.cwg_last_error().decode())
+            free, _ = torch.cuda.mem_get_info(dev)
+            if nbytes > free:
+                raise RuntimeError(f"WaveFlow forward: the workspace for batch {B} x {T} samples needs {nbytes / 2**30:.1f} GiB, "
+                                   f"{free / 2**30:.1f} GiB are free on the device; split the batch")
+            ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
+            ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
+            z = torch.empty(B, T, device=dev, dtype=torch.float32)
+            terms = torch.empty(B, 3, device=dev, dtype=torch.float64)
+            _cabi.check(lib.cwg_wf_forward(self._ccfg, self._cw, mode, cond.data_ptr(), frames, audio.data_ptr(), T,
+                                           z.data_ptr(), terms.data_ptr(), ws_ptr, ws.numel() - (ws_ptr - ws.data_ptr()), B,
+                                           torch.cuda.current_stream(dev).cuda_stream))
+        return z, terms
+
+    @torch.no_grad()
+    def encode(self, spect, audio, speaker_ids=None):
+        """audio [B, T] -> z [B, T] in the layout `inverse(z, spect)` takes (z[b, s*n_group + c]), so
+        `inverse(encode(spect, x), spect)` reproduces x.  The cond is the one `inverse` builds from `spect`."""
+        return self._forward_terms(spect, audio, speaker_ids)[0]
+
+    @torch.no_grad()
+    def log_prob(self, spect, audio, sigma=1.0, speaker_ids=None):
+        """Per-utterance log-density of `audio` in nats, float64 [B]:
+        sum(-z^2 / (2 sigma^2)) - (T/2) log(2 pi sigma^2) + sum_k sum log_s_k (PermuteHeight has |det| = 1)."""
+        _, terms = self._forward_terms(spect, audio, speaker_ids)
+        T = audio.shape[-1]
+        s2 = float(sigma) ** 2
+        return -terms[:, 0] / (2 * s2) - 0.5 * T * float(np.log(2 * np.pi * s2)) + terms[:, 1]
+
+    def forward_launch_count(self) -> int:
+        """Kernels one `encode` / `log_prob` call launches: n_flows * (n_layers + 1) + 3."""
+        lib = _cabi.load()
+        _bind(lib)
+        self._ensure_packed()
+        return int(lib.cwg_wf_forward_launch_count(self._ccfg))
 
     def launch_count(self) -> int:
         lib = _cabi.load()

@@ -365,6 +365,28 @@ int cwg_wf_launch_count(const cwg_wf_config* cfg);
 int cwg_wf_layer(const cwg_wf_config* cfg, const cwg_wf_weights* w, int mode, int flow, int layer, int row,
                  void* x_rings, const void* mel_up, float* eo, int batch, int t_samples, void* cuda_stream);
 
+/* Forward direction (audio -> z) of the tensor-core subset above, CWG_MODE_BF16X3 / CWG_MODE_BF16 (CWG_MODE_FFMA and the
+ * WN_config variants are errors).  With x = audio.view(B, T', h).transpose(1, 2) and the cond of cwg_wf_infer, flows
+ * k = 0 .. F-1 do x = permute_height(x, k), then (log_s_r, t_r) = WN_2d(rows 0 .. h-2 of x, causal in height) and
+ * x[r+1] = x[r+1] * exp(log_s_r) + t_r; z = x in the [batch][t_samples] layout cwg_wf_infer takes (z[b, s*h + c]).
+ * Every height row is known before a flow runs, so each WN_2d layer is one launch over all h-1 rows.
+ *   mel        [batch][n_mel][frames] fp32, interpolated to T' = t_samples / n_group steps (no pad frames)
+ *   audio      [batch][t_samples] fp32; z [batch][t_samples] fp32 out
+ *   logp_terms [batch][3] fp64 out: sum z^2, sum_k sum log_s_k, 0 (PermuteHeight has |det| = 1) per utterance
+ * Sums are reduced in a fixed order: identical calls give identical bytes, and row b of a batch equals the
+ * single-utterance call. */
+size_t cwg_wf_forward_workspace_bytes(const cwg_wf_config* cfg, int mode, int batch, int frames, int t_samples);
+int cwg_wf_forward_launch_count(const cwg_wf_config* cfg);     /* n_flows * (n_layers + 1) + 3 */
+int cwg_wf_forward(const cwg_wf_config* cfg, const cwg_wf_weights* w, int mode, const float* mel, int frames,
+                   const float* audio, int t_samples, float* z, double* logp_terms, void* workspace, size_t workspace_bytes,
+                   int batch, void* cuda_stream);
+
+/* Stage entry point (tests): one full-height WN_2d layer of the forward direction.  x_bufs: bf16 planes (hi then lo), each
+ * two buffers [2][n_group-1][batch][T'][C]; reads buffer layer % 2 at rows r-kernel_h+1 .. r (those >= 0) for every row
+ * r = 0 .. n_group-2 and writes buffer (layer+1) % 2 (not for the last layer); eo [n_group-1][batch*T'][CWG_EO_PAD]. */
+int cwg_wf_forward_layer(const cwg_wf_config* cfg, const cwg_wf_weights* w, int mode, int flow, int layer, void* x_bufs,
+                         const void* mel_up, float* eo, int batch, int t_samples, void* cuda_stream);
+
 /* =====================================================================================
  * Denoiser post-filter (SURVEY 8f-1): CookieTTS/_4_mtw/waveglow/denoiser.py:59-71 on the conv-based STFT of
  * CookieTTS/utils/audio/stft.py:79-146 (reflect pad, windowed Fourier bases, window-sum-square synthesis).
