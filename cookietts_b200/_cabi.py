@@ -51,7 +51,8 @@ EXPORTS = ("cwg_abi_version", "cwg_last_error", "cwg_workspace_bytes", "cwg_laun
            "cwg_conv1d", "cwg_conv_transpose1d", "cwg_resample1d", "cwg_deemphasis",
            "cwg_fd_workspace_bytes", "cwg_fd_launch_count", "cwg_fd_inverse",
            "cwg_axg_workspace_bytes", "cwg_axg_launch_count", "cwg_axg_flow", "cwg_group_transpose",
-           "cwg_pack_forward", "cwg_forward_workspace_bytes", "cwg_forward_launch_count", "cwg_forward")
+           "cwg_pack_forward", "cwg_forward_workspace_bytes", "cwg_forward_launch_count", "cwg_forward",
+           "cwg_ax_forward_workspace_bytes", "cwg_ax_forward_launch_count", "cwg_ax_forward")
 
 
 class CwgError(RuntimeError):

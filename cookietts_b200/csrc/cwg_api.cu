@@ -558,6 +558,97 @@ int cwg_ax_infer(const cwg_config* cfg, const cwg_weights* w, int mode,
   return 0;
 }
 
+// Forward direction of the ax model (audio -> z): flows k = 0 .. F-1, each on the trailing n_rem_k columns (early
+// outputs stay where they are).  mix_first: W_k, WN_k + coupling;  else: WN_k + coupling, W_k.  In flow k the WN sees
+// audio_0 and the cond of the inverse, so the layer launches are cwg_ax_infer's; only the boundaries differ.
+namespace {
+struct AxFwdLayout {
+  Dims d;
+  size_t ls_part, z2_part, bytes;
+};
+
+AxFwdLayout ax_fwd_layout(const cwg_config* cfg, int mode, int batch, int frames, int t_samples) {
+  AxFwdLayout l;
+  l.d = ax_dims(cfg, batch, frames, t_samples);
+  Workspace ws;
+  carve(l.d, mode, nullptr, &ws);
+  size_t off = ws.bytes;
+  auto take = [&](size_t bytes) { size_t o = off; off = align_up(off + bytes, 1024); return o; };
+  const size_t nblk = (size_t)fwd_blocks(l.d);
+  l.ls_part = take((size_t)l.d.F * batch * nblk * sizeof(double));
+  l.z2_part = take((size_t)batch * nblk * sizeof(double));
+  l.bytes = off;
+  return l;
+}
+}  // namespace
+
+size_t cwg_ax_forward_workspace_bytes(const cwg_config* cfg, int mode, int batch, int frames, int t_samples) {
+  if (ax_check(cfg, mode, batch, frames, t_samples)) return 0;
+  return ax_fwd_layout(cfg, mode, batch, frames, t_samples).bytes + 1024;
+}
+
+int cwg_ax_forward_launch_count(const cwg_config* cfg, int mode) {
+  if (check_config(cfg) || check_mode(cfg, mode, false)) return -1;
+  const int per_layer = mode == CWG_MODE_FFMA ? 3 : (cfg->n_channels == 512 ? 2 : 1);
+  // cond interpolation, first boundary, per flow L layers and a boundary, the reduction (+ the non-finite scan of z)
+  return 3 + (mode == CWG_MODE_F16F8 ? 1 : 0) + cfg->n_flows * (per_layer * cfg->n_layers + 1);
+}
+
+int cwg_ax_forward(const cwg_config* cfg, const cwg_weights* w, const float* w_fwd, const double* logabsdet, int mode,
+                   const float* mel, int frames, int upsample_linear, int mix_first, const float* audio, int t_samples,
+                   float* z, double* logp_terms, void* workspace, size_t workspace_bytes, int batch,
+                   const float* b1_batch, void* cuda_stream) {
+  if (int r = ax_check(cfg, mode, batch, frames, t_samples)) return r;
+  CWG_REQUIRE(w && w->b1 && w->b2 && w->eo_b && w->start_w && w->start_b, "missing weight arrays");
+  if (mode == CWG_MODE_FFMA) CWG_REQUIRE(w->w1_f32 && w->w2_f32, "fp32 weight planes missing");
+  else if (mode == CWG_MODE_F16F8) CWG_REQUIRE(w->w1_hi && w->w1_h8 && w->w1_l8 && w->w2_hi && w->w2_h8 && w->w2_l8, "fp16 / e5m2 weight planes missing");
+  else CWG_REQUIRE(w->w1_hi && w->w2_hi && w->w1_lo && w->w2_lo, "bf16 hi/lo weight planes missing");
+  CWG_REQUIRE(w_fwd && logabsdet && mel && audio && z && logp_terms, "NULL tensor argument");
+  CWG_REQUIRE(workspace != nullptr && ((uintptr_t)workspace % 1024) == 0, "workspace must be 1024-byte aligned");
+  const AxFwdLayout l = ax_fwd_layout(cfg, mode, batch, frames, t_samples);
+  CWG_REQUIRE(l.bytes <= workspace_bytes, "workspace too small: need %zu, got %zu", l.bytes, workspace_bytes);
+  Dims d = l.d;
+  d.b1_batch = b1_batch;             // per-utterance gate bias (cwg_ax_speaker_bias) or NULL
+  Workspace ws;
+  carve(d, mode, workspace, &ws);
+  double* ls_part = (double*)((char*)workspace + l.ls_part);
+  double* z2_part = (double*)((char*)workspace + l.z2_part);
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  const bool tc = mode != CWG_MODE_FFMA;
+  const int npass = mode_npass(mode), xfmt = mode_xfmt(mode);
+  const int F = cfg->n_flows, L = cfg->n_layers;
+  const size_t nblk = (size_t)fwd_blocks(d);
+  void* x0 = tc ? (void*)ws.xb[0] : (void*)ws.x[0];
+  void* h2 = tc ? (void*)ws.h2b : (void*)ws.h2;
+  void* a0 = (tc && fold_active(d, w)) ? ws.a0 : nullptr;
+  CWG_CHECK_CUDA(cudaMemsetAsync(ws.status, 0, sizeof(int), s));     // status word as in cwg_forward
+  set_range_flag(mode == CWG_MODE_F16F8 ? ws.status : nullptr);
+  auto run = [&]() -> int {
+  if (int r = launch_mel_up(xfmt, mel, h2, d.B, d.M, frames, frames, d.Tp, d.H, upsample_linear, s)) return r;
+  // z = audio, then (mix_first) W_0 and the start conv of flow 0
+  if (int r = launch_fwd_boundary(cfg, d, w, w_fwd, xfmt, -1, 0, audio, z, nullptr, nullptr, nullptr, nullptr, x0, a0, s,
+                                  mix_first ? -2 : -1)) return r;
+  for (int k = 0; k < F; ++k) {
+    for (int i = 0; i < L; ++i) {
+      if (tc) {
+        if (int r = layer_tc(cfg, d, w, npass, k, i, ws, z, s)) return r;
+      } else {
+        if (int r = launch_layer_ffma(d, w, k, i, ws.x[i & 1], ws.x[(i + 1) & 1], ws.h2, ws.eo, ws.pre, ws.acts, s)) return r;
+      }
+    }
+    // coupling of flow k, then W_k (mix last) or W_{k+1} (mix first), then the start conv of flow k+1 (last: z^2)
+    if (int r = launch_fwd_boundary(cfg, d, w, w_fwd, xfmt, k, k + 1 < F ? k + 1 : -1, nullptr, z, ws.eo, nullptr,
+                                    ls_part + (size_t)k * batch * nblk, z2_part, x0, a0, s, mix_first ? -2 : k)) return r;
+  }
+  return launch_fwd_reduce(d, ls_part, z2_part, logabsdet, logp_terms, s);
+  };
+  const int rc = run();
+  set_range_flag(nullptr);
+  if (rc) return rc;
+  if (mode == CWG_MODE_F16F8) return launch_nonfinite(z, (size_t)batch * t_samples, ws.status, s, false);
+  return 0;
+}
+
 int cwg_ax_speaker_bias(const cwg_config* cfg, const float* b1, const float* spk_w, const float* spk_embed,
                         int speaker_embed_dim, int n_speakers, const int64_t* speaker_ids, int batch,
                         float* b1_batch, void* cuda_stream) {

@@ -122,10 +122,12 @@ int launch_mel_up(int xfmt, const float* mel, void* out, int B, int M, int frame
 // One launch per flow boundary: coupling of flow_done (-1: none; audio_in != NULL copies the waveform in first), log_s
 // store (log_s may be NULL), per-block sums of log_s into ls_part [B][fwd_blocks], then W of flow_next and its start conv
 // into x_out (or the layer-0 fold planes into a0_out).  flow_next = -1 ends the pass: per-block sums of z^2 into z2_part.
+// mix_flow: -2 = W of flow_next before its start conv (mix first); otherwise W of flow mix_flow over its n_rem right after
+// the coupling, and none before the start conv (mix last; -1 = no mixing in this launch).
 int fwd_blocks(const Dims& d);
 int launch_fwd_boundary(const cwg_config* cfg, const Dims& d, const cwg_weights* w, const float* w_fwd, int xfmt,
                         int flow_done, int flow_next, const float* audio_in, float* audio, const float* eo, float* log_s,
-                        double* ls_part, double* z2_part, void* x_out, void* a0_out, cudaStream_t s);
+                        double* ls_part, double* z2_part, void* x_out, void* a0_out, cudaStream_t s, int mix_flow = -2);
 // terms [B][3] = {sum z^2, sum log_s, T' * sum_k log|det W_k|} from the partials (ls_part [F][B][fwd_blocks])
 int launch_fwd_reduce(const Dims& d, const double* ls_part, const double* z2_part, const double* logabsdet, double* terms,
                       cudaStream_t s);

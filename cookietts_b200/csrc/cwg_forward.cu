@@ -1,6 +1,8 @@
 // Flow boundary of WaveGlow's forward direction (audio -> z, glow.py `WaveGlow.forward` in NVIDIA's formulation):
 //   flow k   : audio_1 = exp(log_s) * audio_1 + b            (coupling, after WN_k)
 //   flow k+1 : audio   = W_{k+1} audio   on the trailing n_rem_{k+1} columns, then start_{k+1}(audio_0) -> x_0
+// The ax model with mix_first=False (cwg_ax_forward) mixes after the coupling instead: flow k's W_k follows its own
+// coupling in the same launch (k_fwd_boundary_mixlast).
 // The WN layers between two boundaries are the kernels `infer` runs (cwg_ps.cu, cwg_tc512.cu, cwg_simple.cu).
 // Sums are deterministic: each block writes one fp64 partial per utterance (a fixed shuffle tree), and k_fwd_reduce adds
 // the partials in a fixed order.  No float atomics.
@@ -96,10 +98,13 @@ __device__ __forceinline__ void store_x(const FwdP& p, size_t idx, const float* 
 }
 
 // One block = TBF group-steps of utterance blockIdx.y.  Phase 1: thread -> group-step (input copy, coupling of flow_done,
-// log_s store, W_{flow_next} mixing, layer-0 fold planes); block partial sums.  Phase 2 (no fold): the start conv of
-// flow_next, warp -> group-step and lane -> 8 (MG = 16) or 4 (MG = 32) consecutive channels; VEC = false: any C (fp32).
-template <int XFMT, int MG, bool VEC>
-__global__ void __launch_bounds__(TBF) k_fwd_boundary(FwdP p) {
+// log_s store, mixing, layer-0 fold planes); block partial sums.  Phase 2 (no fold): the start conv of flow_next, warp ->
+// group-step and lane -> 8 (MG = 16) or 4 (MG = 32) consecutive channels; VEC = false: any C (fp32).
+// MIX_LAST = false: W_{flow_next} mixes before the start conv (p.wmix).  MIX_LAST = true (the ax model's mix_first=False):
+// wmix_done (may be NULL) mixes the trailing n_rem_done columns right after the coupling, and nothing mixes before the
+// start conv - flow_next's own W follows its coupling in the next launch.
+template <int XFMT, int MG, bool VEC, bool MIX_LAST>
+__device__ __forceinline__ void fwd_boundary(const FwdP& p, const float* wmix_done, int n_rem_done) {
   __shared__ __align__(16) float a_s[TBF][MG / 2];
   __shared__ double red[TBF / 32];
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, b = blockIdx.y;
@@ -130,7 +135,20 @@ __global__ void __launch_bounds__(TBF) k_fwd_boundary(FwdP p) {
         if (p.log_s) __stcs(p.log_s + ((size_t)b * p.n_half + j) * p.Tp + t, ls);
       }
     }
-    if (p.do_next) {                                               // audio = conv1d(audio, W), glow.py:85-99 (forward branch)
+    if constexpr (MIX_LAST) {
+      if (wmix_done) {                                             // efficient_model_ax.py mix_first=False: W_k after coupling k
+        const int off = p.G - n_rem_done;
+        float v[MG];
+        for (int c = 0; c < n_rem_done; ++c) v[c] = a[off + c];
+        for (int r = 0; r < n_rem_done; ++r) {
+          float acc = 0.f;
+          for (int c = 0; c < n_rem_done; ++c) acc = fmaf(__ldg(wmix_done + r * MG + c), v[c], acc);
+          a[off + r] = acc;
+        }
+      }
+      if (!p.do_next)
+        for (int g = 0; g < p.G; ++g) z2 = fma((double)a[g], (double)a[g], z2);
+    } else if (p.do_next) {                                        // audio = conv1d(audio, W), glow.py:85-99 (forward branch)
       const int off = p.G - p.n_rem2;
       float v[MG];
       for (int c = 0; c < p.n_rem2; ++c) v[c] = a[off + c];
@@ -218,6 +236,16 @@ __global__ void __launch_bounds__(TBF) k_fwd_boundary(FwdP p) {
       store_x<XFMT, NC>(p, (size_t)(m0 + r) * p.C + c, x);
     }
   }
+}
+
+template <int XFMT, int MG, bool VEC>
+__global__ void __launch_bounds__(TBF) k_fwd_boundary(FwdP p) {
+  fwd_boundary<XFMT, MG, VEC, false>(p, nullptr, 0);
+}
+
+template <int XFMT, int MG, bool VEC>
+__global__ void __launch_bounds__(TBF) k_fwd_boundary_mixlast(FwdP p, const float* wmix_done, int n_rem_done) {
+  fwd_boundary<XFMT, MG, VEC, true>(p, wmix_done, n_rem_done);
 }
 
 // terms[b] = {sum z^2, sum log_s (all flows), T' * sum_k log|det W_k|}: the block partials added in a fixed order
@@ -331,7 +359,12 @@ __global__ void __launch_bounds__(TBF) k_wf_fwd_boundary(WfFwdP p) {
 }
 
 template <int XFMT, int MG>
-void launch_fb(dim3 grid, bool vec, const FwdP& p, cudaStream_t s) {
+void launch_fb(dim3 grid, bool vec, const FwdP& p, bool mix_last, const float* wmix_done, int n_rem_done, cudaStream_t s) {
+  if (mix_last) {
+    if (vec) k_fwd_boundary_mixlast<XFMT, MG, true><<<grid, TBF, 0, s>>>(p, wmix_done, n_rem_done);
+    else if constexpr (XFMT == 0) k_fwd_boundary_mixlast<XFMT, MG, false><<<grid, TBF, 0, s>>>(p, wmix_done, n_rem_done);
+    return;
+  }
   if (vec) k_fwd_boundary<XFMT, MG, true><<<grid, TBF, 0, s>>>(p);
   else if constexpr (XFMT == 0) k_fwd_boundary<XFMT, MG, false><<<grid, TBF, 0, s>>>(p);   // other widths: fp32 only
 }
@@ -342,7 +375,8 @@ int fwd_blocks(const Dims& d) { return (d.Tp + TBF - 1) / TBF; }
 
 int launch_fwd_boundary(const cwg_config* cfg, const Dims& d, const cwg_weights* w, const float* w_fwd, int xfmt,
                         int flow_done, int flow_next, const float* audio_in, float* audio, const float* eo, float* log_s,
-                        double* ls_part, double* z2_part, void* x_out, void* a0_out, cudaStream_t s) {
+                        double* ls_part, double* z2_part, void* x_out, void* a0_out, cudaStream_t s, int mix_flow) {
+  const bool mix_last = mix_flow != -2;
   FwdP p{};
   p.Tp = d.Tp; p.G = d.G; p.C = d.C; p.BT = d.BT; p.nblk = fwd_blocks(d);
   p.audio_in = audio_in; p.audio = audio;
@@ -355,26 +389,34 @@ int launch_fwd_boundary(const cwg_config* cfg, const Dims& d, const cwg_weights*
   if (p.do_flow) { int nr; flow_channels(cfg, flow_done, &nr, &p.n_half); p.n_rem = nr; }
   if (p.do_next) {
     flow_channels(cfg, flow_next, &p.n_rem2, &p.n_half2);
-    p.wmix = w_fwd + (size_t)flow_next * d.MG * d.MG;
+    p.wmix = mix_last ? nullptr : w_fwd + (size_t)flow_next * d.MG * d.MG;
     p.start_w = w->start_w + (size_t)flow_next * d.C * (d.MG / 2);
     p.start_b = w->start_b + (size_t)flow_next * d.C;
   }
   CWG_REQUIRE(p.do_flow || p.do_next, "forward boundary: nothing to do");
   CWG_REQUIRE(!p.do_flow || (eo && ls_part), "forward boundary: eo / partials missing");
   CWG_REQUIRE(p.do_next || z2_part, "forward boundary: z^2 partials missing");
+  CWG_REQUIRE(mix_flow >= -2 && mix_flow < cfg->n_flows, "forward boundary: mix flow out of range");
+  const float* wmix_done = nullptr;
+  int n_rem_done = 0;
+  if (mix_flow >= 0) {
+    int nh;
+    flow_channels(cfg, mix_flow, &n_rem_done, &nh);
+    wmix_done = w_fwd + (size_t)mix_flow * d.MG * d.MG;
+  }
   const bool wide = d.MG != 16;
   CWG_REQUIRE(!wide || p.a0_out == nullptr, "the layer-0 fold takes n_group <= 16");
   const bool vec = (d.C & 7) == 0 && ((uintptr_t)x_out & 15) == 0;
   CWG_REQUIRE(vec || xfmt == 0, "the tensor-core modes need n_channels % 8 == 0");
   const dim3 grid((unsigned)p.nblk, (unsigned)d.B);
   if (wide) {
-    if (xfmt == 0) launch_fb<0, 32>(grid, vec, p, s);
-    else if (xfmt == 2) launch_fb<2, 32>(grid, vec, p, s);
-    else launch_fb<1, 32>(grid, vec, p, s);
+    if (xfmt == 0) launch_fb<0, 32>(grid, vec, p, mix_last, wmix_done, n_rem_done, s);
+    else if (xfmt == 2) launch_fb<2, 32>(grid, vec, p, mix_last, wmix_done, n_rem_done, s);
+    else launch_fb<1, 32>(grid, vec, p, mix_last, wmix_done, n_rem_done, s);
   } else {
-    if (xfmt == 0) launch_fb<0, 16>(grid, vec, p, s);
-    else if (xfmt == 2) launch_fb<2, 16>(grid, vec, p, s);
-    else launch_fb<1, 16>(grid, vec, p, s);
+    if (xfmt == 0) launch_fb<0, 16>(grid, vec, p, mix_last, wmix_done, n_rem_done, s);
+    else if (xfmt == 2) launch_fb<2, 16>(grid, vec, p, mix_last, wmix_done, n_rem_done, s);
+    else launch_fb<1, 16>(grid, vec, p, mix_last, wmix_done, n_rem_done, s);
   }
   CWG_CHECK_CUDA(cudaGetLastError());
   return 0;

@@ -1,5 +1,6 @@
 """Drop-in for the reference's "ax" model `efficient_model_ax.py::WaveGlow` with `waveflow=False`
-(1-D WN + affine coupling + invertible 1x1 conv / PermuteHeight), inverse pass only.
+(1-D WN + affine coupling + invertible 1x1 conv / PermuteHeight): the inverse pass, plus the no-grad forward direction
+(audio -> z, log-likelihood) as `encode` / `log_prob` (cwg_ax_forward, on the same layer kernels).
 
 It runs on the SAME sm_100a layer / boundary kernels as the classic model (csrc/cwg_ps.cu,
 cwg_simple.cu): the cond vector is the F.interpolate'd mel (efficient_model_ax.py:171-182, computed
@@ -53,7 +54,9 @@ def pack_ax_state_dict(sd, pc: PackConfig, channel_mixing: str, planes=("hi", "l
     (AffineCouplingBlock.inverse: `log_s, t = WN(...)`, efficient_modules.py:102-103).  Arrays indexed by latent
     channels are padded to MG = group_pad(n_group) (include/cwg.h CWG_GROUP_PAD).  `wn_speaker_dim` > 0: the last
     columns of every WN's cond layer multiply its own speaker embedding (glow_ax.py:284-286, :378-381); they are
-    returned as `spk_w` [F][L][2C][E] next to the tables `spk_embed` [F][S][E] (cwg_ax_speaker_bias)."""
+    returned as `spk_w` [F][L][2C][E] next to the tables `spk_embed` [F][S][E] (cwg_ax_speaker_bias).  The forward
+    direction's mixing (cwg_ax_forward) comes as `w_fwd` [F][MG][MG] (W_k zero-padded; for PermuteHeight the transpose of
+    winv[k]) and `logabsdet` [F] fp64 (log|det W_k|, 0 for a permutation), both computed in fp64."""
     F, L, Cc, H, ks, M = pc.n_flows, pc.n_layers, pc.n_channels, pc.cond_hidden, pc.kernel_size, pc.n_mel
     MG, E = group_pad(pc.n_group), int(wn_speaker_dim)
     K1, N2 = ks * Cc + H, Cc + MG
@@ -61,6 +64,7 @@ def pack_ax_state_dict(sd, pc: PackConfig, channel_mixing: str, planes=("hi", "l
     w2 = np.zeros((F, L, N2, Cc)); b2 = np.zeros((F, L, Cc)); eo_b = np.zeros((F, MG))
     start_w = np.zeros((F, Cc, MG // 2)); start_b = np.zeros((F, Cc))
     winv = np.zeros((F, MG, MG))
+    w_fwd, logabsdet = np.zeros((F, MG, MG)), np.zeros(F)     # forward direction (cwg_ax_forward): W_k, log|det W_k|
     w0 = np.zeros((F, 2 * Cc, 48))                           # layer-0 fold: in_layers.0 * start (include/cwg.h w0_hi / w0_lo)
     spk_w = np.zeros((F, L, 2 * Cc, max(E, 1)), np.float32)
     spk_embed = []
@@ -103,10 +107,15 @@ def pack_ax_state_dict(sd, pc: PackConfig, channel_mixing: str, planes=("hi", "l
         if channel_mixing == "permuteheight":
             for c, src in enumerate(permute_height_index(k, n_rem)):
                 winv[k, c, src] = 1.0
+            w_fwd[k] = winv[k].T                             # the permutation winv[k] undoes; log|det| = 0
         else:
             winv[k, :n_rem, :n_rem] = np.linalg.inv(_np(sd[f"convinv.{k}.weight"]).reshape(n_rem, n_rem))
+            W = np.asarray(_np(sd[f"convinv.{k}.weight"]), np.float64).reshape(n_rem, n_rem)
+            w_fwd[k, :n_rem, :n_rem] = W
+            logabsdet[k] = np.linalg.slogdet(W)[1]
     out = {"b1": b1.astype(np.float32), "b2": b2.astype(np.float32), "eo_b": eo_b.astype(np.float32),
-           "start_w": start_w.astype(np.float32), "start_b": start_b.astype(np.float32), "winv": winv.astype(np.float32)}
+           "start_w": start_w.astype(np.float32), "start_b": start_b.astype(np.float32), "winv": winv.astype(np.float32),
+           "w_fwd": w_fwd.astype(np.float32), "logabsdet": logabsdet}
     if E:
         out["spk_w"], out["spk_embed"] = spk_w, np.stack(spk_embed)
     for name, arr in (("w1", w1), ("w2", w2)):
@@ -353,7 +362,8 @@ class WaveGlowAx(nn.Module, AxFrontEndMixin):
         return self
 
     def forward(self, *a, **kw):
-        raise NotImplementedError("only the inverse pass is in scope of this implementation")
+        raise NotImplementedError("only the inverse pass is in scope of this implementation (the forward direction, "
+                                  "audio -> z, is `encode` / `log_prob`)")
 
     def _device(self):
         return self.WN[0].WN.end.weight.device
@@ -482,6 +492,14 @@ class WaveGlowAx(nn.Module, AxFrontEndMixin):
             lib.cwg_ax_speaker_bias.restype = C.c_int
             lib.cwg_ax_speaker_bias.argtypes = [C.POINTER(_cabi.CwgConfig), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                                 C.c_void_p, C.c_int, C.c_void_p, C.c_void_p]
+            lib.cwg_ax_forward_workspace_bytes.restype = C.c_size_t
+            lib.cwg_ax_forward_workspace_bytes.argtypes = [C.POINTER(_cabi.CwgConfig), C.c_int, C.c_int, C.c_int, C.c_int]
+            lib.cwg_ax_forward_launch_count.restype = C.c_int
+            lib.cwg_ax_forward_launch_count.argtypes = [C.POINTER(_cabi.CwgConfig), C.c_int]
+            lib.cwg_ax_forward.restype = C.c_int
+            lib.cwg_ax_forward.argtypes = [C.POINTER(_cabi.CwgConfig), C.POINTER(_cabi.CwgWeights), C.c_void_p, C.c_void_p, C.c_int,
+                                           C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_size_t, C.c_int, C.c_void_p, C.c_void_p]
             lib._ax_bound = True
         return lib
 
@@ -622,3 +640,106 @@ class WaveGlowAx(nn.Module, AxFrontEndMixin):
         if artifact_trimming > 0:
             audio = audio[:, :-artifact_trimming * self.hop_length]
         return audio.to(in_dtype)
+
+    # ------------------------------------------------------------------ forward direction (audio -> z), cwg_ax_forward
+    def _forward_terms(self, spect, audio, speaker_ids):
+        """audio -> (z [B, T], logp_terms [B, 3] fp64 {sum z^2, sum log_s, T' * sum log|det W|}) on the device."""
+        if self.general:
+            raise NotImplementedError("cookietts_b200.WaveGlowAx: the forward direction (encode / log_prob) runs on the packed "
+                                      "layer kernels only; this WN_config runs in the general fp32 mode")
+        if self.vol_scaling or self.preempthasis:
+            raise NotImplementedError("cookietts_b200.WaveGlowAx: the forward direction is not built for preceived_vol_scaling / "
+                                      "preempthasis models (their post-filter's forward map and Jacobian are not pinned)")
+        if spect.dim() == 2:
+            spect = spect[None]
+        if audio.dim() == 1:
+            audio = audio[None]
+        B, T = audio.shape
+        if T < self.n_group or T % self.n_group:
+            raise ValueError(f"audio length {T} must be a positive multiple of n_group = {self.n_group}")
+        if spect.shape[0] != B:
+            raise ValueError(f"batch mismatch: spect has {spect.shape[0]} utterances, audio {B}")
+        dev = self._device()
+        if dev.type != "cuda":
+            raise RuntimeError("cookietts_b200.WaveGlowAx needs the module on a CUDA device (no CPU fallback)")
+        lib = self._bind()
+        mode = _cabi.MODES[self.precision]
+        cond = spect.to(device=dev, dtype=torch.float32)
+        if self.shift_spect != 0.:
+            cond = cond + self.shift_spect
+        if self.scale_spect != 1.:
+            cond = cond * self.scale_spect
+        cond = cond.contiguous()
+        audio = audio.to(device=dev, dtype=torch.float32).contiguous()
+        with torch.cuda.device(dev):
+            self._ensure_packed()
+            stream = torch.cuda.current_stream(dev).cuda_stream
+            ids = None
+            if self.wn_speaker_embed_dim or self.speaker_embed_dim:      # as in `inverse`
+                if speaker_ids is None:
+                    raise Exception("This WaveFlow/WaveGlow model requires speaker ids or speaker embeddings.")
+                ids = torch.as_tensor(speaker_ids, device=dev).long().view(-1).contiguous()
+                if ids.numel() != B:
+                    raise ValueError(f"speaker_ids must hold one id per utterance ({B}), got {ids.numel()}")
+                if int(ids.min()) < 0 or int(ids.max()) >= 512:
+                    raise IndexError("speaker id out of range [0, 512)")
+            cond = self._fe_apply(cond, ids, T // self.n_group).contiguous()
+            frames = cond.shape[2]
+            nbytes = lib.cwg_ax_forward_workspace_bytes(self._ccfg, mode, B, frames, T)
+            if nbytes == 0:
+                raise _cabi.CwgError(lib.cwg_last_error().decode())
+            b1_batch = None
+            if self.wn_speaker_embed_dim:
+                pc = self.pack_config
+                b1_batch = torch.empty(B, pc.n_flows, pc.n_layers, 2 * pc.n_channels, device=dev, dtype=torch.float32)
+                _cabi.check(lib.cwg_ax_speaker_bias(self._ccfg, self._packed["b1"].data_ptr(), self._packed["spk_w"].data_ptr(),
+                                                    self._packed["spk_embed"].data_ptr(), self.wn_speaker_embed_dim,
+                                                    self._packed["spk_embed"].shape[1], ids.data_ptr(), B, b1_batch.data_ptr(),
+                                                    stream))
+            ws = torch.empty(nbytes + 1024, dtype=torch.uint8, device=dev)
+            ws_ptr = (ws.data_ptr() + 1023) // 1024 * 1024
+            z = torch.empty(B, T, device=dev, dtype=torch.float32)
+            terms = torch.empty(B, 3, device=dev, dtype=torch.float64)
+            _cabi.check(lib.cwg_ax_forward(self._ccfg, self._cw, self._packed["w_fwd"].data_ptr(),
+                                           self._packed["logabsdet"].data_ptr(), mode, cond.data_ptr(), frames,
+                                           int(self.upsample_linear), int(self.mix_first), audio.data_ptr(), T, z.data_ptr(),
+                                           terms.data_ptr(), ws_ptr, ws.numel() - (ws_ptr - ws.data_ptr()), B,
+                                           b1_batch.data_ptr() if b1_batch is not None else None, stream))
+            if self.precision == "f16f8":
+                status = torch.empty(1, dtype=torch.int32, device=dev)        # cwg_infer_status copies the word over it
+                _cabi.check(lib.cwg_infer_status(ws_ptr, status.data_ptr(), stream))
+                self.last_status = int(status.item())
+                if self.last_status:
+                    raise _cabi.CwgError(f"WaveGlowAx(precision='f16f8'): fp16 range guard tripped (status {self.last_status}); "
+                                         "construct the model with precision='bf16x3'")
+        return z, terms
+
+    @torch.no_grad()
+    def encode(self, spect, audio, speaker_ids=None):
+        """audio [B, T] -> z [B, T] in the layout `inverse(z, spect)` takes, so `inverse(encode(spect, x), spect)`
+        reproduces x.  The cond is the one `inverse` builds from `spect` (no artifact-trimming frame: pair it with
+        `inverse`, not with `infer`, whose output is one hop shorter)."""
+        return self._forward_terms(spect, audio, speaker_ids)[0]
+
+    @torch.no_grad()
+    def log_prob(self, spect, audio, sigma=1.0, speaker_ids=None):
+        """Per-utterance log-density of `audio` in nats, float64 [B]:
+        sum(-z^2 / (2 sigma^2)) - (T/2) log(2 pi sigma^2) + sum_k sum log_s_k + T' sum_k log|det W_k|."""
+        _, terms = self._forward_terms(spect, audio, speaker_ids)
+        T = audio.shape[-1]
+        s2 = float(sigma) ** 2
+        return -terms[:, 0] / (2 * s2) - 0.5 * T * float(np.log(2 * np.pi * s2)) + terms[:, 1] + terms[:, 2]
+
+    def forward_launch_count(self) -> int:
+        """Kernels one `encode` / `log_prob` call launches in the flows: n_flows * (n_layers * per-layer launches + 1) + 3
+        (+ 1 in 'f16f8' for the non-finite scan of z).  The conditioning front end and, with WN-level speaker embeddings,
+        the one speaker-bias kernel come on top."""
+        if self.general:
+            raise NotImplementedError("cookietts_b200.WaveGlowAx: the forward direction runs on the packed layer kernels only; "
+                                      "this WN_config runs in the general fp32 mode")
+        lib = self._bind()
+        self._ensure_packed()
+        n = int(lib.cwg_ax_forward_launch_count(self._ccfg, _cabi.MODES[self.precision]))
+        if n < 0:
+            raise _cabi.CwgError(lib.cwg_last_error().decode())
+        return n

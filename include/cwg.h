@@ -254,6 +254,27 @@ int cwg_ax_infer(const cwg_config* cfg, const cwg_weights* w, int mode,
                  const float* z, float sigma, float* audio, void* workspace, size_t workspace_bytes,
                  int batch, int t_samples, const float* b1_batch, void* cuda_stream);
 
+/* Forward direction of the same model (audio -> z, log-likelihood terms; no-grad evaluation).  Flows run k = 0 .. F-1:
+ * at k % n_early_every == 0, k > 0 the first n_early_size channels leave (they stay in their columns of the
+ * [batch][T'][n_group] state, which ends as z in the layout cwg_ax_infer takes); then mix_first: audio = W_k audio,
+ * (t, log_s) = WN_k(audio_0, cond), audio_1 = exp(log_s) * audio_1 + t;  mix_first = 0: the coupling first, then W_k.
+ * The cond is the one cwg_ax_infer builds from the same mel (no pad frames), and the layer launches are its own.
+ *   w_fwd      [F][MG][MG] fp32 device: W_k zero-padded (convinv.{k}.weight; for PermuteHeight the transpose of winv[k])
+ *   logabsdet  [F] fp64 device: log|det W_k| (0 for a permutation)
+ *   audio      [batch][t_samples] fp32, t_samples a positive multiple of n_group
+ *   z          [batch][t_samples] fp32 out (may alias audio)
+ *   logp_terms [batch][3] fp64 out: sum z^2, sum_k sum log_s_k, T' * sum_k log|det W_k| per utterance
+ *   b1_batch   as in cwg_ax_infer (WN-level speaker embeddings) or NULL
+ * Sums are reduced in a fixed order: identical calls give identical bytes, and row b of a batch equals the call for
+ * utterance b alone.  The status word (cwg_infer_status) works as for cwg_forward, with z in place of the waveform. */
+size_t cwg_ax_forward_workspace_bytes(const cwg_config* cfg, int mode, int batch, int frames, int t_samples);
+/* Kernels cwg_ax_forward launches: F * (L * per-layer launches + 1) + 3, plus 1 in CWG_MODE_F16F8. -1 on error. */
+int cwg_ax_forward_launch_count(const cwg_config* cfg, int mode);
+int cwg_ax_forward(const cwg_config* cfg, const cwg_weights* w, const float* w_fwd, const double* logabsdet, int mode,
+                   const float* mel, int frames, int upsample_linear, int mix_first, const float* audio, int t_samples,
+                   float* z, double* logp_terms, void* workspace, size_t workspace_bytes, int batch,
+                   const float* b1_batch, void* cuda_stream);
+
 /* WN-level speaker embedding (glow_ax.py:284-286, :378-381: every flow's WN concatenates speaker_embed(speaker_id),
  * constant over time, to its cond input before the 1x1 cond layer).  A time-constant input of a 1x1 conv is a bias, so
  * the branch is evaluated once per call instead of per group-step:
