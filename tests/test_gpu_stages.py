@@ -74,6 +74,35 @@ def rel_err(a, b):
     return float((a.double() - b.double()).abs().max() / b.double().abs().max())
 
 
+def wn_layer_ref(pk, flow, layer, x, h2, eo):
+    """fp64 evaluation of packed WN layer `layer` of `flow` (glow.py:201-220) on x [B, T', C] and h2 [B, T', H], for any
+    C (256 / 512) and group padding MG (16 / 32).  The dilated taps are zero-padded at each utterance's ends; eo [B, T', MG]
+    is the accumulator before the layer (ignored at layer 0, where eo_b overwrites it).  Returns (x_new, eo_new); x_new is
+    None for the last layer, which has no residual."""
+    n_layers, Cc = pk["b2"].shape[1], x.shape[2]
+    tp, d = x.shape[1], 2 ** layer
+    xd = x.double()
+    xp = torch.nn.functional.pad(xd, (0, 0, d, d))
+    a = torch.cat([xp[:, 0:tp], xd, xp[:, 2 * d:2 * d + tp], h2.double()], dim=2)
+    pre = a @ pk["w1_f32"][flow, layer].double().T + pk["b1"][flow, layer].double()
+    acts = torch.tanh(pre[..., :Cc]) * torch.sigmoid(pre[..., Cc:])
+    rs = acts @ pk["w2_f32"][flow, layer].double().T
+    eo_new = (pk["eo_b"][flow].double() if layer == 0 else eo.double()) + rs[..., Cc:]
+    x_new = xd + rs[..., :Cc] + pk["b2"][flow, layer].double() if layer < n_layers - 1 else None
+    return x_new, eo_new
+
+
+def cond_ref(pk, pc, flow, mel, bias):
+    """fp64 evaluation of the packed cond GEMM of `flow` (upsample + squeeze + cond layers folded, glow.py:318-324,198-199):
+    mel [B, n_mel, T_mel], bias [B, F, H] (one row per utterance) -> H2 [B, T_mel * P, H]."""
+    B, M, tm = mel.shape
+    mel4 = torch.zeros(B, tm, pc.taps * M, device=mel.device, dtype=torch.float64)
+    for j in range(pc.taps):
+        mel4[:, j:, j * M:(j + 1) * M] = mel.double().transpose(1, 2)[:, :tm - j]
+    h = mel4.reshape(B * tm, -1) @ pk["cond_w_f32"][flow][:, :pc.taps * M].double().T
+    return h.reshape(B, tm * pc.phases, -1) + bias[:, flow, None, :].double()
+
+
 def run_cond(model, mode, flow, mel, out):
     lib = _cabi.load()
     bias = model._cond_bias(B, None)
@@ -93,10 +122,7 @@ def test_cond_stage(models, flow):
     run_cond(models["ffma"], _cabi.MODE_FFMA, flow, mel, h_f)
     # fp64 evaluation of the packed form
     pk = models["ffma"].packed_views()
-    mel4 = torch.zeros(B, TM, pc.taps * 80, device="cuda", dtype=torch.float64)
-    for j in range(pc.taps):
-        mel4[:, j:, j * 80:(j + 1) * 80] = mel.double().transpose(1, 2)[:, :TM - j]
-    ref = (mel4.reshape(B * TM, -1) @ pk["cond_w_f32"][flow][:, :pc.taps * 80].double().T).reshape(B, tp, H) + pk["cond_b_base"][flow].double()
+    ref = cond_ref(pk, pc, flow, mel, pk["cond_b_base"][None].expand(B, -1, -1))
     assert rel_err(h_f, ref) < 1e-5
     for prec, mode, tol in (("bf16x3", _cabi.MODE_BF16X3, 2e-5), ("bf16", _cabi.MODE_BF16, 2e-2)):
         h_t = torch.zeros(2, B, tp, H, device="cuda", dtype=torch.bfloat16)
@@ -134,16 +160,7 @@ def test_layer_stage(models, layer):
                                  h2.data_ptr(), eo_f.data_ptr(), ptr, n, B, TM, stream))
     torch.cuda.synchronize()
     # fp64 evaluation of the packed form
-    pk = mf.packed_views()
-    d = 2 ** layer
-    xp = torch.zeros(B, tp + 2 * d, Cc, device="cuda", dtype=torch.float64)
-    xp[:, d:d + tp] = x.double()
-    a = torch.cat([xp[:, 0:tp], xp[:, d:d + tp], xp[:, 2 * d:2 * d + tp], h2.double()], dim=2)
-    pre = a @ pk["w1_f32"][flow, layer].double().T + pk["b1"][flow, layer].double()
-    acts = torch.tanh(pre[..., :Cc]) * torch.sigmoid(pre[..., Cc:])
-    rs = acts @ pk["w2_f32"][flow, layer].double().T
-    x_ref = x.double() + rs[..., :Cc] + pk["b2"][flow, layer].double()
-    eo_ref = (pk["eo_b"][flow].double() if layer == 0 else eo0.double()) + rs[..., Cc:]
+    x_ref, eo_ref = wn_layer_ref(mf.packed_views(), flow, layer, x, h2, eo0)
     assert rel_err(eo_f, eo_ref) < 1e-5
     if layer < pc.n_layers - 1:
         assert rel_err(xo_f, x_ref) < 1e-5
