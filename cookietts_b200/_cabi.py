@@ -15,6 +15,7 @@ MODE_FFMA, MODE_BF16X3, MODE_BF16, MODE_F16F8 = 0, 1, 2, 3
 MODES = {"ffma": MODE_FFMA, "bf16x3": MODE_BF16X3, "bf16": MODE_BF16, "f16f8": MODE_F16F8}
 EO_PAD = 16          # narrow layout; see packing.group_pad / include/cwg.h CWG_GROUP_PAD
 MAX_GROUP = 32
+RAGGED_MAX_BATCH = 1024  # include/cwg.h CWG_RAGGED_MAX_BATCH
 ABI_VERSION = 5
 
 
@@ -52,7 +53,8 @@ EXPORTS = ("cwg_abi_version", "cwg_last_error", "cwg_workspace_bytes", "cwg_laun
            "cwg_fd_workspace_bytes", "cwg_fd_launch_count", "cwg_fd_inverse",
            "cwg_axg_workspace_bytes", "cwg_axg_launch_count", "cwg_axg_flow", "cwg_group_transpose",
            "cwg_pack_forward", "cwg_forward_workspace_bytes", "cwg_forward_launch_count", "cwg_forward",
-           "cwg_ax_forward_workspace_bytes", "cwg_ax_forward_launch_count", "cwg_ax_forward")
+           "cwg_ax_forward_workspace_bytes", "cwg_ax_forward_launch_count", "cwg_ax_forward",
+           "cwg_ragged_workspace_bytes", "cwg_infer_ragged", "cwg_ragged_pairs")
 
 
 class CwgError(RuntimeError):
@@ -103,6 +105,14 @@ def load():
                               C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p]
     lib.cwg_infer_profiled.restype = C.c_int
     lib.cwg_infer_profiled.argtypes = lib.cwg_infer.argtypes + [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int]
+    lib.cwg_ragged_workspace_bytes.restype = C.c_size_t
+    lib.cwg_ragged_workspace_bytes.argtypes = [C.POINTER(CwgConfig), C.c_int, C.c_int, C.c_int]
+    lib.cwg_infer_ragged.restype = C.c_int
+    lib.cwg_infer_ragged.argtypes = [C.POINTER(CwgConfig), C.POINTER(CwgWeights), C.c_int,
+                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_void_p,
+                                     C.c_void_p, C.c_void_p, C.c_size_t, C.c_int, C.c_int, C.c_void_p]
+    lib.cwg_ragged_pairs.restype = C.c_int
+    lib.cwg_ragged_pairs.argtypes = [C.POINTER(CwgConfig), C.c_void_p, C.c_int, C.c_int, C.c_void_p]
     lib.cwg_cond.restype = C.c_int
     lib.cwg_cond.argtypes = [C.POINTER(CwgConfig), C.POINTER(CwgWeights), C.c_int, C.c_int,
                              C.c_void_p, C.c_void_p, C.c_void_p,

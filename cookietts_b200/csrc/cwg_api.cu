@@ -100,15 +100,56 @@ bool fold_active(const Dims& d, const cwg_weights* w) {
 }
 
 int layer_tc(const cwg_config* cfg, const Dims& d, const cwg_weights* w, int npass, int k, int i, const Workspace& ws,
-             const float* audio, cudaStream_t s) {
+             const float* audio, cudaStream_t s, const int* rag_len = nullptr, const int* rag_prefix = nullptr) {
   if (d.C == 512)
     return launch_layer_tc512(d, w, npass, k, i, ws.xb[i & 1], ws.xb[(i + 1) & 1], ws.h2b, ws.actsb, ws.eo, s);
   if (i == 0 && audio && fold_active(d, w)) {
     int n_rem, n_half;
     flow_channels(cfg, k, &n_rem, &n_half);
-    return launch_layer_ps(d, w, npass, k, i, ws.xb[0], ws.xb[1], ws.h2b, ws.eo, s, ws.a0, audio, d.G - n_rem, n_half);
+    return launch_layer_ps(d, w, npass, k, i, ws.xb[0], ws.xb[1], ws.h2b, ws.eo, s, ws.a0, audio, d.G - n_rem, n_half,
+                           rag_len, rag_prefix);
   }
-  return launch_layer_ps(d, w, npass, k, i, ws.xb[i & 1], ws.xb[(i + 1) & 1], ws.h2b, ws.eo, s);
+  return launch_layer_ps(d, w, npass, k, i, ws.xb[i & 1], ws.xb[(i + 1) & 1], ws.h2b, ws.eo, s, nullptr, nullptr, 0, 0,
+                         rag_len, rag_prefix);
+}
+
+// ---- ragged calls (cwg_infer_ragged) ----
+// pairs of 128-step tiles an utterance of `frames` mel frames runs per WN layer
+__host__ __device__ inline int ragged_pairs_of(int frames, int P) { return ((frames * P + 127) / 128 + 1) / 2; }
+
+int check_ragged(const cwg_config* cfg, int mode, int batch) {
+  CWG_REQUIRE(mode != CWG_MODE_FFMA && cfg->n_channels == 256,
+              "ragged batches need the 256-channel persistent layer kernel in a tensor-core mode (f16f8, bf16x3, bf16); "
+              "the 512-channel kernel pair and CWG_MODE_FFMA have no ragged form");
+  CWG_REQUIRE(batch <= CWG_RAGGED_MAX_BATCH, "ragged batches hold at most %d utterances (got %d); split the batch",
+              CWG_RAGGED_MAX_BATCH, batch);
+  return 0;
+}
+
+// Workspace of a ragged call: cwg_infer's, then len [B] (clamped frames) and the tile-pair prefix sums [B + 1]
+size_t ragged_plan_offset(const Dims& d, int mode) {
+  Workspace ws;
+  carve(d, mode, nullptr, &ws);
+  return ws.bytes;
+}
+size_t ragged_plan_bytes(int batch) { return align_up((size_t)(2 * batch + 1) * sizeof(int), 1024); }
+
+// one block: clamp the lengths into [1, Tm] (status bit 2 on a clamp) and scan the utterances' tile pairs
+__global__ void k_ragged_plan(const int32_t* __restrict__ lengths, int B, int Tm, int P, int* __restrict__ len,
+                              int* __restrict__ prefix, int* __restrict__ status) {
+  __shared__ int pairs[CWG_RAGGED_MAX_BATCH];
+  for (int b = threadIdx.x; b < B; b += blockDim.x) {
+    int l = lengths[b];
+    if (l < 1 || l > Tm) { atomicOr(status, 4); l = l < 1 ? 1 : Tm; }
+    len[b] = l;
+    pairs[b] = ragged_pairs_of(l, P);
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    int acc = 0;
+    for (int b = 0; b < B; ++b) { prefix[b] = acc; acc += pairs[b]; }
+    prefix[B] = acc;
+  }
 }
 
 int check_run(const cwg_config* cfg, const cwg_weights* w, int mode, int batch, int t_mel) {
@@ -317,6 +358,101 @@ int cwg_infer_profiled(const cwg_config* cfg, const cwg_weights* w, int mode,
     }
     // coupling inverse + W^-1 of flow k, then start conv of flow k-1 (glow.py:329-347, :189)
     if (int r = launch_flow_boundary(cfg, d, w, xfmt, k, k - 1, nullptr, sigma, audio, ws.eo, x0, s, -2, 0, a0)) return r;
+  }
+  return 0;
+  };
+  const int rc = run();
+  set_range_flag(nullptr);
+  if (rc) return rc;
+  if (mode == CWG_MODE_F16F8) return launch_nonfinite(audio, (size_t)batch * t_mel * cfg->hop_length, ws.status, s, false);
+  return 0;
+}
+
+// ---------------------------------------------------------------------------------------------
+// Ragged batches: cwg_infer's launch sequence with per-utterance lengths.  Zero invariant: throughout the call every row
+// t >= T'_b of the audio state, of eo, of both x buffers (all planes) and of the layer-0-fold planes is 0, so that a
+// dilated tap of a valid row reads the zero padding a call for utterance b alone would see, and nothing of the padding
+// (z, mel, stale workspace) can reach a valid row, the range flag or the waveform.  It is established once here (eo, x,
+// z -> audio); the layers keep it (k_layer_ps<..., RAGGED>), padded audio stays 0 through the boundaries (eo = 0 there:
+// (0 - 0) * exp(-0)), and the start-conv rows the boundaries write into the padding are zeroed after each of them.
+// ---------------------------------------------------------------------------------------------
+size_t cwg_ragged_workspace_bytes(const cwg_config* cfg, int mode, int batch, int t_mel) {
+  if (check_config(cfg) || check_mode(cfg, mode) || check_ragged(cfg, mode, batch)) return 0;
+  const size_t base = cwg_workspace_bytes(cfg, mode, batch, t_mel);
+  if (base == 0) return 0;
+  return ragged_plan_offset(make_dims(cfg, batch, t_mel), mode) + ragged_plan_bytes(batch) + 1024;
+}
+
+int cwg_ragged_pairs(const cwg_config* cfg, const int32_t* lengths, int batch, int t_mel, int32_t* prefix) {
+  if (check_config(cfg)) return -1;
+  if (!lengths || batch < 1 || t_mel < 1) { set_error("cwg_ragged_pairs: NULL lengths or batch / t_mel < 1"); return -1; }
+  const int P = cfg->hop_length / cfg->n_group;
+  if ((long long)t_mel * P >= (1ll << 31) / 4) { set_error("cwg_ragged_pairs: t_mel too large"); return -1; }
+  long long acc = 0;
+  for (int b = 0; b < batch; ++b) {
+    if (lengths[b] < 1 || lengths[b] > t_mel) {
+      set_error("lengths[%d] = %d is outside [1, t_mel = %d]", b, (int)lengths[b], t_mel);
+      return -1;
+    }
+    if (prefix) prefix[b] = (int32_t)acc;
+    acc += ragged_pairs_of(lengths[b], P);
+  }
+  if (acc >= (1ll << 31)) { set_error("cwg_ragged_pairs: too many tile pairs"); return -1; }
+  if (prefix) prefix[batch] = (int32_t)acc;
+  return (int)acc;
+}
+
+int cwg_infer_ragged(const cwg_config* cfg, const cwg_weights* w, int mode,
+                     const float* mel, const float* cond_bias, const float* z, float sigma, const int32_t* lengths,
+                     float* audio, void* workspace, size_t workspace_bytes,
+                     int batch, int t_mel, void* cuda_stream) {
+  if (int r = check_run(cfg, w, mode, batch, t_mel)) return r;
+  if (int r = check_ragged(cfg, mode, batch)) return r;
+  CWG_REQUIRE(mel && cond_bias && z && audio && lengths, "NULL tensor argument");
+  CWG_REQUIRE(workspace != nullptr && ((uintptr_t)workspace % 1024) == 0, "workspace must be 1024-byte aligned");
+  Dims d = make_dims(cfg, batch, t_mel);
+  Workspace ws;
+  carve(d, mode, workspace, &ws);
+  CWG_REQUIRE(ws.bytes + ragged_plan_bytes(batch) <= workspace_bytes, "workspace too small: need %zu, got %zu",
+              ws.bytes + ragged_plan_bytes(batch), workspace_bytes);
+  int* len = (int*)((char*)workspace + ws.bytes);
+  int* prefix = len + batch;
+  cudaStream_t s = (cudaStream_t)cuda_stream;
+  const int npass = mode_npass(mode), xfmt = mode_xfmt(mode);
+  const int F = cfg->n_flows, L = cfg->n_layers;
+  void* a0 = fold_active(d, w) ? ws.a0 : nullptr;
+  const size_t plane = (size_t)d.BT * d.C;
+
+  CWG_CHECK_CUDA(cudaMemsetAsync(ws.status, 0, sizeof(int), s));       // status word as in cwg_infer, + bit 2
+  set_range_flag(mode == CWG_MODE_F16F8 ? ws.status : nullptr);
+  // padded rows of the start-conv output the boundaries write: x_0 (or the layer-0-fold planes, constant-1 channel
+  // included) must read as the conv's zero padding
+  auto clear_x = [&](void* x) -> int {
+    if (int r = launch_ragged_rows(x, nullptr, plane * 2, 2, d.B, d.Tp, d.C / 2, len, d.P, s)) return r;   // 16-bit hi, lo
+    if (mode == CWG_MODE_F16F8)                                                                             // e5m2 planes
+      return launch_ragged_rows((char*)x + 4 * plane, nullptr, plane, 2, d.B, d.Tp, d.C / 4, len, d.P, s);
+    return 0;
+  };
+  auto clear_start = [&]() -> int {
+    return a0 ? launch_ragged_rows(a0, nullptr, (size_t)d.BT * 32, 2, d.B, d.Tp, 8, len, d.P, s) : clear_x(ws.xb[0]);
+  };
+  auto run = [&]() -> int {
+  k_ragged_plan<<<1, 1024, 0, s>>>(lengths, batch, t_mel, d.P, len, prefix, ws.status);
+  CWG_CHECK_CUDA(cudaGetLastError());
+  if (int r = launch_ragged_rows(ws.eo, nullptr, 0, 1, d.B, d.Tp, d.MG, len, d.P, s)) return r;
+  if (int r = clear_x(ws.xb[0])) return r;
+  if (int r = clear_x(ws.xb[1])) return r;
+  // audio = z with the padding zeroed; the first boundary then scales it in place (audio = sigma * audio)
+  if (int r = launch_ragged_rows(audio, z, 0, 1, d.B, d.Tp, d.G, len, d.P, s)) return r;
+  if (int r = launch_flow_boundary(cfg, d, w, xfmt, -1, F - 1, audio, sigma, audio, nullptr, ws.xb[0], s, -2, 0, a0)) return r;
+  if (int r = clear_start()) return r;
+  for (int k = F - 1; k >= 0; --k) {
+    if (int r = launch_cond_tc(d, w, npass, k, k == F - 1 ? mel : nullptr, cond_bias, ws.h2b, ws.mel4, s, len)) return r;
+    for (int i = 0; i < L; ++i)
+      if (int r = layer_tc(cfg, d, w, npass, k, i, ws, audio, s, len, prefix)) return r;
+    if (int r = launch_flow_boundary(cfg, d, w, xfmt, k, k - 1, nullptr, sigma, audio, ws.eo, ws.xb[0], s, -2, 0, a0)) return r;
+    if (k > 0)
+      if (int r = clear_start()) return r;
   }
   return 0;
   };

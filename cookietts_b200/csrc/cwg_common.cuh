@@ -115,6 +115,11 @@ void set_range_all_layers(bool on);
 
 int launch_nonfinite(const float* x, size_t n, int* flag, cudaStream_t s, bool clear);
 
+// Ragged calls: n_planes planes of [B][T] rows of row_words 4-byte words, plane_bytes apart.  Row t of utterance b is
+// valid when t < len[b] * mult: valid rows are copied from src (src == NULL: left as they are), the others set to 0.
+int launch_ragged_rows(void* dst, const void* src, size_t plane_bytes, int n_planes, int B, int T, int row_words,
+                       const int* len, int mult, cudaStream_t s);
+
 int launch_mel_up(int xfmt, const float* mel, void* out, int B, int M, int frames, int frames_padded, int Tp, int H,
                   int linear, cudaStream_t s);
 
@@ -143,15 +148,17 @@ int launch_wf_fwd_boundary(int B, int Tp, int G, int F, const float* audio_in, f
                            cudaStream_t s);
 
 // ---- launchers implemented in cwg_tc.cu (tcgen05 / TMA path) ----
+// mel_len != NULL (ragged calls): frames f >= mel_len[b] of the im2col matrix are zeroed before the GEMM, so the cond rows
+// of the padding hold the bias alone - finite whatever the padded mel holds, and never tripping the f16f8 range check
 int launch_cond_tc(const Dims& d, const cwg_weights* w, int npass, int flow, const float* mel,
                    const float* cond_bias, __nv_bfloat16* h2_planes, __nv_bfloat16* mel4_planes,
-                   cudaStream_t s);
+                   cudaStream_t s, const int* mel_len = nullptr);
 
 // n_channels = 256: one persistent, epilogue-overlapped kernel per WN layer (cwg_ps.cu)
 int launch_layer_ps(const Dims& d, const cwg_weights* w, int npass, int flow, int layer,
                     const __nv_bfloat16* x_in, __nv_bfloat16* x_out, const __nv_bfloat16* h2,
                     float* eo, cudaStream_t s, const void* a0 = nullptr, const float* audio = nullptr,
-                    int a_off = 0, int a_nh = 0);
+                    int a_off = 0, int a_nh = 0, const int* rag_len = nullptr, const int* rag_prefix = nullptr);
 void debug_set_ps_timing(long long* buf);
 
 // n_channels = 512: two kernels per layer (cwg_tc512.cu); `acts` = bf16 hi/lo planes [B*T'][512]

@@ -57,6 +57,11 @@ struct PsArgs {
   int w0_row0;
   int* range_flag;        // f16f8, last residual layer only: |= 2 when x_new leaves the fp16 range (else NULL)
   long long* dbg;         // optional: per CTA {start, end, tiles} clock64 stamps
+  // RAGGED only (appended so that the other instantiations keep their parameter offsets): utterance b holds
+  // T'_b = len[b] * P valid group-steps and tile pairs [prefix[b], prefix[b+1]); n_pairs = prefix[nb] on the device
+  const int* len;         // [nb] mel frames, already clamped to [1, Tm] (cwg_infer_ragged's plan kernel)
+  const int* prefix;      // [nb + 1]
+  int nb, P;
 };
 
 constexpr int P_OFF_WSE = 12 * TILE_A;                 // 196608
@@ -65,6 +70,9 @@ constexpr int P_OFF_B2 = P_OFF_B1 + 2048;
 constexpr int P_OFF_BAR = P_OFF_B2 + 1024;
 constexpr int P_OFF_S = P_OFF_BAR + 256;               // fused0: start weights [256][8] fp32 + bias [256]
 constexpr int P_SMEM = P_OFF_S + 256 * 8 * 4 + 1024 + 1024;   // 226560 (<= 232448)
+constexpr int P_OFF_R = P_OFF_S + 256 * 8 * 4 + 1024;  // RAGGED: tile-pair prefix sums [nb + 1]
+constexpr int P_SMEM_R = P_SMEM + (4 * (CWG_RAGGED_MAX_BATCH + 1) + 15) / 16 * 16;   // 230672
+static_assert(P_SMEM_R <= 232448, "ragged prefix sums do not fit next to the layer kernel's shared memory");
 constexpr int TILE_S = 4096;                           // [128 rows][16 x 16-bit], 32B swizzle
 constexpr int P_EPI_THREADS = 256;
 constexpr int P_THREADS = 128 + P_EPI_THREADS;
@@ -92,7 +100,11 @@ __device__ __forceinline__ void split16_f8_words(const float* v, uint32_t* hi, u
 }
 
 // FUSED0: the layer-0 fold variant (compiled separately so that its extra registers do not burden layers 1..L-1)
-template <int NPASS, bool FUSED0>
+// RAGGED: per-utterance lengths (cwg_infer_ragged).  Pair p maps to (b, t0) through the prefix sums of the utterances'
+// tile pairs, so pairs wholly past T'_b do not exist; rows t >= T'_b of a computed tile are stored as zeros (every
+// plane) and leave eo and the range flag alone.  The caller keeps every row t >= T'_b of both x buffers at 0, so the
+// dilated taps of valid rows read exactly the zero padding a call for utterance b alone would see.
+template <int NPASS, bool FUSED0, bool RAGGED>
 __global__ void __launch_bounds__(P_THREADS, 1)
 k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ CUtensorMap tm_x_lo,
            const __grid_constant__ CUtensorMap tm_h_hi, const __grid_constant__ CUtensorMap tm_h_lo,
@@ -132,8 +144,11 @@ k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ 
   uint64_t* xold_full = r_free + 2;         // [2]: x_old block of column group h has landed
   uint64_t* acts0_ready = xold_full + 2;    // leader: the gate of sweep 0 (channels [0, 128) of acts) is written in both CTAs
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acts0_ready + 1);
+  int* pre_s = reinterpret_cast<int*>(smem + P_OFF_R);                 // RAGGED only
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  if (RAGGED)
+    for (int i = threadIdx.x; i <= a.nb; i += P_THREADS) pre_s[i] = __ldg(a.prefix + i);
   auto slot = [&](int i) { return smem + i * TILE_A; };
   auto wse = [&](int plane, int kb) { return smem + P_OFF_WSE + plane * 8192 + kb * 2048; };
 
@@ -176,10 +191,19 @@ k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ 
     umma_f8_2sm(d, da, db, id, 1u); umma_f8_2sm(d, da + 2, db + 2, id, 1u);
     umma_f8_2sm(d, da + 4, db + 4, id, 1u); umma_f8_2sm(d, da + 6, db + 6, id, 1u);
   };
-  // tile of pair p handled by this CTA
+  // number of tile pairs of the launch, and the tile of pair p handled by this CTA.  RAGGED: every role walks p upwards,
+  // so a per-thread cursor over the prefix sums finds b
+  auto n_pairs = [&]() { return RAGGED ? pre_s[a.nb] : a.n_pairs; };
+  int ub = 0;
   auto tile_of = [&](int p, int& b, int& t0) {
-    b = p / a.pairs_per_utt;
-    t0 = ((p - b * a.pairs_per_utt) * 2 + (int)rank) * 128;
+    if (RAGGED) {
+      while (pre_s[ub + 1] <= p) ++ub;
+      b = ub;
+      t0 = ((p - pre_s[ub]) * 2 + (int)rank) * 128;
+    } else {
+      b = p / a.pairs_per_utt;
+      t0 = ((p - b * a.pairs_per_utt) * 2 + (int)rank) * 128;
+    }
   };
 
   if (warp == 0 && lane == 0) {
@@ -188,7 +212,7 @@ k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ 
     if (F8) { tma_prefetch_desc(&tm_x_l8); tma_prefetch_desc(&tm_x_h8); }
     if (NPASS == 3) { tma_prefetch_desc(&tm_x_lo); tma_prefetch_desc(&tm_h_lo); }
     int s = 0; uint32_t pm = 0;
-    for (int p = cluster_id; p < a.n_pairs; p += n_clusters) {
+    for (int p = cluster_id; p < n_pairs(); p += n_clusters) {
       int b, t0; tile_of(p, b, t0);
       for (int g = 0; g < 2; ++g) {
         if (FUSED0) {
@@ -244,7 +268,7 @@ k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ 
       arm(&full[4 + j], TILE_A);
     };
     const int w2_row = a.w2_row0 + (int)rank * 128;
-    for (int p = cluster_id; p < a.n_pairs; p += n_clusters) {
+    for (int p = cluster_id; p < n_pairs(); p += n_clusters) {
       for (int g = 0; g < 2; ++g) {
         const int w1_row = a.w1_row0 + (int)rank * 256 + g * 128;
         if (FUSED0) {
@@ -320,7 +344,7 @@ k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ 
     bool wse_seen = false;
     int it_no = 0;
     long long* tdbg = a.dbg ? a.dbg + (size_t)blockIdx.x * PS_DBG_STRIDE + 4 : nullptr;
-    for (int p = cluster_id; p < a.n_pairs; p += n_clusters, par ^= 1u, ++it_no) {
+    for (int p = cluster_id; p < n_pairs(); p += n_clusters, par ^= 1u, ++it_no) {
       const bool stamp = tdbg && it_no == 2;
       for (int g = 0; g < 2; ++g) {
         if (stamp) tdbg[3 * g] = clock64();
@@ -493,9 +517,9 @@ k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ 
     int n_tiles = 0;
     uint32_t par = 0, xph = 0;
     int b_cur = 0;
-    for (int p = cluster_id; p < a.n_pairs; p += n_clusters, par ^= 1u, ++n_tiles) {
+    for (int p = cluster_id; p < n_pairs(); p += n_clusters, par ^= 1u, ++n_tiles) {
       int b, t0; tile_of(p, b, t0);
-      const bool valid = t0 + row < a.Tp;
+      const bool valid = t0 + row < (RAGGED ? __ldg(a.len + b) * a.P : a.Tp);
       const size_t m = (size_t)b * a.Tp + (size_t)min(t0 + row, a.Tp - 1);
       if (a.b1_bstride != 0 && b != b_cur) {    // per-utterance gate bias (b is uniform over the CTA): reload on a change
         b_cur = b;
@@ -645,6 +669,9 @@ k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ 
               r[2 * j + 1] += f1 + g1;
             }
           }
+          if (RAGGED && !valid)      // padding of utterance b: zeros in every plane keep the taps of later layers exact
+#pragma unroll
+            for (int j = 0; j < 16; ++j) r[j] = 0.f;
           if (F8) {
             uint32_t nh[8], nl[8], l8[4], h8[4];
             if (a.range_flag) {      // the layer that consumes this x has no residual: an Inf here would not reach the waveform
@@ -658,7 +685,9 @@ k_layer_ps(const __grid_constant__ CUtensorMap tm_x_hi, const __grid_constant__ 
             *reinterpret_cast<uint4*>(u_hi + o1) = make_uint4(nh[4], nh[5], nh[6], nh[7]);
             *reinterpret_cast<uint4*>(u_lo + o0) = make_uint4(nl[0], nl[1], nl[2], nl[3]);
             *reinterpret_cast<uint4*>(u_lo + o1) = make_uint4(nl[4], nl[5], nl[6], nl[7]);
-            if (valid) {     // the two e5m2 planes: 16 bytes per row and chunk, straight to HBM (L2 merges the sectors)
+            // the two e5m2 planes: 16 bytes per row and chunk, straight to HBM (L2 merges the sectors); RAGGED also
+            // stores the zeros of the padded rows below T'_max
+            if (RAGGED ? t0 + row < a.Tp : valid) {
               *reinterpret_cast<uint4*>(a.xo_l8 + m * 256 + c * 16) = make_uint4(l8[0], l8[1], l8[2], l8[3]);
               *reinterpret_cast<uint4*>(a.xo_h8 + m * 256 + c * 16) = make_uint4(h8[0], h8[1], h8[2], h8[3]);
             }
@@ -790,24 +819,32 @@ int get_maps(const Dims& d, const cwg_weights* w, int npass, const __nv_bfloat16
   return 0;
 }
 
-template <int NPASS, bool FUSED0>
+template <int NPASS, bool FUSED0, bool RAGGED>
 int max_clusters(int* out) {
   static int cached = 0;                           // per process; all GPUs of a box are the same part
+  constexpr int smem = RAGGED ? P_SMEM_R : P_SMEM;
   if (cached == 0) {
-    CWG_CHECK_CUDA(cudaFuncSetAttribute(k_layer_ps<NPASS, FUSED0>, cudaFuncAttributeMaxDynamicSharedMemorySize, P_SMEM));
+    CWG_CHECK_CUDA(cudaFuncSetAttribute(k_layer_ps<NPASS, FUSED0, RAGGED>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     cudaLaunchConfig_t lc{};
-    lc.gridDim = dim3(2 * 148); lc.blockDim = dim3(P_THREADS); lc.dynamicSmemBytes = P_SMEM;
+    lc.gridDim = dim3(2 * 148); lc.blockDim = dim3(P_THREADS); lc.dynamicSmemBytes = smem;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     lc.attrs = at; lc.numAttrs = 1;
     int n = 0;
-    CWG_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&n, k_layer_ps<NPASS, FUSED0>, &lc));
+    CWG_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&n, k_layer_ps<NPASS, FUSED0, RAGGED>, &lc));
     CWG_REQUIRE(n >= 1, "k_layer_ps does not fit on this device (cudaOccupancyMaxActiveClusters = %d)", n);
     cached = n;
   }
   *out = cached;
   return 0;
+}
+
+template <bool RAGGED>
+int max_clusters(int npass, bool f0, int* out) {
+  return npass == 3 ? (f0 ? max_clusters<3, true, RAGGED>(out) : max_clusters<3, false, RAGGED>(out))
+       : npass == 2 ? (f0 ? max_clusters<2, true, RAGGED>(out) : max_clusters<2, false, RAGGED>(out))
+                    : (f0 ? max_clusters<1, true, RAGGED>(out) : max_clusters<1, false, RAGGED>(out));
 }
 
 long long* g_ps_dbg = nullptr;
@@ -818,8 +855,12 @@ void debug_set_ps_timing(long long* buf) { g_ps_dbg = buf; }
 
 int launch_layer_ps(const Dims& d, const cwg_weights* w, int npass, int flow, int layer,
                     const __nv_bfloat16* x_in, __nv_bfloat16* x_out, const __nv_bfloat16* h2,
-                    float* eo, cudaStream_t s, const void* a0, const float* audio, int a_off, int a_nh) {
+                    float* eo, cudaStream_t s, const void* a0, const float* audio, int a_off, int a_nh,
+                    const int* rag_len, const int* rag_prefix) {
   // a0 != NULL (layer 0 only): the layer-0 fold - x_in is not read; see PsArgs::fused0
+  // rag_len / rag_prefix != NULL: the ragged form (PsArgs::len / prefix, both device arrays; d.B <= CWG_RAGGED_MAX_BATCH)
+  const bool ragged = rag_len != nullptr;
+  CWG_REQUIRE(!ragged || (rag_prefix && d.B <= CWG_RAGGED_MAX_BATCH), "ragged layer: bad arguments");
   CWG_REQUIRE(a0 == nullptr || (layer == 0 && w->w0_hi && w->w0_lo && audio && d.L >= 2 && d.MG == 16), "layer-0 fold: bad arguments");
   const PsMaps* m = nullptr;
   if (int r = get_maps(d, w, npass, x_in, x_out, h2, a0, &m)) return r;
@@ -841,20 +882,20 @@ int launch_layer_ps(const Dims& d, const cwg_weights* w, int npass, int flow, in
   a.start_w = w->start_w + (size_t)flow * d.C * (d.MG / 2); a.start_b = w->start_b + (size_t)flow * d.C;
   a.w0_row0 = flow * 2 * d.C;
   a.range_flag = (npass == 2 && (layer == d.L - 2 || range_all_layers())) ? range_flag() : nullptr;
+  a.len = rag_len; a.prefix = rag_prefix; a.nb = d.B; a.P = d.P;
   int ncl = 0;
   const bool f0 = a0 != nullptr;
-  if (int r = (npass == 3 ? (f0 ? max_clusters<3, true>(&ncl) : max_clusters<3, false>(&ncl))
-               : npass == 2 ? (f0 ? max_clusters<2, true>(&ncl) : max_clusters<2, false>(&ncl))
-                            : (f0 ? max_clusters<1, true>(&ncl) : max_clusters<1, false>(&ncl)))) return r;
-  if (ncl > a.n_pairs) ncl = a.n_pairs;
+  if (int r = ragged ? max_clusters<true>(npass, f0, &ncl) : max_clusters<false>(npass, f0, &ncl)) return r;
+  if (ncl > a.n_pairs) ncl = a.n_pairs;            // ragged: the padded count bounds the device-side one
   cudaLaunchConfig_t lc{};
-  lc.gridDim = dim3(2 * ncl); lc.blockDim = dim3(P_THREADS); lc.dynamicSmemBytes = P_SMEM; lc.stream = s;
+  lc.gridDim = dim3(2 * ncl); lc.blockDim = dim3(P_THREADS); lc.dynamicSmemBytes = ragged ? P_SMEM_R : P_SMEM; lc.stream = s;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeClusterDimension;
   at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
   lc.attrs = at; lc.numAttrs = 1;
 #define CWG_LAUNCH_PS(NP, F0)                                                                                          \
-  CWG_CHECK_CUDA(cudaLaunchKernelEx(&lc, k_layer_ps<NP, F0>, m->x_hi, m->x_lo, m->h_hi, m->h_lo, m->w1_hi, m->w1_lo,       \
+  CWG_CHECK_CUDA(cudaLaunchKernelEx(&lc, ragged ? k_layer_ps<NP, F0, true> : k_layer_ps<NP, F0, false>,               \
+                                    m->x_hi, m->x_lo, m->h_hi, m->h_lo, m->w1_hi, m->w1_lo,                            \
                                     m->w2_hi, m->w2_lo, m->wse_hi, m->wse_lo, m->xo_hi, m->xo_lo, m->x_l8, m->x_h8,    \
                                     m->h_l8, m->h_h8, m->w1_h8, m->w1_l8, m->w2_l8, m->wse_l8, m->a0_hi, m->a0_lo,  \
                                     m->w0_hi, m->w0_lo, a))

@@ -596,4 +596,30 @@ int launch_nonfinite(const float* x, size_t n, int* flag, cudaStream_t s, bool c
   return 0;
 }
 
+// ragged calls (cwg_infer_ragged): zero the rows of every utterance past its length, copying the valid rows from src
+// when given.  Grid: (RR_BLOCKS, B, planes), grid-stride over one utterance's plane; without src only the padded rows
+// are visited, so a batch without padding costs a few thousand empty blocks
+constexpr int RR_BLOCKS = 64;
+
+__global__ void k_ragged_rows(uint32_t* __restrict__ dst, const uint32_t* __restrict__ src, size_t plane_words, int T,
+                              int row_words, const int* __restrict__ len, int mult) {
+  const int b = blockIdx.y;
+  const long long n = (long long)T * row_words;
+  const long long lim = min((long long)__ldg(len + b) * mult * row_words, n);      // first word of the padding
+  const size_t o = blockIdx.z * plane_words + (size_t)b * n;
+  for (long long i = (src ? 0 : lim) + (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n;
+       i += (long long)gridDim.x * blockDim.x)
+    dst[o + i] = i < lim ? src[o + i] : 0u;
+}
+
+int launch_ragged_rows(void* dst, const void* src, size_t plane_bytes, int n_planes, int B, int T, int row_words,
+                       const int* len, int mult, cudaStream_t s) {
+  CWG_REQUIRE(dst && len && plane_bytes % 4 == 0 && ((uintptr_t)dst & 3) == 0, "ragged rows: bad arguments");
+  const long long blocks = ((long long)T * row_words + 255) / 256;
+  dim3 grid((unsigned)(blocks < RR_BLOCKS ? blocks : RR_BLOCKS), (unsigned)B, (unsigned)n_planes);
+  k_ragged_rows<<<grid, 256, 0, s>>>((uint32_t*)dst, (const uint32_t*)src, plane_bytes / 4, T, row_words, len, mult);
+  CWG_CHECK_CUDA(cudaGetLastError());
+  return 0;
+}
+
 }  // namespace cwg

@@ -182,12 +182,14 @@ k_cond_tc(const __grid_constant__ CUtensorMap tm_a_hi, const __grid_constant__ C
 
 int launch_cond_tc(const Dims& d, const cwg_weights* w, int npass, int flow, const float* mel,
                    const float* cond_bias, __nv_bfloat16* h2_planes, __nv_bfloat16* mel4_planes,
-                   cudaStream_t s) {
+                   cudaStream_t s, const int* mel_len) {
   const size_t n4 = (size_t)d.B * d.Tm * d.KCp;
   __nv_bfloat16* m4_hi = mel4_planes; __nv_bfloat16* m4_lo = mel4_planes + n4;
   if (mel != nullptr) {
     k_im2col_mel<<<(unsigned)((n4 + 255) / 256), 256, 0, s>>>(mel, m4_hi, m4_lo, d.B, d.M, d.Tm, d.J, d.KCp, npass == 2);
     CWG_CHECK_CUDA(cudaGetLastError());
+    if (mel_len)      // row f of utterance b reads frames <= f only (causal upsampler): rows f < len[b] are unaffected
+      if (int r = launch_ragged_rows(m4_hi, nullptr, n4 * 2, 2, d.B, d.Tm, d.KCp / 2, mel_len, 1, s)) return r;
   }
   const uint64_t rows = (uint64_t)d.B * d.Tm, ncol = (uint64_t)d.P * d.H;
   CUtensorMap ta_hi, ta_lo, tb_hi, tb_lo, tc_hi, tc_lo;

@@ -120,6 +120,50 @@ std::tuple<at::Tensor, at::Tensor> waveglow_infer(const at::Tensor& packed, at::
   return std::make_tuple(audio, status);
 }
 
+// waveglow_infer with per-utterance lengths (cwg_infer_ragged): lengths int32 [B] mel frames, 1 <= lengths[b] <= T_mel
+std::tuple<at::Tensor, at::Tensor> waveglow_infer_ragged(const at::Tensor& packed, at::IntArrayRef cfg, int64_t mode,
+                                                         int64_t embed_dim, int64_t n_speakers, const at::Tensor& mel,
+                                                         const c10::optional<at::Tensor>& speaker_ids, const at::Tensor& z,
+                                                         double sigma, const at::Tensor& lengths) {
+  const cwg_config c = config_from(cfg);
+  TORCH_CHECK(mel.is_cuda() && z.is_cuda() && packed.is_cuda() && lengths.is_cuda(),
+              "waveglow_infer_ragged needs CUDA tensors (no CPU fallback)");
+  TORCH_CHECK(mel.scalar_type() == at::kFloat && z.scalar_type() == at::kFloat && mel.is_contiguous() && z.is_contiguous(),
+              "mel and z must be contiguous fp32");
+  TORCH_CHECK(mel.dim() == 3 && mel.size(1) == c.n_mel, "mel must be [B, ", c.n_mel, ", T_mel]");
+  const int64_t B = mel.size(0), Tm = mel.size(2), T = Tm * c.hop_length;
+  TORCH_CHECK(z.dim() == 2 && z.size(0) == B && z.size(1) == T, "z must be [B, T_mel*hop]");
+  TORCH_CHECK(lengths.scalar_type() == at::kInt && lengths.is_contiguous() && lengths.dim() == 1 && lengths.size(0) == B,
+              "lengths must be a contiguous int32 [B] tensor");
+  const at::Device dev = mel.device();
+  TORCH_CHECK(lengths.device() == dev, "lengths must be on the device of mel");
+  c10::cuda::CUDAGuard guard(dev);
+  void* stream = (void*)c10::cuda::getCurrentCUDAStream(dev.index()).stream();
+  cwg_weights w;
+  check(cwg_packed_view(&c, (int)mode, (int)embed_dim, (int)n_speakers, aligned(packed, 256), (size_t)packed.numel() - 256, &w));
+  const int64_t* ids = nullptr;
+  at::Tensor ids_t;
+  if (embed_dim > 0) {
+    TORCH_CHECK(speaker_ids.has_value(), "this model has speaker embeddings: pass speaker ids");
+    ids_t = speaker_ids->to(dev, at::kLong).contiguous();
+    TORCH_CHECK(ids_t.numel() == B, "speaker ids must hold one entry per utterance");
+    ids = ids_t.data_ptr<int64_t>();
+  }
+  const auto f32 = at::TensorOptions().dtype(at::kFloat).device(dev);
+  at::Tensor cond_bias = at::empty({B, c.n_flows, c.cond_hidden}, f32);
+  check(cwg_cond_bias(&c, &w, ids, (int)B, cond_bias.data_ptr<float>(), stream));
+  const size_t ws_bytes = cwg_ragged_workspace_bytes(&c, (int)mode, (int)B, (int)Tm);
+  TORCH_CHECK(ws_bytes > 0, "libcwg: ", cwg_last_error());
+  at::Tensor ws = at::empty({(int64_t)ws_bytes + 1024}, at::TensorOptions().dtype(at::kByte).device(dev));
+  at::Tensor audio = at::empty({B, T}, f32);
+  check(cwg_infer_ragged(&c, &w, (int)mode, mel.data_ptr<float>(), cond_bias.data_ptr<float>(), z.data_ptr<float>(),
+                         (float)sigma, lengths.data_ptr<int32_t>(), audio.data_ptr<float>(), aligned(ws, 1024), ws_bytes,
+                         (int)B, (int)Tm, stream));
+  at::Tensor status = at::empty({1}, at::TensorOptions().dtype(at::kInt).device(dev));
+  check(cwg_infer_status(aligned(ws, 1024), status.data_ptr<int32_t>(), stream));
+  return std::make_tuple(audio, status);
+}
+
 // Forward-direction mixing matrices: uint8 blob = W_k padded [F][MG][MG] fp32, then logdet [2][F] fp64 (cwg_pack_forward)
 at::Tensor waveglow_pack_forward(at::TensorList tensors, std::string names, at::IntArrayRef cfg) {
   TORCH_CHECK(!tensors.empty(), "empty state_dict");
@@ -228,6 +272,8 @@ TORCH_LIBRARY(cookietts_b200, m) {
   m.def("waveglow_pack(Tensor[] tensors, str names, int[] cfg, int mode) -> Tensor");
   m.def("waveglow_infer(Tensor packed, int[] cfg, int mode, int embed_dim, int n_speakers, Tensor mel, Tensor? speaker_ids, "
         "Tensor z, float sigma, int[] ev_begin, int[] ev_end) -> (Tensor, Tensor)");
+  m.def("waveglow_infer_ragged(Tensor packed, int[] cfg, int mode, int embed_dim, int n_speakers, Tensor mel, "
+        "Tensor? speaker_ids, Tensor z, float sigma, Tensor lengths) -> (Tensor, Tensor)");
   m.def("waveglow_pack_forward(Tensor[] tensors, str names, int[] cfg) -> Tensor");
   m.def("waveglow_forward(Tensor packed, Tensor packed_fwd, int[] cfg, int mode, int embed_dim, int n_speakers, Tensor mel, "
         "Tensor? speaker_ids, Tensor audio, bool want_log_s) -> (Tensor z, Tensor log_s, Tensor logp_terms, Tensor status)");
@@ -239,6 +285,7 @@ TORCH_LIBRARY(cookietts_b200, m) {
 TORCH_LIBRARY_IMPL(cookietts_b200, CUDA, m) {
   m.impl("waveglow_pack", &waveglow_pack);
   m.impl("waveglow_infer", &waveglow_infer);
+  m.impl("waveglow_infer_ragged", &waveglow_infer_ragged);
   m.impl("waveglow_pack_forward", &waveglow_pack_forward);
   m.impl("waveglow_forward", &waveglow_forward);
   m.impl("nonfinite", &nonfinite);

@@ -44,10 +44,14 @@ def pcm16(audio: torch.Tensor, n_valid=None, pad_samples: int = 0, saturate: boo
 @torch.no_grad()
 def vocode_pcm16(vocoder, mels: torch.Tensor, output_lengths: Sequence[int], hop_length: int, sampling_rate: int,
                  vocoder_batch_size: int = 16, cat_silence_s: float = 0.0, denoiser=None, denoise_strength: float = 0.1,
-                 saturate: bool = False, **infer_kwargs) -> List[np.ndarray]:
+                 saturate: bool = False, ragged: bool = False, **infer_kwargs) -> List[np.ndarray]:
     """mels [N, n_mel, T_mel] (padded) -> list of N int16 arrays, utterance j holding
     output_lengths[j]*hop_length samples followed by int(cat_silence_s*sampling_rate) zeros
-    (text2speech.py:656-665 the slice loop, :672-694 trim / pad / int16)."""
+    (text2speech.py:656-665 the slice loop, :672-694 trim / pad / int16).
+
+    ragged=True passes each slice's output lengths (clamped to [1, T_mel]) to `vocoder.infer(..., lengths=...)`: every
+    utterance is vocoded as if it were alone, independent of its batch-mates, and the padding costs no WN-layer work.
+    The default keeps the reference's behaviour (the padded slice is vocoded as one batch, then trimmed)."""
     lengths = [int(x) for x in output_lengths]
     if len(lengths) != mels.shape[0]:
         raise ValueError("output_lengths must have one entry per mel")
@@ -59,6 +63,8 @@ def vocode_pcm16(vocoder, mels: torch.Tensor, output_lengths: Sequence[int], hop
         part = mels[i:i + vocoder_batch_size]
         sl = slice(i, i + vocoder_batch_size)
         kw = slice_per_utterance(infer_kwargs, sl, n_items)        # speaker ids follow their utterances
+        if ragged:
+            kw["lengths"] = [min(max(n, 1), part.shape[2]) for n in lengths[i:i + vocoder_batch_size]]
         audio = vocoder.infer(part, **kw) if hasattr(vocoder, "infer") else vocoder(part)
         if isinstance(audio, tuple):
             audio = audio[0]

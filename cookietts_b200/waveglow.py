@@ -383,13 +383,22 @@ class WaveGlow(nn.Module):
 
     # ------------------------------------------------------------------ the hot path
     @torch.no_grad()
-    def infer(self, spect, speaker_id=None, sigma=1.0, *, speaker_ids=None, z=None, layer_events=None):
+    def infer(self, spect, speaker_id=None, sigma=1.0, *, speaker_ids=None, z=None, layer_events=None, lengths=None):
         """mel [B, n_mel, T_mel] -> audio [B, T_mel*hop] (fp32, on the module's device).
 
         `speaker_id` is the reference keyword (glow.py:314); `speaker_ids` is what
         `Denoiser`/notebooks pass (denoiser.py:39).  `z` ([B, T], standard normal) injects the
         latent the reference draws internally; None draws it here.  `layer_events` (optional,
-        (begin, end) lists of torch.cuda.Event) are recorded around each WN-layer launch."""
+        (begin, end) lists of torch.cuda.Event) are recorded around each WN-layer launch.
+
+        `lengths` (optional, B integers in [1, T_mel]: mel frames per utterance of a padded batch) computes utterance b
+        as if it were alone: out[b, :lengths[b]*hop] equals, byte for byte, infer(spect[b:b+1, :, :lengths[b]],
+        z=z[b:b+1, :lengths[b]*hop]) in the same precision, and out[b, lengths[b]*hop:] is 0.  Neither the padded mel
+        nor the padded part of z is read, and WN-layer tiles wholly inside the padding are not computed.  Available in
+        the tensor-core modes of the 256-channel model (f16f8, bf16x3, bf16); runs with direct launches (no graph
+        replay, no layer_events)."""
+        if lengths is not None:
+            lengths = self._check_lengths(spect, lengths, layer_events)
         dev = self._device()
         if dev.type != "cuda":
             raise RuntimeError("cookietts_b200.WaveGlow.infer needs the module on a CUDA device (no CPU fallback)")
@@ -422,7 +431,7 @@ class WaveGlow(nn.Module):
                     if not e.cuda_event:
                         e.record(torch.cuda.current_stream(dev))
                 ev_b, ev_e = [int(e.cuda_event) for e in begin], [int(e.cuda_event) for e in end]
-            use_graph = (layer_events is None and not torch.cuda.is_current_stream_capturing() and
+            use_graph = (lengths is None and layer_events is None and not torch.cuda.is_current_stream_capturing() and
                          (self.graphs is True or (self.graphs == "auto" and batch * t_mel <= self.GRAPH_MAX_FRAMES)))
             if use_graph and self.graphs == "auto":
                 # "auto" captures a shape the second time it is seen: a stream of ever-new lengths (a TTS server) would pay
@@ -433,7 +442,11 @@ class WaveGlow(nn.Module):
                         self._graph_seen.clear()
                     self._graph_seen.add(gkey)
                     use_graph = False
-            if use_graph:
+            if lengths is not None:
+                lens = torch.tensor(lengths, dtype=torch.int32).to(dev)
+                audio, status = ops.waveglow_infer_ragged(self._packed, self._cfg_list, mode, self._embed_dim,
+                                                          self._n_speakers, mel, speaker_id, z, float(sigma), lens)
+            elif use_graph:
                 audio, status = self._graph_infer(ops, mode, mel, speaker_id, z, float(sigma))
             else:
                 audio, status = ops.waveglow_infer(self._packed, self._cfg_list, mode, self._embed_dim, self._n_speakers, mel,
@@ -448,9 +461,60 @@ class WaveGlow(nn.Module):
                                   "re-running this call in bf16x3", RuntimeWarning)
                     self.fallbacks += 1
                     self._ensure_packed("bf16x3")
-                    audio, _ = ops.waveglow_infer(self._packs["bf16x3"][0], self._cfg_list, _cabi.MODES["bf16x3"], self._embed_dim,
-                                                  self._n_speakers, mel, speaker_id, z, float(sigma), [], [])
+                    if lengths is not None:
+                        audio, _ = ops.waveglow_infer_ragged(self._packs["bf16x3"][0], self._cfg_list, _cabi.MODES["bf16x3"],
+                                                             self._embed_dim, self._n_speakers, mel, speaker_id, z,
+                                                             float(sigma), lens)
+                    else:
+                        audio, _ = ops.waveglow_infer(self._packs["bf16x3"][0], self._cfg_list, _cabi.MODES["bf16x3"],
+                                                      self._embed_dim, self._n_speakers, mel, speaker_id, z, float(sigma),
+                                                      [], [])
         return audio
+
+    def _check_lengths(self, spect, lengths, layer_events=None) -> list:
+        """Host-side checks of infer's `lengths` (before any device work) -> list of B ints."""
+        pc = self.pack_config
+        if self.precision not in ("f16f8", "bf16x3", "bf16") or pc.n_channels != 256:
+            raise NotImplementedError(
+                f"lengths needs the 256-channel WN layer kernel in a tensor-core mode (f16f8, bf16x3, bf16); this model runs "
+                f"n_channels = {pc.n_channels} in {self.precision!r}, whose kernels have no ragged form")
+        if layer_events is not None:
+            raise NotImplementedError("layer_events is not recorded for calls with lengths")
+        if spect.dim() != 3:
+            raise ValueError(f"spect must be [B, {pc.n_mel}, T_mel], got {tuple(spect.shape)}")
+        batch, t_mel = int(spect.shape[0]), int(spect.shape[2])
+        if torch.is_tensor(lengths):
+            if lengths.dtype.is_floating_point or lengths.dtype.is_complex or lengths.dtype == torch.bool:
+                raise ValueError(f"lengths must hold integers, got dtype {lengths.dtype}")
+            lengths = lengths.reshape(-1).tolist()
+        elif isinstance(lengths, np.ndarray):
+            if not np.issubdtype(lengths.dtype, np.integer):
+                raise ValueError(f"lengths must hold integers, got dtype {lengths.dtype}")
+            lengths = lengths.reshape(-1).tolist()
+        else:
+            lengths = list(lengths)
+        if len(lengths) != batch:
+            raise ValueError(f"lengths must hold one entry per utterance (B = {batch}), got {len(lengths)}")
+        for n in lengths:
+            if isinstance(n, (bool, np.bool_)) or not isinstance(n, (int, np.integer)):
+                raise ValueError(f"lengths must hold integers, got {n!r}")
+            if not 1 <= n <= t_mel:
+                raise ValueError(f"every length must lie in [1, T_mel = {t_mel}], got {n}")
+        if batch > _cabi.RAGGED_MAX_BATCH:
+            raise ValueError(f"a call with lengths holds at most {_cabi.RAGGED_MAX_BATCH} utterances, got {batch}")
+        return [int(n) for n in lengths]
+
+    def tile_pairs(self, lengths, t_mel: int):
+        """(prefix sums [B + 1], total) of the WN-layer tile pairs a call with `lengths` computes per layer (cwg_ragged_pairs,
+        host arithmetic).  A padded call computes B * tile_pairs([t_mel], t_mel)[1]."""
+        lens = np.ascontiguousarray(np.asarray(lengths, dtype=np.int32).reshape(-1))
+        prefix = np.zeros(lens.size + 1, dtype=np.int32)
+        lib = _cabi.load()
+        n = lib.cwg_ragged_pairs(_cabi.make_config(self.pack_config), lens.ctypes.data, int(lens.size), int(t_mel),
+                                 prefix.ctypes.data)
+        if n < 0:
+            raise ValueError(lib.cwg_last_error().decode())
+        return prefix, int(n)
 
     def _graph_infer(self, ops, mode, mel, speaker_id, z, sigma):
         """Replays the captured launch sequence of this (shape, sigma) on static input buffers; captures it on first use."""

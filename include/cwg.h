@@ -188,6 +188,29 @@ int cwg_nonfinite(const float* x, size_t n, int32_t* flag, void* cuda_stream);
 /* Number of kernels cwg_infer launches for this configuration (bench.py's gpu_launches). */
 int cwg_launch_count(const cwg_config* cfg, int mode);
 
+/* ---- ragged batches: per-utterance lengths ------------------------------------------------------------------------
+ * cwg_infer_ragged is cwg_infer on a padded batch whose utterance b holds lengths[b] mel frames (1 <= lengths[b] <=
+ * t_mel).  Utterance b is computed as if it were alone: audio[b][0 .. lengths[b]*hop) equals, byte for byte, what
+ * cwg_infer returns for mel[b][:][0 .. lengths[b]) and z[b][0 .. lengths[b]*hop) in the same mode; audio[b][lengths[b]*hop
+ * ..) is 0.  WN-layer tiles wholly past an utterance's end are not computed.  Tensor-core modes of the 256-channel layer
+ * kernel only (CWG_MODE_F16F8, CWG_MODE_BF16X3, CWG_MODE_BF16); batch <= CWG_RAGGED_MAX_BATCH.
+ *   lengths    DEVICE int32 [batch], mel frames per utterance.  The device checks them: a value outside [1, t_mel] is
+ *              clamped into it and sets bit 2 (4) of the status word (cwg_infer_status), which otherwise works as for
+ *              cwg_infer.  Check lengths on the host (cwg_ragged_pairs) to reject them before any work is enqueued.
+ * The other arguments are cwg_infer's; the workspace size is cwg_ragged_workspace_bytes'. */
+#define CWG_RAGGED_MAX_BATCH 1024
+size_t cwg_ragged_workspace_bytes(const cwg_config* cfg, int mode, int batch, int t_mel);
+int cwg_infer_ragged(const cwg_config* cfg, const cwg_weights* w, int mode,
+                     const float* mel, const float* cond_bias, const float* z, float sigma, const int32_t* lengths,
+                     float* audio, void* workspace, size_t workspace_bytes,
+                     int batch, int t_mel, void* cuda_stream);
+/* Host-side tile-pair plan of a ragged call (pure host arithmetic): utterance b runs ceil(ceil(T'_b / 128) / 2) pairs of
+ * 128-step tiles per WN layer, T'_b = lengths[b] * hop / n_group.  lengths: HOST int32 [batch].  Writes the prefix sums
+ * [batch + 1] to prefix (may be NULL) and returns their total (the pairs every WN layer launch computes), or -1 on bad
+ * arguments (a length outside [1, t_mel] included; see cwg_last_error).  A padded call computes
+ * batch * ceil(ceil(t_mel * hop / n_group / 128) / 2). */
+int cwg_ragged_pairs(const cwg_config* cfg, const int32_t* lengths, int batch, int t_mel, int32_t* prefix);
+
 /* ---- stage-level entry points (tests bisect the pipeline with these) ---------------- */
 
 /* Folded cond chain for one flow: H2 [batch][T'][H] (fp32 in FFMA mode; bf16 hi/lo planes,
