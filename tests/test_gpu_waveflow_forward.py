@@ -15,7 +15,8 @@ from oracle.make_golden_waveflow import reference_kwargs
 from oracle.waveflow_oracle import WaveFlowConfig, synthetic_state_dict
 from oracle.waveglow_oracle import snr_db
 from tests.helpers import GOLDEN_DIR, max_abs
-from tests.waveflow_forward_ref import forward as ref_forward
+from oracle.waveflow_oracle import inverse as oracle_inverse, upsample_cond
+from tests.waveflow_forward_ref import forward as ref_forward, torch_forward
 
 pytestmark = pytest.mark.gpu
 
@@ -127,19 +128,33 @@ def test_round_trips(layout, frames, precision):
     close(xx.cpu().numpy(), x.cpu().numpy(), precision)
 
 
+SEP = dict(seperable_conv=True, win_length=960, hop_length=240)
+# layout: (config, B, T')
+FULL_HEIGHT = {
+    "config5": ({}, 2, 300),
+    "trained": (TRAINED, 2, 300),
+    "dense_h32": (dict(n_group=32), 3, 129),                                      # 31 rows, a 1-step tail tile
+    "sep2x5": (dict(n_group=12, kernel_size_h=2, kernel_size_w=5, **SEP), 2, 300),
+    "sep1x7": (dict(n_group=12, kernel_size_h=1, kernel_size_w=7, **SEP), 2, 300),
+    "sep7x7_h4": (dict(n_group=4, kernel_size_h=7, kernel_size_w=7, **SEP), 2, 300),   # 3 rows, fewer than the kernel
+}
+
+
 @pytest.mark.parametrize("precision", MODES)
-@pytest.mark.parametrize("layout", ["config5", "trained"])
+@pytest.mark.parametrize("layout", list(FULL_HEIGHT))
 def test_full_height_layer_equals_row_launches(layout, precision):
     """cwg_wf_forward_layer (all h-1 rows in one launch) against h-1 cwg_wf_layer launches (the inverse's row kernels) on
-    the same rows: same K order, so eo and the next layer's rows must be the same bytes."""
-    cfg = WaveFlowConfig(**(TRAINED if layout == "trained" else {}))
+    the same rows: same K order, so eo and the next layer's rows must be the same bytes.  The ring slots of rows not
+    written yet hold NaN: the row launches must skip them (the zero queue)."""
+    shape, B, Tp = FULL_HEIGHT[layout]
+    cfg = WaveFlowConfig(**shape)
     m = build(cfg, synthetic_state_dict(cfg, 8), precision)
     m._ensure_packed()
     lib = _cabi.load()
     _bind(lib)
     mode = _cabi.MODES[precision]
     h, L, KH, Cc = cfg.n_group, cfg.n_layers, cfg.kernel_size_h, 128
-    B, Tp, k = 2, 300, 1
+    k = 1
     stream = torch.cuda.current_stream().cuda_stream
     g = torch.Generator().manual_seed(3)
     mel = torch.zeros(B, Tp, 128)
@@ -154,7 +169,7 @@ def test_full_height_layer_equals_row_launches(layout, precision):
         full_x, full_eo = bufs.clone(), eo_in.clone()
         _cabi.check(lib.cwg_wf_forward_layer(m._ccfg, m._cw, mode, k, layer, full_x.data_ptr(), mel_up.data_ptr(),
                                              full_eo.data_ptr(), B, Tp * h, stream))
-        rings = torch.zeros(2, L, KH, B, Tp, Cc, dtype=torch.bfloat16, device="cuda")
+        rings = torch.full((2, L, KH, B, Tp, Cc), float("nan"), dtype=torch.bfloat16, device="cuda")
         src, dst = layer & 1, (layer + 1) & 1
         for r in range(h - 1):
             rings[:, layer, r % KH] = bufs[:, src, r]
@@ -167,6 +182,81 @@ def test_full_height_layer_equals_row_launches(layout, precision):
         assert torch.equal(full_x[:, src], bufs[:, src])                         # the input buffer is only read
         if layer == L - 1:
             assert torch.equal(full_x, bufs)
+
+
+# The edge configurations the tensor-core kernels accept: name -> (config, T', reference of `inverse`: the fp64 oracle, or
+# the fp32 CUDA-core mode on the device where the oracle is too slow)
+EDGE = {
+    "dense_h2_l1": (dict(n_group=2, n_layers=1, n_flows=2), 150, "oracle"),        # one height row; layer 0 is also the last
+    "dense_h32_l16_tp80": (dict(n_group=32, n_layers=16, n_flows=2), 80, "ffma"),   # 31 rows, dilations up to 32768
+    "dense_h32_l16_tp160": (dict(n_group=32, n_layers=16, n_flows=2), 160, "ffma"),
+    "sep7x7_h4": (dict(n_group=4, kernel_size_h=7, kernel_size_w=7, seperable_conv=True, n_flows=2), 150, "oracle"),
+    "sep2x5": (dict(n_group=12, kernel_size_h=2, kernel_size_w=5, seperable_conv=True, n_flows=2, hop_length=240), 100, "oracle"),
+    "sep1x7": (dict(n_group=12, kernel_size_h=1, kernel_size_w=7, seperable_conv=True, n_flows=2, hop_length=240), 100, "oracle"),
+    "sep4x1": (dict(n_group=12, kernel_size_h=4, kernel_size_w=1, seperable_conv=True, n_flows=2, hop_length=240), 100, "oracle"),
+    "mel1": (dict(n_mel_channels=1, n_flows=2), 150, "oracle"),
+    "mel128": (dict(n_mel_channels=128, n_flows=2), 150, "oracle"),
+    "nearest_tp1": (dict(upsample_mode="nearest", hop_length=16, win_length=64, n_flows=2), 1, "oracle"),   # hop == n_group
+    "nearest_tp129": (dict(upsample_mode="nearest", n_flows=2), 129, "oracle"),
+}
+# log_prob's relative error in the single-pass mode grows with the log_s terms it sums, not with |log p|: measured on a
+# B200 (power limit 1000 W) up to 2.2e-3 (nearest_tp1: 16 samples, |log p| ~ 20) and 1.1e-3 (mel128); bf16x3 stays within
+# LOGP_REL.
+EDGE_LOGP_REL = dict(LOGP_REL, bf16=4e-3)
+_edge_refs = {}
+
+
+def edge_inputs(name):
+    """A batch of 3 whose utterances have 100 %, 60 % and 30 % content (silent mel and zero z after it), the state dict and
+    inverse's reference output [3, T] (fp64)."""
+    if name not in _edge_refs:
+        _edge_refs.clear()
+        shape, tp, ref_kind = EDGE[name]
+        cfg = WaveFlowConfig(**shape)
+        sd = synthetic_state_dict(cfg, 21)
+        T = tp * cfg.n_group
+        frames = -(-T // cfg.hop_length)
+        mel, _ = inputs(cfg, 3, frames, 9)
+        z = torch.randn(3, T, generator=torch.Generator().manual_seed(10)) * 0.666
+        for b, frac in enumerate((1.0, 0.6, 0.3)):
+            mel[b, :, max(1, round(frac * frames)):] = -11.5129
+            z[b, max(cfg.n_group, round(frac * tp) * cfg.n_group):] = 0.0
+        if ref_kind == "oracle":
+            ref = oracle_inverse(sd, cfg, z.numpy(), mel.numpy(), np.float64)
+        else:
+            ref = build(cfg, sd, "ffma", graphs=False).inverse(z.cuda(), mel.cuda(), return_CPU=True)[0].numpy()
+        _edge_refs[name] = (cfg, sd, mel, z, ref)
+    return _edge_refs[name]
+
+
+@pytest.mark.parametrize("precision", MODES)
+@pytest.mark.parametrize("name", list(EDGE))
+def test_edge_configurations(name, precision):
+    """`inverse` against its reference, `encode` / `log_prob` against the fp64 restatement (tests/waveflow_forward_ref.py,
+    full-height torch form on the device), a round trip, and every utterance of the batch against its call alone."""
+    cfg, sd, mel, z, ref = edge_inputs(name)
+    m = build(cfg, sd, precision, graphs=False)
+    assert m.precision == precision
+    x = m.inverse(z.cuda(), mel.cuda(), return_CPU=False)[0]
+    close(x.cpu().numpy(), ref, precision)
+    tp = z.shape[1] // cfg.n_group
+    cond_up = upsample_cond(mel.numpy().astype(np.float64), tp, cfg.upsample_mode)
+    z_ref, ls_ref = torch_forward(sd, cfg, x.double(), cond_up)
+    z_ref, ls_ref = z_ref.cpu().numpy(), ls_ref.cpu().numpy()
+    zz = m.encode(mel, x)
+    close(zz.cpu().numpy(), z_ref, precision)
+    sigma = 0.666
+    T = x.shape[1]
+    lp_ref = -(z_ref ** 2).sum(1) / (2 * sigma ** 2) - 0.5 * T * np.log(2 * np.pi * sigma ** 2) + ls_ref
+    lp = m.log_prob(mel, x, sigma)
+    rel = np.abs(lp.cpu().numpy() - lp_ref).max() / np.abs(lp_ref).max()
+    assert rel <= EDGE_LOGP_REL[precision], (precision, rel)
+    close(zz.cpu().numpy(), z.numpy(), precision)                                # round trip: encode(inverse(z)) ~ z
+    for u in range(3):
+        xu = m.inverse(z[u:u + 1].cuda(), mel[u:u + 1].cuda(), return_CPU=False)[0]
+        assert torch.equal(xu[0], x[u]), f"utterance {u}: inverse differs from its call alone"
+        assert torch.equal(m.encode(mel[u:u + 1], x[u:u + 1])[0], zz[u]), f"utterance {u}: encode differs from its call alone"
+        assert torch.equal(m.log_prob(mel[u:u + 1], x[u:u + 1], sigma)[0], lp[u]), f"utterance {u}: log_prob differs"
 
 
 @pytest.mark.parametrize("layout", ["config5", "trained"])

@@ -55,16 +55,17 @@ def log_prob(sd, cfg, audio, cond, sigma=1.0, cond_up=None):
 def torch_forward(sd, cfg, audio, cond_up):
     """The same forward in torch (fp64, differentiable in `audio` [B, T]), with WN_2d as causal Conv2d over all h-1 rows at
     once rather than row by row; cond_up [B, n_mel, T'] is the interpolated mel.  GTU, res_skip, one 1x1 cond layer, dense
-    or depthwise-separable in_layers (the tensor-core subset).  -> (z [B, T], sum of log_s per utterance)."""
+    or depthwise-separable in_layers (the tensor-core subset).  Runs on audio's device.  -> (z [B, T], sum of log_s per
+    utterance)."""
     import torch
     import torch.nn.functional as F
-    t = lambda a: torch.as_tensor(np.asarray(a, np.float64))
+    t = lambda a: torch.as_tensor(np.asarray(a, np.float64), device=audio.device)
     B, T = audio.shape
     h, C, L, kh, kw = cfg.n_group, cfg.n_channels, cfg.n_layers, cfg.kernel_size_h, cfg.kernel_size_w
     Tp = T // h
     x = audio.reshape(B, Tp, h).transpose(1, 2)
     cond_up = t(cond_up)
-    ls = torch.zeros(B, dtype=torch.float64)
+    ls = torch.zeros(B, dtype=torch.float64, device=audio.device)
     for k in range(cfg.n_flows):
         p = f"WN.{k}.WN."
         x = permute_height(x, k)
