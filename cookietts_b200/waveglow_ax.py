@@ -432,7 +432,8 @@ class WaveGlowAx(nn.Module, AxFrontEndMixin):
         self.pack_config = pc
         self._packed, self._packed_key, self._graphs = {"flows": flows}, key, {}
 
-    def _bind_general(self):
+    @staticmethod
+    def _bind_general():
         lib = _cabi.load()
         if not getattr(lib, "_axg_bound", False):
             lib.cwg_axg_workspace_bytes.restype = C.c_size_t

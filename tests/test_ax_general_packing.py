@@ -1,6 +1,7 @@
 """CPU check of the general fp32 mode's packed arrays (cookietts_b200.waveglow_ax.pack_ax_general): a numpy statement of
-what cwg_axg_flow (csrc/cwg_fd.cu) does with them, step for step, reproduces the reference goldens.  The kernels
-themselves are held to the same goldens on the GPU (tests/test_gpu_waveglow_ax.py)."""
+what cwg_axg_flow (csrc/cwg_fd.cu) does with them, step for step (tests/axg_flow_ref.py), reproduces the reference
+goldens.  The kernels themselves are held to the same goldens on the GPU (tests/test_gpu_waveglow_ax.py), and to that
+numpy statement at many-tile shapes (tests/test_gpu_fp32_shapes.py)."""
 import json
 import os
 
@@ -11,47 +12,10 @@ from cookietts_b200.waveglow_ax import pack_ax_general, GATED_UNITS
 from oracle.ax_frontend_oracle import conv1d, _act
 from oracle.waveflow_oracle import upsample_cond, _w
 from oracle.waveglow_ax_oracle import AxConfig, synthetic_state_dict, GATED_UNITS as ORACLE_UNITS
+from tests.axg_flow_ref import flow_packed
 from tests.helpers import GOLDEN_DIR, max_abs
 
 CASES = ["waveglow_axv_gsirru", "waveglow_axv_merge", "waveglow_axv_noskip", "waveglow_axv_cond", "waveglow_axv_unit_stu"]
-
-
-def flow_packed(pk, cfg, n_rem, c_all, z):
-    """cwg_axg_flow on channels-first z [B, G, T] (in place), c_all [B, 2CL, T]."""
-    G, C, L, ks = cfg.n_group, cfg.n_channels, cfg.n_layers, cfg.kernel_size
-    nh, off = n_rem // 2, G - n_rem
-    T = z.shape[2]
-    ua, ub = ORACLE_UNITS[cfg.gated_unit.upper()]
-
-    def mix():
-        z[:, off:] = np.einsum("oc,bct->bot", pk["winv"].astype(np.float64), z[:, off:])
-    if not cfg.mix_first:
-        mix()
-    h = np.einsum("oc,bct->bot", pk["start_w"].astype(np.float64), z[:, off:off + nh]) + pk["start_b"][None, :, None]
-    out = np.zeros_like(h)
-    split = cfg.res_skip and not cfg.merge_res_skip
-    for i in range(L):
-        d = cfg.dilation(i)
-        pad = d * (ks // 2)
-        hp = np.pad(h, ((0, 0), (0, 0), (pad, pad)))
-        pre = np.zeros((z.shape[0], 2 * C, T))
-        for j in range(ks):
-            pre += np.einsum("oc,bct->bot", pk["in_w"][i, :, :, j].astype(np.float64), hp[:, :, j * d:j * d + T])
-        pre += pk["in_b"][i][None, :, None] + c_all[:, 2 * C * i:2 * C * (i + 1)]
-        acts = ua(pre[:, :C]) * ub(pre[:, C:])
-        if cfg.res_skip:
-            rs = np.einsum("oc,bct->bot", pk["rs_w"][i].astype(np.float64), acts) + pk["rs_b"][i][None, :, None]
-            if split and i < L - 1:
-                h = h + rs[:, :C]
-                out += rs[:, C:]
-            else:
-                out += rs[:, :C]
-        else:
-            out += acts
-    e = np.einsum("oc,bct->bot", pk["end_w"].astype(np.float64), out) + pk["end_b"][None, :, None]
-    z[:, off + nh:] = (z[:, off + nh:] - e[:, nh:]) / np.exp(e[:, :nh])
-    if cfg.mix_first:
-        mix()
 
 
 @pytest.mark.parametrize("name", CASES)
